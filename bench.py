@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- CQL updates/s (batch 1024) and users scored top-10/s on the ML-20M-shaped synthetic log.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     torchrun ... bench.py --gpus N ...        (N > 1: one rank per GPU, NCCL)
 
 One JSON line on stdout (rank 0).  A *step* is one CQL update (temp -> alpha -> critic ->
@@ -28,6 +28,7 @@ import numpy as np
 
 ROOT = Path(__file__).resolve().parent
 sys.path.insert(0, str(ROOT))
+sys.dont_write_bytecode = True    # the benchmark writes nothing into the source tree (it may be read-only)
 
 BATCH = 1024
 K_TOP = 10
@@ -305,6 +306,12 @@ def run_ours(args):
         launches += stepper.launches_per_step * (stepper.replayed_steps - r0)
     clk = clocks.stop(t_w0, t_w1)
     value = world * args.steps / (ms / 1e3)
+    dump = {}                      # --dump-outputs (rank 0): name -> array
+    dumping = bool(args.dump_outputs) and rank == 0
+    if dumping:                    # the learner after the last timed update, read back outside the timed region
+        adam_m, adam_v, _ = eng.get_optimizer()
+        dump.update(update_state=eng.get_state(), update_adam_m=adam_m, update_adam_v=adam_v,
+                    update_metrics=np.array(list(eng.read_metrics().values()), dtype=np.float32))
 
     # ---- per-kernel durations (events inside one real update), rank 0 reporting ----
     timings = [eng.timed_update(stream=sh) for _ in range(5)][1:]
@@ -400,6 +407,8 @@ def run_ours(args):
     users_per_s = n_score / (score_ms / 1e3)
     top_dev = oi.cpu().numpy()
     assert (top_dev[:, 0] >= 0).all() and not np.isin(top_dev[0], seen[indptr[users[0]]:indptr[users[0] + 1]]).any()
+    if dumping:                    # item ids < 2**24: exact in float32
+        dump.update(score_top_items=top_dev.astype(np.float32), score_top_scores=osc.cpu().numpy())
     eng.score_topk(users[:n_warm], items, K_TOP, indptr, seen)         # warm-up of the host-buffer entry (scratch allocation)
     barrier()
     t0 = time.perf_counter()
@@ -517,6 +526,12 @@ def run_ours(args):
             "sampler": {"metric": "replay gather", "value": gather_gbs, "unit": "GB/s", "rows": cnt,
                         "frac_of_hbm": gather_gbs / pk.get("hbm_gbs", 6650.0)},
         }
+        if dumping:
+            assert sum(a.nbytes for a in dump.values()) <= 64 << 20
+            out_dir = Path(args.dump_outputs)
+            out_dir.mkdir(parents=True, exist_ok=True)
+            for name, a in dump.items():
+                np.save(out_dir / f"{name}.npy", a)
         print(json.dumps(line), flush=True)
     # teardown: graphs first (NCCL communicators must not be destroyed under a live captured graph); a watchdog
     # guarantees the process exits even if a collective teardown stalls -- the JSON line is already out
@@ -697,7 +712,15 @@ def main():
     ap.add_argument("--stress-rows", type=int, default=1_000_000_000)
     ap.add_argument("--stress-precision", choices=["fp32", "tf32x3", "f16x3", "bf16"], default="bf16",
                     help="stress workload: bf16 = the variant BASELINE configs[4] names; f16x3 = the FP32-grade product path")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="ml20m workload: write what the timed paths computed as DIR/<name>.npy (float32, rank 0): the learner "
+                         "state, Adam moments and metrics after the last timed update, and the top-10 items and scores of the "
+                         "timed scoring pass (rank 0's users).  Inputs are seeded, so two builds can be compared output for output")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be >= 1")
+    if args.dump_outputs and (args.impl != "ours" or args.workload != "ml20m"):
+        ap.error("--dump-outputs is implemented for --impl ours --workload ml20m")
     if args.impl == "reference":
         run_reference(args)
     elif args.workload == "ml1m":
