@@ -716,13 +716,15 @@ inline void launch_fwd_tc(Handle* h, const FwdJobs& jobs, cudaStream_t st, QSrc*
   using C = std::conditional_t<F16X3, tc::HCfg, tc::Cfg<TF32>>;
   tc::TcFwdJobs tj{};
   tj.n = jobs.n;
-  // big launches of the f16x3 path run on CTA pairs (one H1 tile feeds all 256 output columns); CQL_NO_PAIR=1 = A/B switch
+  // big launches of the f16x3 path run on CTA pairs (one H1 tile feeds all 256 output columns); CQL_NO_PAIR=1 = A/B switch.
+  // Critics only: the actor has no CTA-pair operand copy (pack_slots, adam_pack), so its forward stays on one-CTA kernels
+  // at any batch size, as its backward does in launch_bwd_tc.
   bool pair = false;
   if constexpr (F16X3) {
     static const bool no_pair = std::getenv("CQL_NO_PAIR") != nullptr;
     int pair_items = 0;
     for (int i = 0; i < jobs.n; ++i) pair_items += jobs.j[i].n_nets * ((jobs.j[i].rows + 2 * tc::TM - 1) / (2 * tc::TM));
-    pair = !no_pair && pair_items >= h->num_sms / 2;
+    pair = !no_pair && IN == 3 && pair_items >= h->num_sms / 2;
   }
   // small launches (the B-row passes of the actor step: 16-32 work items of 128 columns) run on 32-column work items
   // instead -- four times as many CTAs, a quarter of the operand load each; CQL_NO_SMALL=1 = A/B switch

@@ -22,36 +22,7 @@ from replay_cql_b200 import layout
 from tests import helpers as Hp
 
 pytestmark = pytest.mark.gpu
-TOL = 1e-4
-NAMES = ("temp_loss", "temp", "alpha_loss", "alpha", "critic_loss", "actor_loss")
-
-
-def _tensors(flat, C):
-    """flat state (or flat Adam buffer) -> {tag: array} over every network tensor + the two scalars"""
-    un = layout.unpack_state(np.asarray(flat, dtype=np.float32), C)
-    out = {}
-    for grp in ("actor", "targ_actor"):
-        for k in layout.NET_KEYS:
-            out[(grp, k)] = un[grp][k]
-    for grp in ("critics", "targ_critics"):
-        for c in range(C):
-            for k in layout.NET_KEYS:
-                out[(grp, c, k)] = un[grp][c][k]
-    out[("log_temp",)] = np.array([un["log_temp"]])
-    out[("log_alpha",)] = np.array([un["log_alpha"]])
-    return out
-
-
-def _check(tag, gpu, ref32, ref64, budgeted):
-    e32 = Hp.rel_err(gpu, ref32)
-    if e32 <= TOL:
-        return
-    d = Hp.rel_err(ref32, ref64)
-    # the budget rule is only legitimate where the float32 oracle itself misses
-    assert d > TOL / 4, (tag, "float32 oracle is accurate here, the GPU must be too", e32, d)
-    e64 = Hp.rel_err(gpu, ref64)
-    assert e64 <= max(TOL, 4 * d), (tag, e32, e64, d)
-    budgeted.append((tag, e32, e64, d))
+TOL = Hp.TOL
 
 
 @pytest.mark.parametrize("precision", ["f16x3", "fp32"])
@@ -71,7 +42,7 @@ def test_update_on_benched_configuration(engine_factory, precision, B, n_users, 
         m64, _ = O.update(cfg, st64, {k: v.double() for k, v in batch.items()}, {k: v.double() for k, v in noise.items()})
         m32, _ = O.update(cfg, st, batch, noise)                       # st advances: next step starts from it
         mg, _ = eng.update_batch(Hp.batch_to_numpy(batch), Hp.noise_to_numpy(noise))
-        for name in NAMES:
+        for name in Hp.METRIC_NAMES:
             e32 = abs(mg[name] - m32[name])
             if e32 <= TOL * max(1.0, abs(m32[name])):
                 continue
@@ -80,22 +51,22 @@ def test_update_on_benched_configuration(engine_factory, precision, B, n_users, 
             assert abs(mg[name] - m64[name]) <= max(TOL * max(1.0, abs(m64[name])), 4 * d), (step, name, mg[name], m32[name], m64[name])
             budgeted.append(((step, name), e32, abs(mg[name] - m64[name]), d))
         # every updated tensor, targets included
-        g_t = _tensors(eng.get_state(), C)
-        r32 = _tensors(Hp.oracle_state_to_flat(st), C)
-        r64 = _tensors(Hp.oracle_state_to_flat(O.cast_state(st64, torch.float32)), C)
+        g_t = Hp.state_tensors(eng.get_state(), C)
+        r32 = Hp.state_tensors(Hp.oracle_state_to_flat(st), C)
+        r64 = Hp.state_tensors(Hp.oracle_state_to_flat(O.cast_state(st64, torch.float32)), C)
         for tag in r32:
-            _check((step, "state") + tag, g_t[tag], r32[tag], r64[tag], budgeted)
+            Hp.check_f64_budget((step, "state") + tag, g_t[tag], r32[tag], r64[tag], budgeted)
         # Adam moments (the gradients of this step are in them: m = 0.9 m' + 0.1 g) and the step counter
         gm, gv, gstep = eng.get_optimizer()
         om, ov, ostep = Hp.oracle_adam_to_flat(st)
         om64, ov64, _ = Hp.oracle_adam_to_flat(O.cast_state(st64, torch.float32))
         assert gstep == ostep == step + 1
         for name, g_, o_, o64_ in (("adam_m", gm, om, om64), ("adam_v", gv, ov, ov64)):
-            gt, ot, ot64 = _tensors(g_, C), _tensors(o_, C), _tensors(o64_, C)
+            gt, ot, ot64 = Hp.state_tensors(g_, C), Hp.state_tensors(o_, C), Hp.state_tensors(o64_, C)
             for tag in ot:
                 if tag[0].startswith("targ"):
                     continue
-                _check((step, name) + tag, gt[tag], ot[tag], ot64[tag], budgeted)
+                Hp.check_f64_budget((step, name) + tag, gt[tag], ot[tag], ot64[tag], budgeted)
     print(f"\n[{precision} B={B}] comparisons that needed the float64 budget: {len(budgeted)}")
     for b in budgeted:
         print("   ", b)
