@@ -155,7 +155,9 @@ int  cql_update_batches(cql_handle* h, int64_t n_batches, const float* obs, cons
 
 /* Data-parallel split of one update.  The host all-reduces (mean) the exposed
  * gradient buffer between phases; with world_size==1 the phases can be called
- * back to back.  phase 0: sample + forward passes + temp/alpha grads
+ * back to back (f16x3 at world_size==1: the critic and actor gradients are summed
+ * by the Adam step, i.e. they are in the buffer after phase 2 and phase 3).
+ *                phase 0: sample + forward passes + temp/alpha grads
  *                phase 1: temp/alpha Adam, critic backward  -> critic grads
  *                phase 2: critic Adam + Polyak, actor passes -> actor grads
  *                phase 3: actor Adam + Polyak, step counter

@@ -12,6 +12,11 @@
 // at most ~3.2 lr), with one spare binade.  The scale only has to keep fp16 in range: entries 2^-15 of the maximum are
 // still represented to 2^-24 of the maximum (fp16 subnormals), far inside the 1e-4 gates (DESIGN.md section 3).
 // The last CTA of each network handles the small tensors (W1, b1, b2, W3, b3) and the layer maxima (HMeta::wmax).
+//
+// At world size 1 the launch also sums the backward's gradient partials itself (k_reduce_grads_tc's fixed order, so the
+// gradients are bit-identical): a W2 CTA sums the dW2 split partials of its own 8 rows, and the small tensors are spread
+// over AP_SMALL_BLOCKS CTAs of 128 entries x 8 partial chunks each, whose layer maxima meet in global memory (the last of
+// them writes HMeta::wmax).  One launch boundary and one dependent L2 round trip less per gradient group.
 #pragma once
 #include "mlp_tc_h2.cuh"
 
@@ -22,7 +27,7 @@ struct AdamPackNet {
   float* p;            // network slot (fp32 parameters)
   float* m;
   float* v;
-  const float* g;
+  float* g;            // gradient (read; written when the launch sums the partials itself)
   float* targ;         // target slot
   uint8_t* fwd;        // packed forward, one-CTA layout (HCfg)            -- never null
   uint8_t* fwd2;       // packed forward, pair layout (H2Cfg)              -- null for the actor
@@ -40,6 +45,12 @@ struct AdamPackJobs {
   DpPeer dp;                // data-parallel peers (world > 1: gradients = mean over the ranks' staging buffers)
   int dp_group;             // gradient group of this launch (1 critics, 2 actor)
   long long dp_off;         // offset of network 0 of this launch inside a staging buffer
+  // world size 1: the gradient partials of the backward (small1 == nullptr: the gradient is read from n[i].g)
+  const float* small1;      // [n_nets][slots1][SMALL_STRIDE]  W1 | b1  (bwd1)
+  const float* small2;      // [n_nets][splits][SMALL_STRIDE]  b2 | W3 | b3  (bwd2)
+  const float* pw2;         // [n_nets][splits][H * H]         W2  (bwd2)
+  int slots1, splits;
+  int* wmax_acc;            // [CQL_MAX_CRITICS][16] layer maxima across the small-tensor CTAs, then [CQL_MAX_CRITICS] tickets
 };
 
 __device__ __forceinline__ float adam_one(float& p, float& m, float& v, float g, float step_size, float bc2s, float beta1,
@@ -69,10 +80,90 @@ __device__ __forceinline__ void store_chunk(const float (&x)[8], float s, uint8_
 
 constexpr int AP_ROWS = 8;                    // W2 rows per CTA
 constexpr int AP_W2_BLOCKS = H / AP_ROWS;     // 32
+constexpr int AP_SMALL_E = 128;               // small-tensor entries per CTA (x 8 partial chunks = 1024 threads)
+// small-tensor CTAs per network when the launch sums the partials: W1 | b1 | b2 | W3 | b3 (1537 / 1538 entries)
+constexpr int ap_small_blocks(int in_dim, int out_dim) { return (net_floats(in_dim, out_dim) - H * H + AP_SMALL_E - 1) / AP_SMALL_E; }
+
+// The small tensors when the launch sums the partials (world size 1): CTA AP_W2_BLOCKS + s takes the compact entries
+// [128 s, 128 s + 128) of W1 | b1 | b2 | W3 | b3; thread (chunk, entry) sums one of the 8 partial chunks, the first 128
+// threads combine them in chunk order and apply Adam + Polyak to their entry (loads issued before the partials').
+__device__ __forceinline__ void adam_small_fold(const AdamPackJobs& jobs, const AdamPackNet& nt, float step_size, float bc2s,
+                                             int slot_clr, int* wm) {
+  __shared__ float part[8][AP_SMALL_E];
+  __shared__ int last;
+  const int tid = threadIdx.x, in_dim = jobs.in_dim, out_dim = jobs.out_dim;
+  const int w2_lo = off_W2(in_dim), n_e = net_floats(in_dim, out_dim) - H * H;
+  const int s_blk = blockIdx.x - AP_W2_BLOCKS, n_blk = gridDim.x - AP_W2_BLOCKS;
+  const int el = tid % AP_SMALL_E, chunk = tid / AP_SMALL_E;
+  const int e = s_blk * AP_SMALL_E + el;                     // compact index: W1 | b1 then b2 | W3 | b3
+  const int idx = e < w2_lo ? e : e + H * H;                 // index inside the network slot
+  const bool own = tid < AP_SMALL_E && e < n_e;
+  float p = 0.f, m = 0.f, v = 0.f, t = 0.f;
+  if (own) { p = nt.p[idx]; m = nt.m[idx]; v = nt.v[idx]; t = nt.targ[idx]; }
+  float s = 0.f;
+  if (e < n_e) {                                             // small1 / small2 are indexed by the compact index
+    if (e < w2_lo) s = chunk_sum8<float, 16>(jobs.small1 + (size_t)blockIdx.y * jobs.slots1 * SMALL_STRIDE + e, jobs.slots1, SMALL_STRIDE, chunk);
+    else s = chunk_sum8<float, 16>(jobs.small2 + (size_t)blockIdx.y * jobs.splits * SMALL_STRIDE + e, jobs.splits, SMALL_STRIDE, chunk);
+  }
+  part[chunk][el] = s;
+  if (tid < 16) wm[tid] = 0;
+  if (s_blk == 0 && tid == 0) {
+    nt.w2max[slot_clr] = 0;
+    // the step counter (position in the epoch permutation, Philox stream); nothing in this launch reads it
+    if (jobs.step_inc != nullptr && blockIdx.y == 0) *jobs.step_inc += 1;
+  }
+  __syncthreads();
+  if (own) {
+    float g = part[0][el];
+#pragma unroll
+    for (int c = 1; c < 8; ++c) g += part[c][el];
+    nt.g[idx] = g;
+    // adam_one + Polyak with every rounding written out, as the per-unit path below is compiled: there the second moment
+    // is contracted as fma(g, g (1 - beta2), beta2 v) and the step as fma(-m / denom, step_size, p); left to the compiler
+    // this context got fma(v, beta2, (1 - beta2) g g) -- one rounding apart, which Adam carries into every later step
+    m = __fmaf_rn(__fsub_rn(g, m), __fsub_rn(1.f, jobs.beta1), m);
+    v = __fmaf_rn(g, __fmul_rn(g, __fsub_rn(1.f, jobs.beta2)), __fmul_rn(jobs.beta2, v));
+    p = __fmaf_rn(-__fdiv_rn(m, __fadd_rn(__fdiv_rn(__fsqrt_rn(v), bc2s), jobs.eps)), step_size, p);
+    t = __fmaf_rn(t, __fsub_rn(1.f, jobs.tau), __fmul_rn(jobs.tau, p));
+    nt.p[idx] = p; nt.m[idx] = m; nt.v[idx] = v; nt.targ[idx] = t;
+    // layer maxima for the operand generators: W1 columns -> wm[c], b1 -> wm[3], W3 rows -> wm[4 + o] (targets at + 8)
+    int slot = -1;
+    if (idx < off_b1(in_dim)) slot = idx % in_dim;
+    else if (idx < w2_lo) slot = 3;
+    else if (idx >= off_W3(in_dim) && idx < off_b3(in_dim, out_dim)) slot = 4 + (idx - off_W3(in_dim)) / H;
+    if (slot >= 0) {
+      atomicMax(&wm[slot], __float_as_int(fabsf(p)));
+      atomicMax(&wm[8 + slot], __float_as_int(fabsf(t)));
+    }
+  }
+  __syncthreads();
+  int* acc = jobs.wmax_acc + blockIdx.y * 16;
+  unsigned int* ticket = reinterpret_cast<unsigned int*>(jobs.wmax_acc + CQL_MAX_CRITICS * 16) + blockIdx.y;
+  if (tid < 16 && wm[tid] != 0) atomicMax(&acc[tid], wm[tid]);
+  __threadfence();
+  __syncthreads();
+  if (tid == 0) {
+    const unsigned int k = atomicAdd(ticket, 1u);
+    last = k == (unsigned int)n_blk - 1;
+    if (last) *ticket = 0;
+  }
+  __syncthreads();
+  if (!last) return;
+  __threadfence();
+  if (tid < 8) {                                             // read and clear for the next launch
+    const float w = __int_as_float(atomicExch(&acc[tid], 0)), wt = __int_as_float(atomicExch(&acc[8 + tid], 0));
+    reinterpret_cast<HMeta*>(nt.fwd + HCfg::META_OFF)->wmax[tid] = w;
+    reinterpret_cast<HMeta*>(nt.bwd + HCfg::META_OFF)->wmax[tid] = w;
+    reinterpret_cast<HMeta*>(nt.tfwd + HCfg::META_OFF)->wmax[tid] = wt;
+    if (nt.fwd2) reinterpret_cast<HMeta*>(nt.fwd2 + H2Cfg::META_OFF)->wmax[tid] = w;
+    if (nt.bwd2) reinterpret_cast<HMeta*>(nt.bwd2 + H2Cfg::META_OFF)->wmax[tid] = w;
+    if (nt.tfwd2) reinterpret_cast<HMeta*>(nt.tfwd2 + H2Cfg::META_OFF)->wmax[tid] = wt;
+  }
+}
 
 __global__ void __launch_bounds__(1024, 1) k_adam_pack(const AdamPackJobs jobs, const StepInfo* __restrict__ si) {
   grid_dep_wait();
-  __shared__ float tile[AP_ROWS][H + 4];
+  __shared__ __align__(16) float tile[AP_ROWS][H + 4];   // (vector accesses: 16-byte alignment stated, not left to the layout)
   __shared__ int wm[16];
   const AdamPackNet nt = jobs.n[blockIdx.y];
   const int in_dim = jobs.in_dim, out_dim = jobs.out_dim;
@@ -94,15 +185,21 @@ __global__ void __launch_bounds__(1024, 1) k_adam_pack(const AdamPackJobs jobs, 
     // 1024 threads, TWO consecutive entries each (128 threads per row).  With 256 threads x 8 entries the kernel was bound
     // by the latency of each thread's 24 IEEE sqrt / divide sequences at 8 warps per SM (ncu r02: 11.4 us warm, issue
     // slots 20 %, 1390 warp instructions per warp).
-    __shared__ float gw2[AP_ROWS][H];                 // data-parallel: the rows' mean gradients
+    __shared__ __align__(16) float gw2[AP_ROWS][H];                 // data-parallel: the rows' mean gradients
     __shared__ float rmax[AP_ROWS][4], rmaxt[AP_ROWS][4];
     const int r8 = tid >> 7, c2 = tid & 127;
     const int n = blockIdx.x * AP_ROWS + r8;
     const size_t off = (size_t)off_W2(in_dim) + (size_t)n * H + c2 * 2;
     const float w2max_prev = __int_as_float(nt.w2max[slot_rd]);      // (read with the first loads, not after the barrier)
-    float2 g = *reinterpret_cast<const float2*>(nt.g + off);
+    float2 g;
+    if (jobs.small1 == nullptr) g = *reinterpret_cast<const float2*>(nt.g + off);
     float2 m = *reinterpret_cast<const float2*>(nt.m + off), v = *reinterpret_cast<const float2*>(nt.v + off);
     float2 p = *reinterpret_cast<const float2*>(nt.p + off), t = *reinterpret_cast<const float2*>(nt.targ + off);
+    if (jobs.small1 != nullptr) {                      // this thread's two entries summed over the dW2 split partials
+      g = reduce8<float2, 4>(jobs.pw2 + (size_t)blockIdx.y * jobs.splits * H * H + (off - off_W2(in_dim)), jobs.splits,
+                             (size_t)H * H);
+      *reinterpret_cast<float2*>(nt.g + off) = g;
+    }
     if (dp) {                                          // every fourth thread fetches the chunk's 8 means (from the slice's owner)
       if ((c2 & 3) == 0) {
         float4 g0 = *reinterpret_cast<const float4*>(nt.g + off), g1 = *reinterpret_cast<const float4*>(nt.g + off + 4);
@@ -183,6 +280,10 @@ __global__ void __launch_bounds__(1024, 1) k_adam_pack(const AdamPackJobs jobs, 
     if (dp) dp_consume_done(jobs.dp, jobs.dp_group, gridDim.x * gridDim.y);
     return;
   }
+  if (jobs.small1 != nullptr) {
+    adam_small_fold(jobs, nt, step_size, bc2s, slot_clr, wm);
+    return;
+  }
   if (tid >= 256) return;     // the small tensors are 256 threads' work (exited threads do not count at the barriers below)
   // ---------------- the small tensors: W1 | b1, b2, W3 | b3 (+ layer maxima for the operand generators) ----------------
   if (tid < 16) wm[tid] = 0;
@@ -190,7 +291,7 @@ __global__ void __launch_bounds__(1024, 1) k_adam_pack(const AdamPackJobs jobs, 
   __syncthreads();
   // data-parallel: the mean gradients of the small entries are fetched into shared memory FIRST, two 16-byte groups per
   // thread with all ranks' loads in flight together (one after the other, each entry would cost an NVLink round trip)
-  __shared__ float gsm[2048];
+  __shared__ __align__(16) float gsm[2048];
   const int w2_lo = off_W2(in_dim), w2_hi = w2_lo + H * H;
   if (dp) {
     {                                                        // 2048 compact entries = 256 threads x two 16-byte groups

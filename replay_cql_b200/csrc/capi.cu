@@ -219,6 +219,7 @@ void create_impl(const cql_config* cfg, cql_handle* ch) {
       h.packed_fwd2 = h.dalloc<uint8_t>((size_t)(2 + 2 * C) * h.packed_net_bytes2);
       h.packed_bwd2 = h.dalloc<uint8_t>((size_t)(1 + C) * h.packed_net_bytes2);
       h.w2max = h.dalloc<int>((size_t)(2 + 2 * C) * 4);
+      h.ap_wmax = h.dalloc<int>((size_t)CQL_MAX_CRITICS * 17);
       if (const char* sw = std::getenv("CQL_PAIR_SWAP")) h.pair_swap_b = std::atoi(sw);
     }
     h.slots1 = (f16 ? tc::HCfg::NEW : 4) * h.num_sms;

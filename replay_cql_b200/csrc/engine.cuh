@@ -109,6 +109,7 @@ struct Handle {
   unsigned int* b2_tickets = nullptr;   // [C][64] group tickets of the f16x3 bwd2 kernel
   int slots1 = 0, splits_tc = 0, tc_slices = 1;
   int last_dx_parts = 0;           // parts (nets x column slices) of dX_part written by the last dx launch
+  int last_slots1 = 0, last_splits = 0;   // partial counts of the last weight-gradient backward (summed by k_adam_pack)
   // CTA-pair (cta_group::2) f16x3 kernels: W2 of every slot in the pair layout (mlp_tc_h2.cuh)
   uint8_t* packed_fwd2 = nullptr;  // [(2+2C) slots][H2Cfg::PACKED_NET_BYTES]  B[n][k] = W2[n][k]
   uint8_t* packed_bwd2 = nullptr;  // [(1+C) slots]                           B[n][k] = W2[k][n]
@@ -116,6 +117,7 @@ struct Handle {
   DpPeer dp;                       // data-parallel peers (cql_dp_attach); world <= 1: single GPU
   bool dp_fused = false;           // the gradient exchange happens INSIDE the update kernels (f16x3 path, dp_peer.cuh)
   int* w2max = nullptr;            // [(2+2C) slots][4]: rotating max|W2| slots of the fused Adam + pack kernel (adam_pack.cuh)
+  int* ap_wmax = nullptr;          // k_adam_pack's layer maxima across its small-tensor CTAs + tickets (AdamPackJobs::wmax_acc)
   int pair_swap_b = 0;             // which cluster rank holds the first half of the operand rows (probed at create)
 
   // optional event marks for cql_timed_update

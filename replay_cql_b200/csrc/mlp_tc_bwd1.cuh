@@ -18,6 +18,7 @@ struct Bwd1Job {
   const float* params;    // first net slot (fp32)
   const uint8_t* packedT; // packed W2^T of the first net (B[n=k][kk=j] = W2[j][k])
   float* small1;          // [n_nets][slots][SMALL_STRIDE]: only W1 | b1 entries written; slots = 4*gridDim.x, zeroed by caller
+                          // (or by the kernel itself: zero_small1)
   float4* dX_part;        // [n_nets][SLICES][rows] or nullptr
   int rows, n_nets, slots;
   // dx-only launch of the actor step (f16x3): dOut = d(actor loss)/dQ through the min over the critics, taken by the
@@ -26,7 +27,22 @@ struct Bwd1Job {
   const float* q_part = nullptr;   // [n_nets][q_parts][rows]
   int q_parts = 0;
   float dq_scale = 0.f;            // -1 / B
+  // f16x3 kernels: every CTA zeroes its own slots (W1 | b1 of every network) before its first flush, so that no memset
+  // node sits between this launch and its predecessor in the step graph (which would cost the programmatic edge)
+  int zero_small1 = 0;
 };
+// (zero_small1) slots [blockIdx.x * per_cta, + per_cta) of every network, W1 | b1 entries; ends with a CTA barrier
+template <int IN>
+__device__ __forceinline__ void zero_small1_slots(const Bwd1Job& jb, int per_cta) {
+  if (!jb.zero_small1) return;
+  constexpr int NF4 = off_W2(IN) / 4;
+  for (int net = 0; net < jb.n_nets; ++net)
+    for (int s = 0; s < per_cta; ++s) {
+      float4* o = reinterpret_cast<float4*>(jb.small1 + ((size_t)net * jb.slots + (size_t)blockIdx.x * per_cta + s) * SMALL_STRIDE);
+      for (int f = threadIdx.x; f < NF4; f += blockDim.x) o[f] = make_float4(0.f, 0.f, 0.f, 0.f);
+    }
+  __syncthreads();
+}
 // d(actor loss)/dQ of row r for network net_i: dq_scale on the critic with the smallest Q (first one on ties), else 0
 template <int IN, int OUT>
 __device__ __forceinline__ float actor_dq_of(const Bwd1Job& jb, int net_i, int r) {
@@ -569,6 +585,57 @@ __device__ __forceinline__ float4 sum_strided4(const float* __restrict__ p, int 
   }
   return make_float4((s0.x + s1.x) + (s2.x + s3.x), (s0.y + s1.y) + (s2.y + s3.y), (s0.z + s1.z) + (s2.z + s3.z),
                      (s0.w + s1.w) + (s2.w + s3.w));
+}
+
+// The same sums for one or two components of sum_strided4's float4 (per component they are the same additions in the same
+// order, so the results are bit-identical), with every load of a chunk of at most NPRE partials issued before the first
+// addition.  reduce8 = k_reduce_grads_tc's whole reduction of n partials: 8 chunks of ceil(n/8), combined in chunk order.
+__device__ __forceinline__ void vacc(float& s, float a) { s += a; }
+__device__ __forceinline__ void vacc(float2& s, float2 a) { s.x += a.x; s.y += a.y; }
+__device__ __forceinline__ float vfold(float a, float b, float c, float d) { return (a + b) + (c + d); }
+__device__ __forceinline__ float2 vfold(float2 a, float2 b, float2 c, float2 d) {
+  return make_float2((a.x + b.x) + (c.x + d.x), (a.y + b.y) + (c.y + d.y));
+}
+template <typename V> __device__ __forceinline__ V vld(const float* p);
+template <> __device__ __forceinline__ float vld<float>(const float* p) { return __ldg(p); }
+template <> __device__ __forceinline__ float2 vld<float2>(const float* p) { return __ldg(reinterpret_cast<const float2*>(p)); }
+template <typename V, int NPRE>
+__device__ __forceinline__ V sum_strided_pre(const float* __restrict__ p, int n, size_t stride) {
+  static_assert(NPRE % 4 == 0, "groups of four");
+  V s0{}, s1{}, s2{}, s3{};
+  if (n <= NPRE) {
+    V a[NPRE];
+#pragma unroll
+    for (int i = 0; i < NPRE; ++i)
+      if (i < n) a[i] = vld<V>(p + (size_t)i * stride);
+#pragma unroll
+    for (int i = 0; i < NPRE; i += 4)
+      if (i + 4 <= n) { vacc(s0, a[i]); vacc(s1, a[i + 1]); vacc(s2, a[i + 2]); vacc(s3, a[i + 3]); }
+#pragma unroll
+    for (int i = 0; i < NPRE; ++i)
+      if (i >= (n & ~3) && i < n) vacc(s0, a[i]);
+  } else {
+    int i = 0;
+    for (; i + 4 <= n; i += 4) {
+      const V a = vld<V>(p + (size_t)i * stride), b = vld<V>(p + (size_t)(i + 1) * stride);
+      const V c = vld<V>(p + (size_t)(i + 2) * stride), d = vld<V>(p + (size_t)(i + 3) * stride);
+      vacc(s0, a); vacc(s1, b); vacc(s2, c); vacc(s3, d);
+    }
+    for (; i < n; ++i) vacc(s0, vld<V>(p + (size_t)i * stride));
+  }
+  return vfold(s0, s1, s2, s3);
+}
+template <typename V, int NPRE>
+__device__ __forceinline__ V chunk_sum8(const float* __restrict__ p, int n, size_t stride, int chunk) {
+  const int per = (n + 7) / 8, lo = chunk * per, hi = min(n, lo + per);
+  return hi > lo ? sum_strided_pre<V, NPRE>(p + (size_t)lo * stride, hi - lo, stride) : V{};
+}
+template <typename V, int NPRE>
+__device__ __forceinline__ V reduce8(const float* __restrict__ p, int n, size_t stride) {
+  V t = chunk_sum8<V, NPRE>(p, n, stride, 0);
+#pragma unroll
+  for (int c = 1; c < 8; ++c) vacc(t, chunk_sum8<V, NPRE>(p, n, stride, c));
+  return t;
 }
 
 // block = 32 float4 groups (128 consecutive parameters) x 8 slot-chunks; chunk partials combined through shared

@@ -502,6 +502,7 @@ __global__ void __launch_bounds__(HCfg::THREADS, 1) tc_bwd1_h_kernel(const Bwd1J
   tc_fence_after();
   const uint32_t tmem = *slot;
   grid_dep_wait();            // everything above overlapped the predecessor's tail (programmatic dependent launch)
+  if (WGRADS) zero_small1_slots<IN>(jb, 2);          // slots (CTA, epilogue group)
 
   if (warp == C::MMA_WARP) {
     const uint32_t idesc = instr_desc(FMT_F16, TM, C::NS);

@@ -552,6 +552,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(H2Cfg::THREADS, 1) t
   tc_fence_after();
   const uint32_t tmem = *slot;
   grid_dep_wait();
+  if (WGRADS) zero_small1_slots<IN>(jb, 2);          // slots (CTA, column half)
 
   if (warp == C::MMA_WARP) {
     const uint32_t idesc = instr_desc(FMT_F16, C::TMP, C::NP);

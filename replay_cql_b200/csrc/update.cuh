@@ -843,6 +843,15 @@ inline void pack_weights(Handle* h, int slot, int n_slots, int /*in_dim*/, cudaS
   pack_slots(h, slots, n_slots, st);
 }
 
+// f16x3 at world size 1: k_adam_pack sums the backward's gradient partials itself and the weight-gradient bwd1 kernels
+// zero their own partial slots -- no k_reduce_grads_tc launch and no memset node per gradient group, so every edge of
+// the backward chain is a programmatic one.  Data-parallel runs keep the separate reduction: it is where their gradient
+// exchange starts (phase A of dp_peer.cuh, or the exchange between cql_step_phase calls).  CQL_NO_FOLD=1 = A/B switch.
+inline bool fold_grads(const Handle* h) {
+  static const bool no_fold = std::getenv("CQL_NO_FOLD") != nullptr || std::getenv("CQL_NO_FUSED_ADAM") != nullptr;
+  return !no_fold && h->cfg.precision == CQL_PREC_F16X3 && h->cfg.world_size <= 1 && h->dp.world <= 1;
+}
+
 // ---- tensor-core backward of one job: bwd1 (dH1, dW1, db1, dx) + bwd2 (dW2, db2, dW3, db3) + reduce
 template <bool TF32, int IN, int OUT, bool WGRADS, bool DX, bool F16X3 = false>
 inline void launch_bwd_tc(Handle* h, const BwdJob& jb, float* grads_out, cudaStream_t st, int mark_mid = -1, int mark_end = -1) {
@@ -876,11 +885,13 @@ inline void launch_bwd_tc(Handle* h, const BwdJob& jb, float* grads_out, cudaStr
   const int grid1 = pair ? 2 * clusters1 : (items_s < h->num_sms ? items_s : h->num_sms);
   h->last_dx_parts = jb.n_nets * (pair ? (int)tc::H2Cfg::PARTS : n_slices);
   const int slots1 = (F16X3 ? 2 : 4) * grid1;      // f16x3: one slot per (CTA, epilogue group)
-  if (WGRADS) CQL_CUDA(cudaMemsetAsync(h->small1, 0, (size_t)jb.n_nets * slots1 * SMALL_STRIDE * sizeof(float), st));
+  const bool fold = F16X3 && WGRADS && fold_grads(h);
+  if (WGRADS && !fold) CQL_CUDA(cudaMemsetAsync(h->small1, 0, (size_t)jb.n_nets * slots1 * SMALL_STRIDE * sizeof(float), st));
   tc::Bwd1Job j1{jb.X, jb.dOut, jb.h2, jb.params,
                  pair ? h->packed_bwd2 + (size_t)slot * h->packed_net_bytes2 : h->packed_bwd + (size_t)slot * h->packed_net_bytes_bwd,
                  h->small1, DX ? h->dX_part : nullptr, jb.rows, jb.n_nets, slots1};
   j1.q_part = jb.q_part; j1.q_parts = jb.q_parts; j1.dq_scale = jb.dq_scale;
+  j1.zero_small1 = fold ? 1 : 0;
   // bwd1 and bwd2 of one job are independent (both only read X, dOut, H2).  For the small jobs (the actor's B rows:
   // a few dozen CTAs each) they run side by side on a forked branch -- the fork/join is captured into the step graph.
   constexpr int RS2 = F16X3 ? tc::B2HCfg::RS : tc::B2Cfg<TF32>::RS;
@@ -941,6 +952,11 @@ inline void launch_bwd_tc(Handle* h, const BwdJob& jb, float* grads_out, cudaStr
     CQL_CUDA(cudaStreamWaitEvent(st, h->ev_join, 0));
   }
   if (mark_end >= 0) mark(h, st, mark_end);
+  if (fold) {                          // summed by the group's k_adam_pack
+    h->last_slots1 = slots1;
+    h->last_splits = splits;
+    return;
+  }
   if (!skip_launch(64))
     launch_pdl(tc::k_reduce_grads_tc, dim3(dim3((NET_STRIDE / 4 + 31) / 32, jb.n_nets)), dim3(256), 0, st, h->small1, slots1, h->small2, h->pw2_tc,
                                                                                   splits, IN, OUT, grads_out,
@@ -977,8 +993,15 @@ inline void adam_pack(Handle* h, int first_slot, int n_nets, int in_dim, int out
     n.tfwd2 = critic ? h->packed_fwd2 + (size_t)tslot * h->packed_net_bytes2 : nullptr;
     n.w2max = h->w2max + slot * 4;
   }
+  const bool fold = fold_grads(h);
+  if (fold) {                          // the partials of this group's backward (launch_bwd_tc)
+    j.small1 = h->small1; j.small2 = h->small2; j.pw2 = h->pw2_tc;
+    j.slots1 = h->last_slots1; j.splits = h->last_splits;
+    j.wmax_acc = h->ap_wmax;
+  }
+  const int blocks = tc::AP_W2_BLOCKS + (fold ? tc::ap_small_blocks(in_dim, out_dim) : 1);
   if (!skip_launch(128))
-    launch_pdl(tc::k_adam_pack, dim3(tc::AP_W2_BLOCKS + 1, n_nets), dim3(1024), 0, st, j, h->stepinfo);
+    launch_pdl(tc::k_adam_pack, dim3(blocks, n_nets), dim3(1024), 0, st, j, h->stepinfo);
   CQL_LAUNCH_CHECK(h);
 }
 
