@@ -34,6 +34,7 @@ extern "C" {
 #define CQL_ACT_DIM 1           /* relevance */
 #define CQL_MAX_CRITICS 4
 #define CQL_MAX_TOPK 1024
+#define CQL_MAX_N_STEPS 64      /* longest n-step TD horizon (cql_set_n_steps) */
 
 /* precision of the 256x256 hidden-layer contraction */
 enum { CQL_PREC_FP32 = 0,      /* CUDA-core FP32 (exact-order reference path on the GPU) */
@@ -123,6 +124,20 @@ int  cql_set_table_sharded(cql_handle* h, int32_t sharded);
  * Row i depends only on (seed, i).  replaces: nothing in the reference -- stands in for SURVEY 8d's generator where
  * the log itself (24 GB of columns) is not worth moving through the host. */
 int  cql_synth_table(cql_handle* h, int64_t n_rows, int64_t n_users, int64_t n_items, uint64_t seed);
+/* n-step TD returns (d3rlpy's `n_steps`, DESIGN.md section 1), 1..CQL_MAX_N_STEPS, default 1.  With n_steps > 1 every
+ * table built after the call (cql_build_mdp, cql_mdp_finish, cql_load_transitions, cql_synth_table) holds n-step rows:
+ * for one-step row t with k = min(n_steps, steps from t to its episode's end, t included) -- an episode ends at a
+ * terminal row or at the end of the table -- the row is (s_t, a_t, R | s'_{t+k-1}, term_{t+k-1}, discount) with
+ * R = sum_{j<k} gamma^j r_{t+j} and discount = gamma^k, both accumulated in float64 and stored as float; the TD
+ * target is then y = R + discount * min_i Q_targ_i(s', tanh(mu(s'))) * (1 - term).  The one-step expansion is an
+ * out-of-place pass over the rows the builder writes (transiently twice the table's memory); the builders' optional
+ * host outputs stay the one-step episode steps.  With n_steps = 1 the tables (slot 7 = 0) and the update are as they
+ * always were.  A table already loaded is DROPPED when the value changes (it was built for the other horizon: rebuild
+ * or reload it); captured update graphs are destroyed. */
+int  cql_set_n_steps(cql_handle* h, int32_t n_steps);
+/* Replay table uploaded verbatim from rows_host [n][8] in the table's own format (e.g. cql_sample_rows / a checkpoint
+ * of this handle's table): no expansion, whatever n_steps is. */
+int  cql_set_table_rows(cql_handle* h, const float* rows_host, int64_t n);
 /* stand-alone gather for the K1 roofline sweep: out_dev [count][8] floats.
  * idx_dev NULL => the handle's epoch permutation starting at position `pos`. */
 int  cql_sample_rows(cql_handle* h, const int64_t* idx_dev, int64_t pos, int64_t count,
@@ -144,6 +159,11 @@ int  cql_update(cql_handle* h, int64_t n_steps, float* metrics6, void* stream);
 int  cql_update_batch(cql_handle* h, const float* obs, const float* act, const float* rew,
                       const float* next_obs, const float* term, const float* noise,
                       float* metrics6, float* grads_out, void* stream);
+/* The same update on B table-format rows (host [B][8]: s.x s.y a r s'.x s'.y term discount), e.g. rows of an n-step
+ * table; slot 7 is the row's TD discount when n_steps > 1 and is ignored otherwise.  cql_update_batch (and the
+ * one-step batches of cql_update_batches / cql_upload_batch) stage discount = gamma when n_steps > 1. */
+int  cql_update_batch_rows(cql_handle* h, const float* rows_host, const float* noise, float* metrics6, float* grads_out,
+                           void* stream);
 
 /* n_batches consecutive updates on caller-supplied minibatches (host buffers, n_batches x B rows each, Philox noise):
  * the host loop of an offline trainer that owns its batches.  Per step the minibatch goes host -> pinned ring -> device

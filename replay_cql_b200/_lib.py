@@ -19,6 +19,7 @@ SQUASH_EPS, SQUASH_SOFTPLUS = 0, 1
 SCORE_Q, SCORE_POLICY = 0, 1
 BUF_SCALAR_GRADS, BUF_CRITIC_GRADS, BUF_ACTOR_GRADS, BUF_METRICS, BUF_PARAMS, BUF_ALL_GRADS = range(6)
 MAX_TOPK = 1024
+MAX_N_STEPS = 64                                     # CQL_MAX_N_STEPS: longest n-step TD horizon
 DT_I32, DT_I64, DT_F32, DT_F64 = 0, 1, 2, 3          # cql_mdp_append chunk dtypes
 
 
@@ -78,6 +79,9 @@ SIGNATURES = {
     "cql_mma_bench": (C.c_int, [_P, C.c_int, C.c_int, _P]),
     "cql_synth_table": (C.c_int, [_P, C.c_int64, C.c_int64, C.c_int64, C.c_uint64]),
     "cql_set_table_sharded": (C.c_int, [_P, C.c_int32]),
+    "cql_set_n_steps": (C.c_int, [_P, C.c_int32]),
+    "cql_set_table_rows": (C.c_int, [_P, _P, C.c_int64]),
+    "cql_update_batch_rows": (C.c_int, [_P, _P, _P, _P, _P, _P]),
     "cql_mdp_begin": (C.c_int, [_P, C.c_int64]),
     "cql_mdp_append": (C.c_int, [_P, C.c_int32, C.c_int32, _P, C.c_int64]),
     "cql_mdp_finish": (C.c_int, [_P, C.c_int32, C.c_float, _P, _P, _P, _P, _P]),

@@ -384,7 +384,75 @@ void score_topk_dev_impl(cql_handle* ch, const int32_t* users, int64_t U, const 
   }
 }
 
+// n_steps > 1: a device buffer for the one-step rows a table producer writes before the n-step expansion
+// (finish_n_steps expands and frees it); n_steps == 1: the table itself
+float* one_step_rows(Handle& h, int64_t n) {
+  if (h.n_steps == 1) return h.table;
+  float* p = nullptr;
+  CQL_CUDA(cudaMalloc(&p, (size_t)n * 8 * sizeof(float)));
+  return p;
+}
+void finish_n_steps(Handle& h, float* one_step, int64_t n, cudaStream_t st) {
+  if (one_step == h.table) return;
+  expand_n_steps(h, one_step, n, st);
+  h.launches++;
+  CQL_CUDA(cudaStreamSynchronize(st));
+  CQL_CUDA(cudaFree(one_step));
+}
+
+// the host minibatch in h.batch_host -> one update (cql_update_batch, cql_update_batch_rows)
+void update_staged_batch(cql_handle* ch, const float* noise, float* metrics6, float* grads_out, cudaStream_t st) {
+  Handle& h = ch->h;
+  const int B = h.B;
+  if (noise) std::memcpy(h.noise_host, noise, h.noise_floats * sizeof(float));
+  // pinned staging -> device, the 26 launches of the step and the metrics read-back replay as ONE CUDA graph
+  // (26 runtime launches + 3 copies cost ~100 us of host time per step)
+  auto enqueue = [&] {
+    CQL_CUDA(cudaMemcpyAsync(h.batch, h.batch_host, (size_t)B * 8 * sizeof(float), cudaMemcpyHostToDevice, st));
+    if (noise) CQL_CUDA(cudaMemcpyAsync(h.noise, h.noise_host, h.noise_floats * sizeof(float), cudaMemcpyHostToDevice, st));
+    run_full_step(&h, st, BatchSource::Provided, noise ? NoiseSource::Provided : NoiseSource::Philox);
+    CQL_CUDA(cudaMemcpyAsync(h.metrics_host, h.metrics, 8 * sizeof(float), cudaMemcpyDeviceToHost, st));
+  };
+  const int gi = noise ? 1 : 0;
+  if (h.timing) {
+    enqueue();
+  } else {
+    if (!ch->batch_graph[gi] || ch->batch_graph_stream[gi] != st) {
+      if (ch->batch_graph[gi]) { cudaGraphExecDestroy(ch->batch_graph[gi]); ch->batch_graph[gi] = nullptr; }
+      cudaGraph_t g = nullptr;
+      const int64_t before = h.launches;
+      CQL_CUDA(cudaStreamBeginCapture(st, cudaStreamCaptureModeThreadLocal));
+      try {
+        enqueue();
+      } catch (...) {
+        cudaStreamEndCapture(st, &g);
+        if (g) cudaGraphDestroy(g);
+        throw;
+      }
+      CQL_CUDA(cudaStreamEndCapture(st, &g));
+      ch->batch_graph_launches[gi] = h.launches - before;
+      h.launches = before;
+      CQL_CUDA(cudaGraphInstantiate(&ch->batch_graph[gi], g, 0));
+      CQL_CUDA(cudaGraphDestroy(g));
+      ch->batch_graph_stream[gi] = st;
+    }
+    CQL_CUDA(cudaGraphLaunch(ch->batch_graph[gi], st));
+    h.launches += ch->batch_graph_launches[gi];
+  }
+  if (grads_out)
+    CQL_CUDA(cudaMemcpyAsync(grads_out, h.grads, grad_floats(h.C) * sizeof(float), cudaMemcpyDeviceToHost, st));
+  CQL_CUDA(cudaStreamSynchronize(st));
+  if (metrics6) std::memcpy(metrics6, h.metrics_host, 6 * sizeof(float));
+}
+
 }  // namespace
+
+void cql::expand_n_steps(Handle& h, const float* one_step, int64_t n, cudaStream_t st) {
+  const size_t smem = (size_t)(NSTEP_TILE + h.n_steps - 1) * 2 * sizeof(float4);
+  k_nstep_rows<<<(unsigned)((n + NSTEP_TILE - 1) / NSTEP_TILE), NSTEP_TILE, smem, st>>>(
+      reinterpret_cast<const float4*>(one_step), n, h.n_steps, (double)h.cfg.gamma, reinterpret_cast<float4*>(h.table));
+  CQL_CUDA(cudaGetLastError());
+}
 
 extern "C" {
 
@@ -485,6 +553,7 @@ int cql_load_transitions(cql_handle* ch, const float* obs, const float* act, con
     CQL_REQUIRE(obs && act && rew && term && n >= 1, "cql_load_transitions: bad arguments");
     CQL_CUDA(cudaDeviceSynchronize());
     ensure_table(h, n);
+    float* rows = one_step_rows(h, n);
     // stage the 20 B/step columns on the device, expand to 32 B rows there
     float *d_obs, *d_act, *d_rew, *d_term;
     CQL_CUDA(cudaMalloc(&d_obs, (size_t)n * 2 * sizeof(float)));
@@ -496,11 +565,36 @@ int cql_load_transitions(cql_handle* ch, const float* obs, const float* act, con
     CQL_CUDA(cudaMemcpyAsync(d_rew, rew, (size_t)n * sizeof(float), cudaMemcpyHostToDevice, st));
     CQL_CUDA(cudaMemcpyAsync(d_term, term, (size_t)n * sizeof(float), cudaMemcpyHostToDevice, st));
     k_build_transitions<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(reinterpret_cast<const float2*>(d_obs), d_act, d_rew,
-                                                                    d_term, n, reinterpret_cast<float4*>(h.table));
+                                                                    d_term, n, reinterpret_cast<float4*>(rows));
     CQL_LAUNCH_CHECK(&h);
+    finish_n_steps(h, rows, n, st);
     CQL_CUDA(cudaStreamSynchronize(st));
     CQL_CUDA(cudaFree(d_obs));
     CQL_CUDA(cudaFree(d_act));
+    h.n_trans = n;
+    destroy_graph(ch);
+  });
+}
+
+int cql_set_n_steps(cql_handle* ch, int32_t n_steps) {
+  return guarded(ch, [&] {
+    Handle& h = ch->h;
+    CQL_REQUIRE(n_steps >= 1 && n_steps <= CQL_MAX_N_STEPS, "cql_set_n_steps: n_steps must be 1..64 (CQL_MAX_N_STEPS)");
+    CQL_CUDA(cudaDeviceSynchronize());
+    if (n_steps != h.n_steps) h.n_trans = 0;         // the table was built for the other horizon
+    h.n_steps = n_steps;
+    destroy_graph(ch);
+  });
+}
+
+int cql_set_table_rows(cql_handle* ch, const float* rows, int64_t n) {
+  return guarded(ch, [&] {
+    Handle& h = ch->h;
+    CQL_REQUIRE(rows && n >= 1, "cql_set_table_rows: bad arguments");
+    CQL_CUDA(cudaDeviceSynchronize());
+    ensure_table(h, n);
+    CQL_CUDA(cudaMemcpyAsync(h.table, rows, (size_t)n * 8 * sizeof(float), cudaMemcpyHostToDevice, h.own_stream));
+    CQL_CUDA(cudaStreamSynchronize(h.own_stream));
     h.n_trans = n;
     destroy_graph(ch);
   });
@@ -538,8 +632,10 @@ int cql_synth_table(cql_handle* ch, int64_t n, int64_t n_users, int64_t n_items,
     CQL_REQUIRE(n_users < (1ll << 24) && n_items < (1ll << 24), "cql_synth_table: ids must stay below 2^24 (exact in float32)");
     CQL_CUDA(cudaDeviceSynchronize());
     ensure_table(h, n);
-    k_synth_table<<<(unsigned)((n + 255) / 256), 256, 0, h.own_stream>>>(reinterpret_cast<float4*>(h.table), n, n_users, n_items, seed);
+    float* rows = one_step_rows(h, n);
+    k_synth_table<<<(unsigned)((n + 255) / 256), 256, 0, h.own_stream>>>(reinterpret_cast<float4*>(rows), n, n_users, n_items, seed);
     CQL_LAUNCH_CHECK(&h);
+    finish_n_steps(h, rows, n, h.own_stream);
     CQL_CUDA(cudaStreamSynchronize(h.own_stream));
     h.n_trans = n;
     destroy_graph(ch);
@@ -719,50 +815,24 @@ int cql_update_batch(cql_handle* ch, const float* obs, const float* act, const f
     CQL_REQUIRE(obs && act && rew && next_obs && term, "cql_update_batch: NULL batch pointer");
     cudaStream_t st = pick_stream(&h, stream);
     const int B = h.B;
+    const float disc = h.n_steps > 1 ? h.cfg.gamma : 0.f;     // one-step transitions: discount gamma in n-step mode
     for (int b = 0; b < B; ++b) {
       float* r = h.batch_host + (size_t)b * 8;
       r[0] = obs[2 * b]; r[1] = obs[2 * b + 1]; r[2] = act[b]; r[3] = rew[b];
-      r[4] = next_obs[2 * b]; r[5] = next_obs[2 * b + 1]; r[6] = term[b]; r[7] = 0.f;
+      r[4] = next_obs[2 * b]; r[5] = next_obs[2 * b + 1]; r[6] = term[b]; r[7] = disc;
     }
-    if (noise) std::memcpy(h.noise_host, noise, h.noise_floats * sizeof(float));
-    // pinned staging -> device, the 26 launches of the step and the metrics read-back replay as ONE CUDA graph
-    // (26 runtime launches + 3 copies cost ~100 us of host time per step)
-    auto enqueue = [&] {
-      CQL_CUDA(cudaMemcpyAsync(h.batch, h.batch_host, (size_t)B * 8 * sizeof(float), cudaMemcpyHostToDevice, st));
-      if (noise) CQL_CUDA(cudaMemcpyAsync(h.noise, h.noise_host, h.noise_floats * sizeof(float), cudaMemcpyHostToDevice, st));
-      run_full_step(&h, st, BatchSource::Provided, noise ? NoiseSource::Provided : NoiseSource::Philox);
-      CQL_CUDA(cudaMemcpyAsync(h.metrics_host, h.metrics, 8 * sizeof(float), cudaMemcpyDeviceToHost, st));
-    };
-    const int gi = noise ? 1 : 0;
-    if (h.timing) {
-      enqueue();
-    } else {
-      if (!ch->batch_graph[gi] || ch->batch_graph_stream[gi] != st) {
-        if (ch->batch_graph[gi]) { cudaGraphExecDestroy(ch->batch_graph[gi]); ch->batch_graph[gi] = nullptr; }
-        cudaGraph_t g = nullptr;
-        const int64_t before = h.launches;
-        CQL_CUDA(cudaStreamBeginCapture(st, cudaStreamCaptureModeThreadLocal));
-        try {
-          enqueue();
-        } catch (...) {
-          cudaStreamEndCapture(st, &g);
-          if (g) cudaGraphDestroy(g);
-          throw;
-        }
-        CQL_CUDA(cudaStreamEndCapture(st, &g));
-        ch->batch_graph_launches[gi] = h.launches - before;
-        h.launches = before;
-        CQL_CUDA(cudaGraphInstantiate(&ch->batch_graph[gi], g, 0));
-        CQL_CUDA(cudaGraphDestroy(g));
-        ch->batch_graph_stream[gi] = st;
-      }
-      CQL_CUDA(cudaGraphLaunch(ch->batch_graph[gi], st));
-      h.launches += ch->batch_graph_launches[gi];
-    }
-    if (grads_out)
-      CQL_CUDA(cudaMemcpyAsync(grads_out, h.grads, grad_floats(h.C) * sizeof(float), cudaMemcpyDeviceToHost, st));
-    CQL_CUDA(cudaStreamSynchronize(st));
-    if (metrics6) std::memcpy(metrics6, h.metrics_host, 6 * sizeof(float));
+    update_staged_batch(ch, noise, metrics6, grads_out, st);
+  });
+}
+
+int cql_update_batch_rows(cql_handle* ch, const float* rows, const float* noise, float* metrics6, float* grads_out,
+                          void* stream) {
+  return guarded(ch, [&] {
+    Handle& h = ch->h;
+    CQL_REQUIRE(rows != nullptr, "cql_update_batch_rows: NULL rows");
+    cudaStream_t st = pick_stream(&h, stream);
+    std::memcpy(h.batch_host, rows, (size_t)h.B * 8 * sizeof(float));
+    update_staged_batch(ch, noise, metrics6, grads_out, st);
   });
 }
 
@@ -821,6 +891,7 @@ int cql_update_batches(cql_handle* ch, int64_t n_batches, const float* obs, cons
     // step paid both PCIe copies' start-up latency in series (e2e 0.885 of the HBM-resident rate).
     CQL_CUDA(cudaEventRecord(ch->ev_used[0], st));                        // orders the copy stream behind earlier work on st
     CQL_CUDA(cudaStreamWaitEvent(cs, ch->ev_used[0], 0));
+    const float disc = h.n_steps > 1 ? h.cfg.gamma : 0.f;     // one-step transitions: discount gamma in n-step mode
     for (int64_t i = 0; i < n_batches; ++i) {
       const int slot = (int)(i % RING);
       if (i >= RING) CQL_CUDA(cudaEventSynchronize(ch->ring_ev[slot]));     // that slot's host->device copy has run
@@ -830,7 +901,7 @@ int cql_update_batches(cql_handle* ch, int64_t n_batches, const float* obs, cons
       for (int b = 0; b < B; ++b) {
         float* w = stage + (size_t)b * 8;
         w[0] = o[2 * b]; w[1] = o[2 * b + 1]; w[2] = a[b]; w[3] = r[b];
-        w[4] = no[2 * b]; w[5] = no[2 * b + 1]; w[6] = t[b]; w[7] = 0.f;
+        w[4] = no[2 * b]; w[5] = no[2 * b + 1]; w[6] = t[b]; w[7] = disc;
       }
       float* dslot = ch->dev_ring + (size_t)slot * row_floats;
       if (i >= RING) CQL_CUDA(cudaStreamWaitEvent(cs, ch->ev_used[slot], 0));   // the device slot has been consumed
@@ -864,10 +935,11 @@ int cql_upload_batch(cql_handle* ch, const float* obs, const float* act, const f
     cudaStream_t st = pick_stream(&h, stream);
     const int B = h.B;
     CQL_CUDA(cudaStreamSynchronize(st));      // the staging buffer may still be in flight from the previous step
+    const float disc = h.n_steps > 1 ? h.cfg.gamma : 0.f;     // one-step transitions: discount gamma in n-step mode
     for (int b = 0; b < B; ++b) {
       float* r = h.batch_host + (size_t)b * 8;
       r[0] = obs[2 * b]; r[1] = obs[2 * b + 1]; r[2] = act[b]; r[3] = rew[b];
-      r[4] = next_obs[2 * b]; r[5] = next_obs[2 * b + 1]; r[6] = term[b]; r[7] = 0.f;
+      r[4] = next_obs[2 * b]; r[5] = next_obs[2 * b + 1]; r[6] = term[b]; r[7] = disc;
     }
     CQL_CUDA(cudaMemcpyAsync(h.batch, h.batch_host, (size_t)B * 8 * sizeof(float), cudaMemcpyHostToDevice, st));
   });

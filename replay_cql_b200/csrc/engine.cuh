@@ -51,8 +51,9 @@ struct Handle {
   float* metrics_host = nullptr;   // pinned
 
   // ---- replay table ----
-  float* table = nullptr;    // [n_trans][8]: obs.x obs.y act rew nobs.x nobs.y term pad
+  float* table = nullptr;    // [n_trans][8]: obs.x obs.y act rew nobs.x nobs.y term discount (0 when n_steps == 1)
   int64_t n_trans = 0;
+  int n_steps = 1;           // TD horizon of the tables built from now on and of the TD target (cql_set_n_steps)
   int64_t table_cap = 0;     // rows the table allocation can hold (re-ingesting a log of the same size re-uses it)
   bool table_sharded = false;   // data parallel: this rank holds only its own users' episodes (cql_set_table_sharded)
   int64_t sample_pos_host = 0;  // position in the epoch stream for the stand-alone sampler
@@ -174,6 +175,9 @@ inline void ensure_table(Handle& h, int64_t n) {
   CQL_CUDA(cudaMalloc(&h.table, (size_t)n * 8 * sizeof(float)));
   h.table_cap = n;
 }
+
+// n_steps > 1: one-step rows (device [n][8], not h.table) -> n-step rows in h.table, on `st` (capi.cu)
+void expand_n_steps(Handle& h, const float* one_step, int64_t n, cudaStream_t st);
 
 inline void mark(Handle* h, cudaStream_t st, int i) {
   if (h->timing) CQL_CUDA(cudaEventRecord(h->ev[i], st));

@@ -313,8 +313,10 @@ int64_t cql::mdp_finish(Handle& h, int top_k, float noise_scale, float* obs_out,
   k_rewarded<<<nb, 256, 0, st>>>(m.ib, gstart, n, top_k, m.rewarded);
   m.launches += 13;
 
-  // ---- emit transition rows straight into the replay table
+  // ---- emit transition rows straight into the replay table (n_steps > 1: into session scratch, expanded from there)
   ensure_table(h, n);
+  float4* rows = reinterpret_cast<float4*>(h.table);
+  if (h.n_steps > 1) rows = dmalloc<float4>(2 * (size_t)n, m.pool, m.alloc_stream);
   float *d_obs = nullptr, *d_act = nullptr, *d_rew = nullptr, *d_term = nullptr;
   if (obs_out) {
     CQL_REQUIRE(act_out && rew_out && term_out, "cql_build_mdp: give all four output columns or none");
@@ -322,9 +324,13 @@ int64_t cql::mdp_finish(Handle& h, int top_k, float noise_scale, float* obs_out,
     d_rew = dmalloc<float>(n, m.pool, m.alloc_stream); d_term = dmalloc<float>(n, m.pool, m.alloc_stream);
   }
   k_emit<<<nb, 256, 0, st>>>(m.order, m.user, m.item, m.rel, m.noise, m.rewarded, n, noise_scale, h.cfg.seed,
-                             reinterpret_cast<float4*>(h.table), d_obs, d_act, d_rew, d_term);
+                             rows, d_obs, d_act, d_rew, d_term);
   CQL_CUDA(cudaGetLastError());
   m.launches += 1;
+  if (h.n_steps > 1) {
+    expand_n_steps(h, reinterpret_cast<const float*>(rows), n, st);
+    m.launches += 1;
+  }
   if (obs_out) {
     CQL_CUDA(cudaMemcpyAsync(obs_out, d_obs, 2 * n * sizeof(float), cudaMemcpyDeviceToHost, st));
     CQL_CUDA(cudaMemcpyAsync(act_out, d_act, n * sizeof(float), cudaMemcpyDeviceToHost, st));

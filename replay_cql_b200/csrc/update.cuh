@@ -116,6 +116,35 @@ __global__ void k_synth_table(float4* __restrict__ table, int64_t n, int64_t n_u
   table[2 * i + 1] = make_float4(nx.x, nx.y, last ? 1.f : 0.f, 0.f);
 }
 
+// One-step rows -> n-step rows (d3rlpy n_steps, DESIGN.md section 1), out of place: row t reads rows t .. t + n_steps - 1.
+// k = min(n_steps, steps from t to its episode's end, t included); an episode ends at a terminal row or at the table's end.
+// R and the discount g are accumulated in float64 in the pinned order (R += g * r, then g *= gamma) with explicit
+// roundings, so k = 1 gives R = r and g = gamma exactly; s' and term are row t + k - 1's.  A block stages its
+// NSTEP_TILE rows plus the n_steps - 1 halo rows in shared memory with coalesced 16-byte loads, then each thread walks
+// its window there.
+constexpr int NSTEP_TILE = 256;
+__global__ void __launch_bounds__(NSTEP_TILE) k_nstep_rows(const float4* __restrict__ src, int64_t n, int n_steps,
+                                                           double gamma, float4* __restrict__ dst) {
+  extern __shared__ float4 tile[];           // [NSTEP_TILE + n_steps - 1][2]
+  const int64_t base = (int64_t)blockIdx.x * NSTEP_TILE;
+  const int rows = (int)min((int64_t)(NSTEP_TILE + n_steps - 1), n - base);
+  for (int q = threadIdx.x; q < 2 * rows; q += NSTEP_TILE) tile[q] = src[2 * base + q];
+  __syncthreads();
+  const int t = threadIdx.x;
+  if (base + t >= n) return;
+  double R = 0.0, g = 1.0;
+  int last = t;
+  for (int j = 0; j < n_steps && t + j < rows; ++j) {
+    last = t + j;
+    R = __dadd_rn(R, __dmul_rn(g, (double)tile[2 * last].w));
+    g = __dmul_rn(g, gamma);
+    if (tile[2 * last + 1].z != 0.f) break;
+  }
+  const float4 a = tile[2 * t], b = tile[2 * last + 1];
+  dst[2 * (base + t)] = make_float4(a.x, a.y, a.z, (float)R);
+  dst[2 * (base + t) + 1] = make_float4(b.x, b.y, b.z, (float)g);
+}
+
 // ---------------------------------------------------------------- noise (Philox)
 __global__ void k_noise(float* __restrict__ noise, int64_t total, int B, int n, uint64_t seed,
                         const long long* __restrict__ step_dev, int rank) {
@@ -329,6 +358,7 @@ __device__ __forceinline__ float lse_rows(const float* __restrict__ q, const flo
 struct LossConsts {
   int B, n, C;
   float gamma, cw, thr, temp_lr, alpha_lr, beta1, beta2, eps;
+  int nstep;               // 1: the rows carry their own TD discount in slot 7 (n_steps > 1), else gamma applies
 };
 
 // ---- loss glue, split so that nothing heavy runs in a single CTA -------------------------------
@@ -392,7 +422,8 @@ __global__ void __launch_bounds__(256) k_lse(const float4* __restrict__ batch, c
       float qt = q_at(srcT, 0, b);
       for (int c2 = 1; c2 < k.C; ++c2) qt = fminf(qt, q_at(srcT, c2, b));
       const float4 r0 = batch[2 * b], r1 = batch[2 * b + 1];
-      const float y = r0.w + k.gamma * qt * (1.f - r1.z);
+      const float disc = k.nstep ? r1.w : k.gamma;
+      const float y = r0.w + disc * qt * (1.f - r1.z);
       pv.qd = qd;
       pv.err = pv.qd - y;
       pairv[p] = pv;
@@ -1031,7 +1062,7 @@ inline void launch_bwd2(Handle* h, const BwdJob& jb, cudaStream_t st) {
 inline LossConsts loss_consts(const Handle* h) {
   const cql_config& c = h->cfg;
   return LossConsts{h->B, h->n, h->C, c.gamma, c.conservative_weight, c.alpha_threshold,
-                    c.temp_lr, c.alpha_lr, c.beta1, c.beta2, c.adam_eps};
+                    c.temp_lr, c.alpha_lr, c.beta1, c.beta2, c.adam_eps, h->n_steps > 1 ? 1 : 0};
 }
 
 constexpr int TIMED_FWD_REPS = 4;

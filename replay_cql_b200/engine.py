@@ -49,6 +49,7 @@ class CqlHyperParams:
     precision: str = "f16x3"   # tcgen05 fp16 hi/lo 3-term split, FP32-grade (1e-4 gates); "fp32" = CUDA-core FMA
     squash: str = "eps"
     seed: int = 12345
+    n_steps: int = 1           # n-step TD horizon of the replay table and the TD target (d3rlpy ``n_steps``)
 
 
 def _ptr(arr: Optional[np.ndarray]):
@@ -103,6 +104,8 @@ class CqlEngine:
         self.device, self.rank, self.world_size = device, rank, world_size
         self.n_state = int(self._lib.cql_state_floats(self._h))
         assert self.n_state == layout.state_floats(self.hp.n_critics)
+        if self.hp.n_steps != 1:
+            self._check(self._lib.cql_set_n_steps(self._h, int(self.hp.n_steps)), "cql_set_n_steps")
         self.set_state(layout.init_state(self.hp.n_critics, self.hp.seed, self.hp.initial_temperature,
                                          self.hp.initial_alpha))
 
@@ -164,6 +167,14 @@ class CqlEngine:
         act, rew, term = (_f32(np.reshape(a, -1), (n,)) for a in (act, rew, term))
         self._check(self._lib.cql_load_transitions(self._h, _ptr(obs), _ptr(act), _ptr(rew), _ptr(term), n),
                     "cql_load_transitions")
+
+    def set_table_rows(self, rows) -> None:
+        """Replay table uploaded verbatim from [n, 8] rows in the table's own format (``export_transitions`` output,
+        n-step rows included): no expansion."""
+        rows = _f32(rows)
+        if rows.ndim != 2 or rows.shape[1] != 8 or rows.shape[0] == 0:
+            raise ValueError("rows must be a non-empty [n, 8] array")
+        self._check(self._lib.cql_set_table_rows(self._h, _ptr(rows), rows.shape[0]), "cql_set_table_rows")
 
     def build_mdp_on_device(self, user_idx, item_idx, timestamp, relevance, top_k: int = 10,
                             action_randomization_scale: float = 1e-3, action_noise=None, want_outputs: bool = False):
@@ -234,7 +245,7 @@ class CqlEngine:
     def sample_rows(self, count: int, idx=None, pos: int = 0, out=None, stream: int | None = None):
         """Stand-alone replay gather (K1).  ``idx``: explicit int64 indices (numpy or cuda tensor) or
         None for the epoch permutation stream starting at ``pos``.  -> cuda tensor [count, 8]
-        rows ``(obs.x, obs.y, act, rew, next_obs.x, next_obs.y, term, 0)``."""
+        rows ``(obs.x, obs.y, act, rew, next_obs.x, next_obs.y, term, discount)`` (discount 0 when n_steps = 1)."""
         import torch
         dev = f"cuda:{self.device}"
         if out is None:
@@ -303,15 +314,28 @@ class CqlEngine:
 
     def update_batch(self, batch: Dict[str, np.ndarray], noise: Optional[Dict[str, np.ndarray]] = None,
                      want_grads: bool = False, stream: int | None = None):
-        """One update on a host minibatch (parity / end-to-end entry).  -> (metrics, grads|None)"""
+        """One update on a host minibatch (parity / end-to-end entry).  -> (metrics, grads|None)
+
+        ``batch["discount"]`` (optional, [B] or [B, 1]): each row's TD discount (gamma^k of an n-step row, see
+        ``cql_set_n_steps``) in place of gamma; needs ``n_steps > 1``.  ``rew`` is then the n-step return and
+        ``next_obs`` / ``term`` those of the window's last step."""
         B = self.hp.batch_size
         obs, nobs = _f32(batch["obs"], (B, 2)), _f32(batch["next_obs"], (B, 2))
         act, rew, term = (_f32(np.reshape(batch[k], -1), (B,)) for k in ("act", "rew", "term"))
         nz = self.pack_noise(noise) if noise is not None else None
         m = np.zeros(6, dtype=np.float32)
         g = np.zeros(layout.grad_floats(self.hp.n_critics), dtype=np.float32) if want_grads else None
-        self._check(self._lib.cql_update_batch(self._h, _ptr(obs), _ptr(act), _ptr(rew), _ptr(nobs), _ptr(term),
-                                               _ptr(nz), _ptr(m), _ptr(g), stream), "cql_update_batch")
+        if batch.get("discount") is not None:
+            if self.hp.n_steps == 1:
+                raise ValueError("batch['discount'] needs n_steps > 1 (with n_steps = 1 the TD discount is gamma)")
+            disc = _f32(np.reshape(batch["discount"], -1), (B,))
+            rows = np.ascontiguousarray(np.concatenate([obs, act[:, None], rew[:, None], nobs, term[:, None],
+                                                        disc[:, None]], axis=1))
+            self._check(self._lib.cql_update_batch_rows(self._h, _ptr(rows), _ptr(nz), _ptr(m), _ptr(g), stream),
+                        "cql_update_batch_rows")
+        else:
+            self._check(self._lib.cql_update_batch(self._h, _ptr(obs), _ptr(act), _ptr(rew), _ptr(nobs), _ptr(term),
+                                                   _ptr(nz), _ptr(m), _ptr(g), stream), "cql_update_batch")
         metrics = dict(zip(METRIC_NAMES, map(float, m)))
         return metrics, (layout.unpack_grads(g, self.hp.n_critics) if want_grads else None)
 

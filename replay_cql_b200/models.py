@@ -26,6 +26,11 @@ class CQL(Recommender):
     Observation = ``(user_idx, item_idx)``, action = ``relevance`` (one episode per user);
     relevance of a pair at predict time is ``mean_i Q_i(x, pi_greedy(x))`` (``score="q"``,
     d3rlpy ``predict_value(x, predict(x))``) or the greedy action itself (``score="policy"``).
+
+    ``n_steps`` (d3rlpy's name, default 1) is the TD horizon: each replay row carries the discounted reward sum of up to
+    ``n_steps`` steps of its user's episode and the TD target bootstraps from the state that many steps later with
+    discount ``gamma ** k`` (``k`` shorter where the episode ends first).  It is unrelated to ``resume(n_steps=...)`` and
+    ``engine.update(n_steps)``, which count update steps.
     """
 
     SHARD_ROWS = 200_000_000      # data-parallel fits shard the replay table by user range from this log size on
@@ -74,7 +79,11 @@ class CQL(Recommender):
         save_replay_table: bool = False,
         log_every: int = 1000,
         shard_table: Optional[bool] = None,
+        n_steps: int = 1,
     ):
+        from . import _lib
+        if not isinstance(n_steps, (int, np.integer)) or not 1 <= n_steps <= _lib.MAX_N_STEPS:
+            raise ValueError(f"n_steps (the n-step TD horizon) must be an integer in 1..{_lib.MAX_N_STEPS}")
         if soft_q_backup:
             raise ValueError("soft_q_backup=True is not supported (d3rlpy default False is restated)")
         if not use_gpu:
@@ -109,6 +118,7 @@ class CQL(Recommender):
         self.save_replay_table = save_replay_table
         self.log_every = log_every
         self.shard_table = shard_table
+        self.n_steps = int(n_steps)
         self.engine: Optional[CqlEngine] = None
         self.last_metrics: Optional[Dict[str, float]] = None
 
@@ -141,6 +151,7 @@ class CQL(Recommender):
             "save_replay_table": self.save_replay_table,
             "log_every": self.log_every,
             "shard_table": self.shard_table,
+            "n_steps": self.n_steps,
         }
 
     # ------------------------------------------------------------------ engine
@@ -151,7 +162,7 @@ class CQL(Recommender):
             temp_lr=self.temp_learning_rate, alpha_lr=self.alpha_learning_rate,
             initial_temperature=self.initial_temperature, initial_alpha=self.initial_alpha,
             alpha_threshold=self.alpha_threshold, conservative_weight=self.conservative_weight,
-            precision=self.precision, squash=self.squash, seed=self.seed,
+            precision=self.precision, squash=self.squash, seed=self.seed, n_steps=self.n_steps,
         )
 
     def _make_engine(self) -> CqlEngine:
@@ -381,7 +392,7 @@ class CQL(Recommender):
         m, v, step = self.engine.get_optimizer()
         np.savez(os.path.join(path, "state.npz"), state=self.engine.get_state(), adam_m=m, adam_v=v)
         n_rows = self.engine.n_transitions if self.save_replay_table else 0
-        if n_rows:                                          # [n, 8] rows: obs.x obs.y act rew next.x next.y term pad
+        if n_rows:                                          # [n, 8] rows: obs.x obs.y act rew next.x next.y term discount
             np.save(os.path.join(path, "replay_table.npy"), self.engine.export_transitions())
         with open(os.path.join(path, "meta.json"), "w") as f:
             json.dump({"fitted": True, "step": step, "format": 2, "replay_rows": int(n_rows)}, f)
@@ -396,5 +407,5 @@ class CQL(Recommender):
         eng.set_state(data["state"])
         eng.set_optimizer(data["adam_m"], data["adam_v"], int(meta["step"]))
         if meta.get("replay_rows"):
-            rows = np.load(os.path.join(path, "replay_table.npy"))
-            eng.load_transitions(rows[:, 0:2], rows[:, 2], rows[:, 3], rows[:, 6])
+            # verbatim: n-step rows cannot be rebuilt from their columns, and one-step rows come back bit for bit
+            eng.set_table_rows(np.load(os.path.join(path, "replay_table.npy")))
