@@ -138,6 +138,38 @@ int  cql_set_n_steps(cql_handle* h, int32_t n_steps);
 /* Replay table uploaded verbatim from rows_host [n][8] in the table's own format (e.g. cql_sample_rows / a checkpoint
  * of this handle's table): no expansion, whatever n_steps is. */
 int  cql_set_table_rows(cql_handle* h, const float* rows_host, int64_t n);
+/* Column statistics of the loaded table (d3rlpy's scaler fit, DESIGN.md section 1): every table producer
+ * (cql_build_mdp, cql_mdp_finish, cql_load_transitions, cql_synth_table, cql_set_table_rows) reduces the one-step rows
+ * it builds -- before any n-step expansion -- to count, min, max, mean and M2 = sum (x - mean)^2 per column, in float64
+ * and in a fixed order that depends only on the row count: the same steps give the same bits whichever producer built
+ * them.  col[]: 0 obs.x (user), 1 obs.y (item), 2 act, 3 rew.  cql_set_table_rows with n_steps > 1 sees n-step
+ * returns in the reward slot: rew_available = 0 there (and 0 when no table is loaded). */
+typedef struct cql_column_stats { int64_t count; double min, max, mean, m2; } cql_column_stats;
+typedef struct cql_table_stats {
+  cql_column_stats col[4];
+  int32_t rew_available;
+  int32_t pad;
+} cql_table_stats;
+int  cql_get_table_stats(cql_handle* h, cql_table_stats* out);
+/* d3rlpy's observation / action / reward scalers (scaler, action_scaler, reward_scaler; DESIGN.md section 1), applied
+ * to every minibatch as the update gathers it (s and s', a, r; the table stays raw) and to the (user, item)
+ * observations of the scorers; CQL_SCORE_POLICY returns the reverse action transform of tanh(mu(x')).  All float32,
+ * each operation rounded separately:
+ *   min_max (obs, rew): x' = (x - a) / (b - a)              a = minimum, b = maximum, (b - a) rounded once
+ *   standard (obs, rew): x' = (x - a) / (b + 1e-3)          a = mean, b = std, (b + 1e-3) rounded once
+ *   min_max (act): a' = ((a - min) / (max - min)) * 2 - 1;  reverse ((a' + 1) / 2) * (max - min) + min
+ * Observation parameters are per dimension (user, item).  Kinds: obs and rew NONE / MIN_MAX / STANDARD, act NONE /
+ * MIN_MAX; a min_max column needs max > min, a standard one std >= 0.  Captured update graphs are destroyed when the
+ * parameters change.  A staged minibatch (cql_upload_batch) stays raw: phase 4 scales it on every run.  All kinds NONE (the default) leaves every kernel on its unscaled path. */
+enum { CQL_SCALER_NONE = 0, CQL_SCALER_MIN_MAX = 1, CQL_SCALER_STANDARD = 2 };
+typedef struct cql_preprocessing {
+  int32_t obs_kind, act_kind, rew_kind, pad;
+  float obs_a[2], obs_b[2];     /* per dimension: min_max (minimum, maximum), standard (mean, std) */
+  float act_a, act_b;
+  float rew_a, rew_b;
+} cql_preprocessing;
+int  cql_set_preprocessing(cql_handle* h, const cql_preprocessing* p);
+int  cql_get_preprocessing(cql_handle* h, cql_preprocessing* out);
 /* stand-alone gather for the K1 roofline sweep: out_dev [count][8] floats.
  * idx_dev NULL => the handle's epoch permutation starting at position `pos`. */
 int  cql_sample_rows(cql_handle* h, const int64_t* idx_dev, int64_t pos, int64_t count,

@@ -21,6 +21,7 @@ BUF_SCALAR_GRADS, BUF_CRITIC_GRADS, BUF_ACTOR_GRADS, BUF_METRICS, BUF_PARAMS, BU
 MAX_TOPK = 1024
 MAX_N_STEPS = 64                                     # CQL_MAX_N_STEPS: longest n-step TD horizon
 DT_I32, DT_I64, DT_F32, DT_F64 = 0, 1, 2, 3          # cql_mdp_append chunk dtypes
+SCALER_NONE, SCALER_MIN_MAX, SCALER_STANDARD = 0, 1, 2   # cql_preprocessing kinds
 
 
 class CqlConfig(C.Structure):
@@ -36,6 +37,28 @@ class CqlConfig(C.Structure):
         ("alpha_threshold", C.c_float), ("conservative_weight", C.c_float),
         ("beta1", C.c_float), ("beta2", C.c_float), ("adam_eps", C.c_float),
         ("seed", C.c_uint64),
+    ]
+
+
+class ColumnStats(C.Structure):
+    """Mirror of ``struct cql_column_stats``."""
+
+    _fields_ = [("count", C.c_int64), ("min", C.c_double), ("max", C.c_double), ("mean", C.c_double), ("m2", C.c_double)]
+
+
+class TableStats(C.Structure):
+    """Mirror of ``struct cql_table_stats``: col = obs.x, obs.y, act, rew."""
+
+    _fields_ = [("col", ColumnStats * 4), ("rew_available", C.c_int32), ("pad", C.c_int32)]
+
+
+class Preprocessing(C.Structure):
+    """Mirror of ``struct cql_preprocessing``."""
+
+    _fields_ = [
+        ("obs_kind", C.c_int32), ("act_kind", C.c_int32), ("rew_kind", C.c_int32), ("pad", C.c_int32),
+        ("obs_a", C.c_float * 2), ("obs_b", C.c_float * 2),
+        ("act_a", C.c_float), ("act_b", C.c_float), ("rew_a", C.c_float), ("rew_b", C.c_float),
     ]
 
 
@@ -82,6 +105,9 @@ SIGNATURES = {
     "cql_set_n_steps": (C.c_int, [_P, C.c_int32]),
     "cql_set_table_rows": (C.c_int, [_P, _P, C.c_int64]),
     "cql_update_batch_rows": (C.c_int, [_P, _P, _P, _P, _P, _P]),
+    "cql_get_table_stats": (C.c_int, [_P, C.POINTER(TableStats)]),
+    "cql_set_preprocessing": (C.c_int, [_P, C.POINTER(Preprocessing)]),
+    "cql_get_preprocessing": (C.c_int, [_P, C.POINTER(Preprocessing)]),
     "cql_mdp_begin": (C.c_int, [_P, C.c_int64]),
     "cql_mdp_append": (C.c_int, [_P, C.c_int32, C.c_int32, _P, C.c_int64]),
     "cql_mdp_finish": (C.c_int, [_P, C.c_int32, C.c_float, _P, _P, _P, _P, _P]),

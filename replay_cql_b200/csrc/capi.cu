@@ -1,4 +1,5 @@
 // capi.cu -- the extern "C" surface declared in include/cql_b200.h.
+#include <cmath>
 #include <cstring>
 #include <cstdio>
 #include <algorithm>
@@ -168,8 +169,11 @@ void create_impl(const cql_config* cfg, cql_handle* ch) {
   h.sample_pos = h.dalloc<long long>(1);
   h.stepinfo = h.dalloc<StepInfo>(1);
   h.metrics = h.dalloc<float>(8);
+  h.stats_dev = h.dalloc<double>(STATS_DEV_DOUBLES);
+  CQL_CUDA(cudaMallocHost(&h.stats_host, 4 * 5 * sizeof(double)));
   CQL_CUDA(cudaMallocHost(&h.metrics_host, 8 * sizeof(float)));
   h.batch = h.dalloc<float>((size_t)B * 8);
+  h.batch_in = h.dalloc<float>((size_t)B * 8);
   CQL_CUDA(cudaMallocHost(&h.batch_host, (size_t)B * 8 * sizeof(float)));
   h.noise_floats = 2 * (int64_t)B + 6 * (int64_t)B * n;
   h.noise = h.dalloc<float>(h.noise_floats);
@@ -273,6 +277,17 @@ void run_full_step(Handle* h, cudaStream_t st, BatchSource bs, NoiseSource ns) {
   phase3(h, st);
 }
 
+// obs scaler on: the candidate items' scaled coordinates (k_scale_items) in scratch slot 7; off: nullptr (the scorers
+// convert the ids themselves, as without preprocessing)
+const float* scaled_items(cql_handle* ch, const int32_t* items, int64_t I, cudaStream_t st) {
+  Handle* h = &ch->h;
+  if (!h->prep.obs[1].on) return nullptr;
+  float* out = static_cast<float*>(scratch(ch, 7, (size_t)I * sizeof(float)));
+  k_scale_items<<<(unsigned)((I + 255) / 256), 256, 0, st>>>(items, I, h->prep.obs[1], out);
+  CQL_LAUNCH_CHECK(h);
+  return out;
+}
+
 void score_topk_dev_impl(cql_handle* ch, const int32_t* users, int64_t U, const int32_t* items, int64_t I,
                          const int64_t* seen_indptr, const int32_t* seen_items, int k, int mode, int32_t* out_items,
                          float* out_scores, cudaStream_t st) {
@@ -326,7 +341,8 @@ void score_topk_dev_impl(cql_handle* ch, const int32_t* users, int64_t U, const 
       ps = ch->part_s;
       pi = ch->part_i;
     }
-    tc::ScoreTcArgs a{h->params, ch->packed_score, users, items, seen_indptr, seen_items, U, I, h->C, k, mode, chunks, ps, pi};
+    tc::ScoreTcArgs a{h->params, ch->packed_score, users, items, seen_indptr, seen_items, U, I, h->C, k, mode, chunks, ps, pi,
+                      scaled_items(ch, items, I, st), h->prep};
     const int64_t n_blocks = U * chunks;
     const int grid = (int)std::min<int64_t>(n_blocks, h->num_sms);
     if (f16) tc::tc_score_h_kernel<<<grid, tc::HCfg4::THREADS, tc::ScoreSmemH::bytes(k), st>>>(a);
@@ -350,6 +366,8 @@ void score_topk_dev_impl(cql_handle* ch, const int32_t* users, int64_t U, const 
   a.params = h->params; a.users = users; a.items = items;
   a.seen_indptr = seen_indptr; a.seen_items = seen_items;
   a.n_users = U; a.n_items = I; a.C = h->C; a.k = k; a.mode = mode; a.chunks = chunks; a.tiles_per_chunk = tpc;
+  a.item_x = scaled_items(ch, items, I, st);
+  a.prep = h->prep;
   // users go on grid.y (max 65535): process in slabs
   const int64_t slab = 65535;
   for (int64_t u0 = 0; u0 < U; u0 += slab) {
@@ -408,7 +426,7 @@ void update_staged_batch(cql_handle* ch, const float* noise, float* metrics6, fl
   // pinned staging -> device, the 26 launches of the step and the metrics read-back replay as ONE CUDA graph
   // (26 runtime launches + 3 copies cost ~100 us of host time per step)
   auto enqueue = [&] {
-    CQL_CUDA(cudaMemcpyAsync(h.batch, h.batch_host, (size_t)B * 8 * sizeof(float), cudaMemcpyHostToDevice, st));
+    CQL_CUDA(cudaMemcpyAsync(h.staged_batch(), h.batch_host, (size_t)B * 8 * sizeof(float), cudaMemcpyHostToDevice, st));
     if (noise) CQL_CUDA(cudaMemcpyAsync(h.noise, h.noise_host, h.noise_floats * sizeof(float), cudaMemcpyHostToDevice, st));
     run_full_step(&h, st, BatchSource::Provided, noise ? NoiseSource::Provided : NoiseSource::Philox);
     CQL_CUDA(cudaMemcpyAsync(h.metrics_host, h.metrics, 8 * sizeof(float), cudaMemcpyDeviceToHost, st));
@@ -452,6 +470,21 @@ void cql::expand_n_steps(Handle& h, const float* one_step, int64_t n, cudaStream
   k_nstep_rows<<<(unsigned)((n + NSTEP_TILE - 1) / NSTEP_TILE), NSTEP_TILE, smem, st>>>(
       reinterpret_cast<const float4*>(one_step), n, h.n_steps, (double)h.cfg.gamma, reinterpret_cast<float4*>(h.table));
   CQL_CUDA(cudaGetLastError());
+}
+
+int cql::table_stats(Handle& h, const float* rows, int64_t n, bool rew_ok, cudaStream_t st) {
+  const int64_t nb = std::min<int64_t>((n + STATS_ROWS - 1) / STATS_ROWS, STATS_MAX_BLOCKS);
+  const int64_t per_block = (n + nb - 1) / nb;
+  Moments* part = reinterpret_cast<Moments*>(h.stats_dev);
+  k_stats_partial<<<(unsigned)nb, STATS_THREADS, 0, st>>>(reinterpret_cast<const float4*>(rows), n, per_block, part);
+  CQL_CUDA(cudaGetLastError());
+  Moments* result = part + 4 * STATS_MAX_BLOCKS;
+  k_stats_final<<<1, STATS_THREADS, 0, st>>>(part, nb, result);
+  CQL_CUDA(cudaGetLastError());
+  CQL_CUDA(cudaMemcpyAsync(h.stats_host, result, 4 * sizeof(Moments), cudaMemcpyDeviceToHost, st));
+  h.stats_pending = true;
+  h.stats_rew_ok = rew_ok;
+  return 2;
 }
 
 extern "C" {
@@ -567,6 +600,7 @@ int cql_load_transitions(cql_handle* ch, const float* obs, const float* act, con
     k_build_transitions<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(reinterpret_cast<const float2*>(d_obs), d_act, d_rew,
                                                                     d_term, n, reinterpret_cast<float4*>(rows));
     CQL_LAUNCH_CHECK(&h);
+    h.launches += table_stats(h, rows, n, true, st);
     finish_n_steps(h, rows, n, st);
     CQL_CUDA(cudaStreamSynchronize(st));
     CQL_CUDA(cudaFree(d_obs));
@@ -594,9 +628,69 @@ int cql_set_table_rows(cql_handle* ch, const float* rows, int64_t n) {
     CQL_CUDA(cudaDeviceSynchronize());
     ensure_table(h, n);
     CQL_CUDA(cudaMemcpyAsync(h.table, rows, (size_t)n * 8 * sizeof(float), cudaMemcpyHostToDevice, h.own_stream));
+    h.launches += table_stats(h, h.table, n, h.n_steps == 1, h.own_stream);   // n-step rows: returns in the reward slot
     CQL_CUDA(cudaStreamSynchronize(h.own_stream));
     h.n_trans = n;
     destroy_graph(ch);
+  });
+}
+
+int cql_get_table_stats(cql_handle* ch, cql_table_stats* out) {
+  return guarded(ch, [&] {
+    CQL_REQUIRE(out != nullptr, "cql_get_table_stats: NULL output");
+    Handle& h = ch->h;
+    if (h.stats_pending) {            // the producer's asynchronous copy: every producer synchronises before returning
+      CQL_CUDA(cudaDeviceSynchronize());
+      const double* m = h.stats_host;   // per column: n, mean, m2, min, max (struct Moments)
+      for (int c = 0; c < 4; ++c)
+        h.stats.col[c] = cql_column_stats{(int64_t)m[5 * c], m[5 * c + 3], m[5 * c + 4], m[5 * c + 1], m[5 * c + 2]};
+      h.stats.rew_available = h.stats_rew_ok ? 1 : 0;
+      if (!h.stats_rew_ok) h.stats.col[3] = cql_column_stats{};
+      h.stats_pending = false;
+    }
+    *out = h.n_trans > 0 ? h.stats : cql_table_stats{};
+  });
+}
+
+int cql_set_preprocessing(cql_handle* ch, const cql_preprocessing* p) {
+  return guarded(ch, [&] {
+    Handle& h = ch->h;
+    CQL_REQUIRE(p != nullptr, "cql_set_preprocessing: NULL parameters");
+    const cql_preprocessing& c = *p;
+    CQL_REQUIRE(c.obs_kind >= CQL_SCALER_NONE && c.obs_kind <= CQL_SCALER_STANDARD, "cql_set_preprocessing: bad obs_kind");
+    CQL_REQUIRE(c.act_kind == CQL_SCALER_NONE || c.act_kind == CQL_SCALER_MIN_MAX,
+                "cql_set_preprocessing: act_kind must be NONE or MIN_MAX");
+    CQL_REQUIRE(c.rew_kind >= CQL_SCALER_NONE && c.rew_kind <= CQL_SCALER_STANDARD, "cql_set_preprocessing: bad rew_kind");
+    // (a, b) of one column -> the kernels' (off, den): den = b - a (min_max) or b + 1e-3 (standard), rounded once
+    auto affine = [](int kind, float a, float b, const char* what) {
+      if (kind == CQL_SCALER_NONE) return Affine{0, 0.f, 1.f};
+      CQL_REQUIRE(std::isfinite(a) && std::isfinite(b), std::string("cql_set_preprocessing: non-finite parameter of ") + what);
+      if (kind == CQL_SCALER_MIN_MAX) {
+        CQL_REQUIRE(b > a, std::string("cql_set_preprocessing: min_max needs maximum > minimum for ") + what);
+        const volatile float den = b - a;
+        return Affine{1, a, den};
+      }
+      CQL_REQUIRE(b >= 0.f, std::string("cql_set_preprocessing: standard needs std >= 0 for ") + what);
+      const volatile float den = b + 1e-3f;
+      return Affine{1, a, den};
+    };
+    Prep q{};
+    q.obs[0] = affine(c.obs_kind, c.obs_a[0], c.obs_b[0], "obs.x");
+    q.obs[1] = affine(c.obs_kind, c.obs_a[1], c.obs_b[1], "obs.y");
+    q.act = affine(c.act_kind, c.act_a, c.act_b, "act");
+    q.rew = affine(c.rew_kind, c.rew_a, c.rew_b, "rew");
+    CQL_CUDA(cudaDeviceSynchronize());
+    h.prep = q;
+    h.prep_cfg = c;
+    h.prep_cfg.pad = 0;
+    destroy_graph(ch);              // the parameters are kernel arguments of the captured graphs
+  });
+}
+
+int cql_get_preprocessing(cql_handle* ch, cql_preprocessing* out) {
+  return guarded(ch, [&] {
+    CQL_REQUIRE(out != nullptr, "cql_get_preprocessing: NULL output");
+    *out = ch->h.prep_cfg;
   });
 }
 
@@ -635,6 +729,7 @@ int cql_synth_table(cql_handle* ch, int64_t n, int64_t n_users, int64_t n_items,
     float* rows = one_step_rows(h, n);
     k_synth_table<<<(unsigned)((n + 255) / 256), 256, 0, h.own_stream>>>(reinterpret_cast<float4*>(rows), n, n_users, n_items, seed);
     CQL_LAUNCH_CHECK(&h);
+    h.launches += table_stats(h, rows, n, true, h.own_stream);
     finish_n_steps(h, rows, n, h.own_stream);
     CQL_CUDA(cudaStreamSynchronize(h.own_stream));
     h.n_trans = n;
@@ -908,7 +1003,7 @@ int cql_update_batches(cql_handle* ch, int64_t n_batches, const float* obs, cons
       CQL_CUDA(cudaMemcpyAsync(dslot, stage, row_floats * sizeof(float), cudaMemcpyHostToDevice, cs));
       CQL_CUDA(cudaEventRecord(ch->ring_ev[slot], cs));
       CQL_CUDA(cudaStreamWaitEvent(st, ch->ring_ev[slot], 0));
-      CQL_CUDA(cudaMemcpyAsync(h.batch, dslot, row_floats * sizeof(float), cudaMemcpyDeviceToDevice, st));
+      CQL_CUDA(cudaMemcpyAsync(h.staged_batch(), dslot, row_floats * sizeof(float), cudaMemcpyDeviceToDevice, st));
       CQL_CUDA(cudaEventRecord(ch->ev_used[slot], st));
       CQL_CUDA(cudaGraphLaunch(ch->step_graph, st));
       h.launches += ch->step_graph_launches;
@@ -941,7 +1036,7 @@ int cql_upload_batch(cql_handle* ch, const float* obs, const float* act, const f
       r[0] = obs[2 * b]; r[1] = obs[2 * b + 1]; r[2] = act[b]; r[3] = rew[b];
       r[4] = next_obs[2 * b]; r[5] = next_obs[2 * b + 1]; r[6] = term[b]; r[7] = disc;
     }
-    CQL_CUDA(cudaMemcpyAsync(h.batch, h.batch_host, (size_t)B * 8 * sizeof(float), cudaMemcpyHostToDevice, st));
+    CQL_CUDA(cudaMemcpyAsync(h.staged_batch(), h.batch_host, (size_t)B * 8 * sizeof(float), cudaMemcpyHostToDevice, st));
   });
 }
 
@@ -1111,7 +1206,7 @@ int cql_score_pairs(cql_handle* ch, const int32_t* users, const int32_t* items, 
     float* d_o = (float*)scratch(ch, 3, (size_t)n * 4);
     CQL_CUDA(cudaMemcpyAsync(d_u, users, (size_t)n * 4, cudaMemcpyHostToDevice, st));
     CQL_CUDA(cudaMemcpyAsync(d_i, items, (size_t)n * 4, cudaMemcpyHostToDevice, st));
-    k_score_pairs<<<(unsigned)((n + BM - 1) / BM), NT, FWD_SMEM, st>>>(h.params, d_u, d_i, n, h.C, mode, d_o);
+    k_score_pairs<<<(unsigned)((n + BM - 1) / BM), NT, FWD_SMEM, st>>>(h.params, d_u, d_i, n, h.C, mode, d_o, h.prep);
     CQL_LAUNCH_CHECK(&h);
     CQL_CUDA(cudaMemcpyAsync(out_scores, d_o, (size_t)n * 4, cudaMemcpyDeviceToHost, st));
     CQL_CUDA(cudaStreamSynchronize(st));

@@ -25,6 +25,39 @@ struct NvtxRange {
   NvtxRange& operator=(const NvtxRange&) = delete;
 };
 
+// d3rlpy's scalers as the kernels apply them (cql_set_preprocessing, DESIGN.md section 1): x' = (x - off) / den with
+// den = max - min or std + 1e-3 already rounded on the host; every operation rounded separately (no FMA contraction).
+// on == 0: the value passes untouched.  Passed by value: a change destroys the captured graphs.
+struct Affine {
+  int on;
+  float off, den;
+};
+struct Prep {
+  Affine obs[2];   // user, item
+  Affine act;      // min_max: off = min, den = max - min; forward maps onto [-1, 1]
+  Affine rew;
+  __host__ __device__ bool any() const { return obs[0].on | obs[1].on | act.on | rew.on; }
+};
+__device__ __forceinline__ float prep_fwd(const Affine& p, float x) {
+  return p.on ? __fdiv_rn(__fsub_rn(x, p.off), p.den) : x;
+}
+__device__ __forceinline__ float act_fwd(const Affine& p, float a) {
+  return p.on ? __fsub_rn(__fmul_rn(__fdiv_rn(__fsub_rn(a, p.off), p.den), 2.f), 1.f) : a;
+}
+__device__ __forceinline__ float act_rev(const Affine& p, float a) {
+  return p.on ? __fadd_rn(__fmul_rn(__fdiv_rn(__fadd_rn(a, 1.f), 2.f), p.den), p.off) : a;
+}
+// transition row (s.x s.y a r | s'.x s'.y term discount) in the network's coordinates; term and discount untouched
+__device__ __forceinline__ float4 prep_row0(const Prep& p, float4 r) {
+  return make_float4(prep_fwd(p.obs[0], r.x), prep_fwd(p.obs[1], r.y), act_fwd(p.act, r.z), prep_fwd(p.rew, r.w));
+}
+__device__ __forceinline__ float4 prep_row1(const Prep& p, float4 r) {
+  return make_float4(prep_fwd(p.obs[0], r.x), prep_fwd(p.obs[1], r.y), r.z, r.w);
+}
+
+constexpr int STATS_MAX_BLOCKS = 1024;                               // table_stats (update.cuh)
+constexpr size_t STATS_DEV_DOUBLES = (STATS_MAX_BLOCKS + 1) * 4 * 5;
+
 struct MdpSession;                   // chunked ingestion session (mdp_gpu.cu)
 // seen-items CSR of a log on the device (mdp_gpu.cu); returns the number of (user, item) entries written
 int64_t seen_csr_on_device(struct Handle& h, const int32_t* users_h, const int32_t* items_h, int64_t n, int64_t n_users,
@@ -58,12 +91,21 @@ struct Handle {
   bool table_sharded = false;   // data parallel: this rank holds only its own users' episodes (cql_set_table_sharded)
   int64_t sample_pos_host = 0;  // position in the epoch stream for the stand-alone sampler
   long long* sample_pos = nullptr;   // device: next position in the permutation stream
+  cql_table_stats stats{};   // column statistics of the table's one-step rows (table_stats; filled from stats_host)
+  double* stats_dev = nullptr;    // [STATS_DEV_DOUBLES] k_stats_partial / k_stats_final partials and result
+  double* stats_host = nullptr;   // pinned [4][5]: the result (count, mean, m2, min, max per column), copied async
+  bool stats_pending = false;     // stats_host holds the current table's statistics, not yet moved into `stats`
+  bool stats_rew_ok = false;
+  cql_preprocessing prep_cfg{};   // as given to cql_set_preprocessing
+  Prep prep{};               // ... as the kernels apply it
 
   // ---- per-step scratch (B = batch, n = action samples, C = critics) ----
   int B = 0, n = 0, C = 0;
   int rsA = 0, rsC = 0;      // rows per batch element: alpha job (3n), critic job (3n+1)
   float* batch = nullptr;    // [B][8] sampled transition rows (same row format as table)
   float* batch_host = nullptr;   // pinned staging for cql_update_batch
+  float* batch_in = nullptr;     // [B][8] the provided / k_sample minibatch as staged, when preprocessing is on
+                                 // (k_actor_rows writes its scaled rows to `batch`; the staged rows stay raw)
   float* noise = nullptr;    // packed, see header
   float* noise_host = nullptr;
   int64_t noise_floats = 0;
@@ -145,6 +187,7 @@ struct Handle {
     if (table) { cudaFree(table); table = nullptr; table_cap = 0; }
     if (metrics_host) { cudaFreeHost(metrics_host); metrics_host = nullptr; }
     if (batch_host) { cudaFreeHost(batch_host); batch_host = nullptr; }
+    if (stats_host) { cudaFreeHost(stats_host); stats_host = nullptr; }
     if (noise_host) { cudaFreeHost(noise_host); noise_host = nullptr; }
     if (own_stream) { cudaStreamDestroy(own_stream); own_stream = nullptr; }
     if (side_stream) { cudaStreamDestroy(side_stream); side_stream = nullptr; }
@@ -153,6 +196,9 @@ struct Handle {
     for (auto& e : ev) if (e) { cudaEventDestroy(e); e = nullptr; }
   }
 
+  // where a minibatch is staged before k_actor_rows: `batch` itself without preprocessing, else batch_in (the captured
+  // graphs bake this address in; cql_set_preprocessing destroys them)
+  float* staged_batch() const { return prep.any() ? batch_in : batch; }
   float* net_params(int slot) const { return params + (size_t)slot * NET_STRIDE; }
   float* scalars() const { return params + scalars_off(C); }
   // grads buffer parts
@@ -170,6 +216,8 @@ int64_t mdp_finish(Handle& h, int top_k, float noise_scale, float* obs_out, floa
 // ingestion synchronises the device and costs milliseconds to tens of milliseconds)
 inline void ensure_table(Handle& h, int64_t n) {
   h.n_trans = 0;
+  h.stats = cql_table_stats{};
+  h.stats_pending = false;
   if (h.table != nullptr && h.table_cap >= n) return;
   if (h.table) { CQL_CUDA(cudaFree(h.table)); h.table = nullptr; h.table_cap = 0; }
   CQL_CUDA(cudaMalloc(&h.table, (size_t)n * 8 * sizeof(float)));
@@ -178,6 +226,10 @@ inline void ensure_table(Handle& h, int64_t n) {
 
 // n_steps > 1: one-step rows (device [n][8], not h.table) -> n-step rows in h.table, on `st` (capi.cu)
 void expand_n_steps(Handle& h, const float* one_step, int64_t n, cudaStream_t st);
+// column statistics of one-step rows (device [n][8]), enqueued on `st` into the handle's buffers (no allocation, no
+// synchronisation; cql_get_table_stats reads them).  rew_ok = false: the reward slot holds n-step returns, the reward
+// statistics are marked unavailable.  Returns the launches it made (capi.cu).
+int table_stats(Handle& h, const float* rows, int64_t n, bool rew_ok, cudaStream_t st);
 
 inline void mark(Handle* h, cudaStream_t st, int i) {
   if (h->timing) CQL_CUDA(cudaEventRecord(h->ev[i], st));

@@ -327,6 +327,7 @@ int64_t cql::mdp_finish(Handle& h, int top_k, float noise_scale, float* obs_out,
                              rows, d_obs, d_act, d_rew, d_term);
   CQL_CUDA(cudaGetLastError());
   m.launches += 1;
+  m.launches += table_stats(h, reinterpret_cast<const float*>(rows), n, true, st);
   if (h.n_steps > 1) {
     expand_n_steps(h, reinterpret_cast<const float*>(rows), n, st);
     m.launches += 1;

@@ -235,14 +235,23 @@ struct ScoreArgs {
   int C, k, mode, chunks, tiles_per_chunk;
   float* part_s;              // [U][chunks][k]
   int* part_i;
+  const float* item_x;        // [I] scaled item coordinates (obs scaler on), or nullptr: (float)item
+  Prep prep;                  // user coordinate and the policy score's reverse action transform
 };
 
 constexpr int SCORE_SMEM_BASE = FWD_SMEM;
 inline int score_smem(int k) { return SCORE_SMEM_BASE + k * 8 + BM * 8; }
 
+// obs scaler on: the scaled item coordinates of a candidate list, once per scoring call -- the tensor-core producers
+// would otherwise divide once per (user, item) pair
+__global__ void k_scale_items(const int32_t* __restrict__ items, int64_t n, const Affine f, float* __restrict__ out) {
+  const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i < n) out[i] = prep_fwd(f, (float)items[i]);
+}
+
 // relevance of the 64 rows in Xs (x = user, y = item); result in sc[r] (smem) after return
 __device__ __forceinline__ void score_tile(const float* __restrict__ params, int C, int mode, float4* Xs, float* As,
-                                           float* Bs, float* outs, float* sc) {
+                                           float* Bs, float* outs, float* sc, const Affine& act) {
   const int tid = threadIdx.x;
   fwd_tile<2, 2>(params + (size_t)slot_actor() * NET_STRIDE, Xs, As, Bs, outs, nullptr);
   float a = 0.f;
@@ -252,7 +261,7 @@ __device__ __forceinline__ void score_tile(const float* __restrict__ params, int
   }
   __syncthreads();
   if (mode == CQL_SCORE_POLICY) {
-    if (tid < BM) sc[tid] = a;
+    if (tid < BM) sc[tid] = act_rev(act, a);     // relevance in the data's action units
     __syncthreads();
     return;
   }
@@ -279,6 +288,7 @@ __global__ void __launch_bounds__(NT, 2) k_score_topk(const ScoreArgs a) {
   const int tid = threadIdx.x;
   const int64_t urow = blockIdx.y;
   const int user = a.users[urow];
+  const float uf = prep_fwd(a.prep.obs[0], (float)user);
   for (int e = tid; e < a.k; e += NT) { topS[e] = -INFINITY; topI[e] = -1; }
   int64_t lo = 0, hi = 0;
   if (a.seen_indptr) { lo = a.seen_indptr[user]; hi = a.seen_indptr[user + 1]; }
@@ -289,11 +299,11 @@ __global__ void __launch_bounds__(NT, 2) k_score_topk(const ScoreArgs a) {
     const int cnt = (int)min((int64_t)BM, a.n_items - i0);
     if (tid < BM) {
       const int item = tid < cnt ? a.items[i0 + tid] : -1;
-      Xs[tid] = make_float4((float)user, (float)max(item, 0), 0.f, 0.f);
+      Xs[tid] = make_float4(uf, a.item_x && tid < cnt ? a.item_x[i0 + tid] : (float)max(item, 0), 0.f, 0.f);
       ci[tid] = item;
     }
     __syncthreads();
-    score_tile(a.params, a.C, a.mode, Xs, As, Bs, outs, cs);
+    score_tile(a.params, a.C, a.mode, Xs, As, Bs, outs, cs, a.prep.act);
     if (tid < 32) warp_fold_tile(topS, topI, a.k, cs, ci, cnt, a.seen_indptr ? a.seen_items : nullptr, lo, hi);
     __syncthreads();
   }
@@ -329,7 +339,7 @@ __global__ void k_topk_merge(const float* __restrict__ part_s, const int* __rest
 // explicit (user,item) pairs -> relevance
 __global__ void __launch_bounds__(NT, 2) k_score_pairs(const float* __restrict__ params, const int32_t* __restrict__ users,
                                                        const int32_t* __restrict__ items, int64_t n, int C, int mode,
-                                                       float* __restrict__ out) {
+                                                       float* __restrict__ out, const Prep prep) {
   extern __shared__ __align__(16) float smem[];
   float* As = smem;
   float* Bs = As + H * BM;
@@ -340,10 +350,11 @@ __global__ void __launch_bounds__(NT, 2) k_score_pairs(const float* __restrict__
   const int64_t r0 = (int64_t)blockIdx.x * BM;
   if (tid < BM) {
     const int64_t r = r0 + tid;
-    Xs[tid] = r < n ? make_float4((float)users[r], (float)items[r], 0.f, 0.f) : make_float4(0.f, 0.f, 0.f, 0.f);
+    Xs[tid] = r < n ? make_float4(prep_fwd(prep.obs[0], (float)users[r]), prep_fwd(prep.obs[1], (float)items[r]), 0.f, 0.f)
+                    : make_float4(0.f, 0.f, 0.f, 0.f);
   }
   __syncthreads();
-  score_tile(params, C, mode, Xs, As, Bs, outs, sc);
+  score_tile(params, C, mode, Xs, As, Bs, outs, sc, prep.act);
   if (tid < BM && r0 + tid < n) out[r0 + tid] = sc[tid];
 }
 

@@ -28,7 +28,16 @@ struct ScoreTcArgs {
   int C, k, mode, chunks;     // chunks = blocks per user
   float* part_s;              // [U][chunks][k]
   int* part_i;
+  const float* item_x;        // [I] scaled item coordinates (obs scaler on), or nullptr: (float)item
+  Prep prep;                  // user coordinate (once per block) and the policy score's reverse action transform
 };
+// observation coordinates of a scored pair; the producers and the f16x3 epilogue's row-scale recomputation both come here
+__device__ __forceinline__ float score_user(const ScoreTcArgs& a, int64_t urow) {
+  return prep_fwd(a.prep.obs[0], (float)a.users[urow]);
+}
+__device__ __forceinline__ float score_item(const ScoreTcArgs& a, int64_t idx) {
+  return idx < a.n_items ? (a.item_x ? __ldg(a.item_x + idx) : (float)__ldg(a.items + idx)) : 0.f;
+}
 
 struct ScoreSmem : TsCfg {
   static constexpr uint32_t OFF_STA = OFF_SLOT + 16;                       // float[CH*128] greedy action
@@ -157,7 +166,7 @@ __global__ void __launch_bounds__(TsCfg::THREADS, 1) tc_score_kernel(const Score
     for (int64_t blk = blk_lo; blk < blk_hi; ++blk) {
       const int tb = tiles_of_block(blk);
       if (tb == 0) continue;
-      const float uf = (float)a.users[blk / a.chunks];
+      const float uf = score_user(a, blk / a.chunks);
       const int64_t i0 = (blk % a.chunks) * SC_CH * TM;
       for (int p = 0; p < n_pass; ++p) {
         const int net_i = p / C::SLICES;
@@ -177,7 +186,7 @@ __global__ void __launch_bounds__(TsCfg::THREADS, 1) tc_score_kernel(const Score
         }
         for (int t = 0; t < tb; ++t) {
           const int64_t idx = i0 + (int64_t)t * TM + row_in_tile;
-          const float itf = idx < a.n_items ? (float)__ldg(a.items + idx) : 0.f;
+          const float itf = score_item(a, idx);
           const float av = net_i == 0 ? 0.f : st_a[t * TM + row_in_tile];
           const float2 xx = make_float2(uf, uf), xy = make_float2(itf, itf), xz = make_float2(av, av);
           for (int c = 0; c < C::NCHUNK; ++c, ++it) {
@@ -272,7 +281,7 @@ __global__ void __launch_bounds__(TsCfg::THREADS, 1) tc_score_kernel(const Score
             if (net_i == 0 && slice == C::SLICES - 1) {
               const float act = tanhf(sum + b3mu);
               st_a[ridx] = act;
-              if (a.mode == CQL_SCORE_POLICY) score[ridx] = act;
+              if (a.mode == CQL_SCORE_POLICY) score[ridx] = act_rev(a.prep.act, act);
             } else if (net_i == a.C && slice == C::SLICES - 1) {
               score[ridx] = (sum + b3sum) / (float)a.C;
             }

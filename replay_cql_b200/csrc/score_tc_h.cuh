@@ -146,7 +146,7 @@ __global__ void __launch_bounds__(HCfg4::THREADS, 1) tc_score_h_kernel(const Sco
     for (int64_t blk = blk_lo; blk < blk_hi; ++blk) {
       const int tb = tiles_of_block(blk);
       if (tb == 0) continue;
-      const float uf = (float)a.users[blk / a.chunks];
+      const float uf = score_user(a, blk / a.chunks);
       const int64_t i0 = (blk % a.chunks) * SC_CH * TM;
       for (int p = 0; p < n_pass; ++p) {
         const int net_i = p / C::SLICES;
@@ -171,7 +171,7 @@ __global__ void __launch_bounds__(HCfg4::THREADS, 1) tc_score_h_kernel(const Sco
         }
         for (int t = 0; t < tb; ++t) {
           const int64_t idx = i0 + (int64_t)t * TM + row_in_tile;
-          const float itf = idx < a.n_items ? (float)__ldg(a.items + idx) : 0.f;
+          const float itf = score_item(a, idx);
           const float av = net_i == 0 ? 0.f : st_a[t * TM + row_in_tile];
           const float2 xx = make_float2(uf, uf), xy = make_float2(itf, itf), xz = make_float2(av, av);
           float sa, inv_sa;
@@ -220,7 +220,7 @@ __global__ void __launch_bounds__(HCfg4::THREADS, 1) tc_score_h_kernel(const Sco
         sv = stage_seen(a.seen_indptr, a.seen_items, a.users[urow], seen_cache, tid, 128);
       }
       asm volatile("bar.sync 2, 128;");
-      const float uf = (float)a.users[urow];
+      const float uf = score_user(a, urow);
       const int64_t i0e = (int64_t)chunk * SC_CH * TM;
       float4 wm = make_float4(0.f, 0.f, 0.f, 0.f);
       if (tb > 0) {
@@ -249,7 +249,7 @@ __global__ void __launch_bounds__(HCfg4::THREADS, 1) tc_score_h_kernel(const Sco
             // the producers' scale of this row, recomputed from the same inputs (greedy action for the critics)
             const int ridx0 = t * TM + row_in_tile;
             const int64_t iidx = i0e + ridx0;
-            const float itf = iidx < a.n_items ? (float)__ldg(a.items + iidx) : 0.f;
+            const float itf = score_item(a, iidx);
             float sa, inv_sa;
             pow2_scale(h1_row_bound(make_float4(uf, itf, net_i == 0 ? 0.f : st_a[ridx0], 0.f), wm), sa, inv_sa);
             mbar_wait(&tfull[acc], (tcount >> 1) & 1);
@@ -277,7 +277,7 @@ __global__ void __launch_bounds__(HCfg4::THREADS, 1) tc_score_h_kernel(const Sco
             if (net_i == 0 && slice == C::SLICES - 1) {
               const float act = tanhf(sum + b3mu);
               st_a[ridx] = act;
-              if (a.mode == CQL_SCORE_POLICY) score[ridx] = act;
+              if (a.mode == CQL_SCORE_POLICY) score[ridx] = act_rev(a.prep.act, act);
             } else if (net_i == a.C && slice == C::SLICES - 1) {
               score[ridx] = (sum + b3sum) / (float)a.C;
             }

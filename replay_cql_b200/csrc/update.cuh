@@ -145,6 +145,70 @@ __global__ void __launch_bounds__(NSTEP_TILE) k_nstep_rows(const float4* __restr
   dst[2 * (base + t) + 1] = make_float4(b.x, b.y, b.z, (float)g);
 }
 
+// Column statistics of one-step rows (d3rlpy's scaler fit, cql_get_table_stats): count, mean, M2, min, max of obs.x,
+// obs.y, act and rew in float64.  Each thread runs Welford's update over its rows (j = t, t + 256, ... of the block's
+// STATS_ROWS), the block merges its threads with Chan's formula in a fixed tree, and k_stats_final merges the block
+// partials the same way: the order depends only on n, so the same rows always give the same bits.
+struct Moments { double n, mean, m2, mn, mx; };
+__device__ __forceinline__ Moments mom_merge(Moments a, const Moments& b) {
+  if (b.n == 0.0) return a;
+  if (a.n == 0.0) return b;
+  const double n = a.n + b.n, d = b.mean - a.mean;
+  a.mean = a.mean + d * (b.n / n);
+  a.m2 = a.m2 + b.m2 + d * d * (a.n * b.n / n);
+  a.mn = fmin(a.mn, b.mn);
+  a.mx = fmax(a.mx, b.mx);
+  a.n = n;
+  return a;
+}
+constexpr int STATS_THREADS = 256, STATS_ROWS = 32 * STATS_THREADS;
+// blocks of k_stats_partial: ceil(n / STATS_ROWS), at most STATS_MAX_BLOCKS (then each takes ceil(n / blocks) rows); the
+// partials live in the handle's stats_dev, [(STATS_MAX_BLOCKS + 1) * 4] Moments (engine.cuh: STATS_DEV_DOUBLES)
+static_assert(sizeof(Moments) == 5 * sizeof(double), "Moments is five doubles");
+static_assert(STATS_DEV_DOUBLES == (STATS_MAX_BLOCKS + 1) * 4 * 5, "stats_dev holds the partials and the result");
+__device__ void stats_block_store(Moments (&m)[4], Moments* __restrict__ out) {
+  __shared__ Moments sm[STATS_THREADS];
+  for (int c = 0; c < 4; ++c) {
+    sm[threadIdx.x] = m[c];
+    __syncthreads();
+    for (int s = STATS_THREADS / 2; s > 0; s >>= 1) {
+      if (threadIdx.x < s) sm[threadIdx.x] = mom_merge(sm[threadIdx.x], sm[threadIdx.x + s]);
+      __syncthreads();
+    }
+    if (threadIdx.x == 0) out[c] = sm[0];
+    __syncthreads();
+  }
+}
+__global__ void __launch_bounds__(STATS_THREADS) k_stats_partial(const float4* __restrict__ rows, int64_t n,
+                                                                  int64_t per_block, Moments* __restrict__ part) {
+  Moments m[4];
+  for (int c = 0; c < 4; ++c) m[c] = Moments{0.0, 0.0, 0.0, INFINITY, -INFINITY};
+  const int64_t base = (int64_t)blockIdx.x * per_block;
+  for (int64_t j = threadIdx.x; j < per_block && base + j < n; j += STATS_THREADS) {
+    const float4 r = rows[2 * (base + j)];
+    const float v[4] = {r.x, r.y, r.z, r.w};
+#pragma unroll
+    for (int c = 0; c < 4; ++c) {
+      const double x = v[c];
+      m[c].n += 1.0;
+      const double d = x - m[c].mean;
+      m[c].mean += d / m[c].n;
+      m[c].m2 += d * (x - m[c].mean);
+      m[c].mn = fmin(m[c].mn, x);
+      m[c].mx = fmax(m[c].mx, x);
+    }
+  }
+  stats_block_store(m, part + 4 * (size_t)blockIdx.x);
+}
+__global__ void __launch_bounds__(STATS_THREADS) k_stats_final(const Moments* __restrict__ part, int64_t nb,
+                                                                Moments* __restrict__ out) {
+  Moments m[4];
+  for (int c = 0; c < 4; ++c) m[c] = Moments{0.0, 0.0, 0.0, INFINITY, -INFINITY};
+  for (int64_t b = threadIdx.x; b < nb; b += STATS_THREADS)
+    for (int c = 0; c < 4; ++c) m[c] = mom_merge(m[c], part[4 * b + c]);
+  stats_block_store(m, out);
+}
+
 // ---------------------------------------------------------------- noise (Philox)
 __global__ void k_noise(float* __restrict__ noise, int64_t total, int B, int n, uint64_t seed,
                         const long long* __restrict__ step_dev, int rank) {
@@ -174,9 +238,9 @@ __global__ void k_step_end(long long* step_dev) {
 __global__ void k_step_head(const float4* __restrict__ table, int64_t n_trans, const long long* __restrict__ step_dev,
                             StepInfo* __restrict__ info, float beta1, float beta2, int B, int n, int rank, int world,
                             uint64_t seed, float4* __restrict__ batch, float4* __restrict__ XA,
-                            float* __restrict__ noise, int64_t noise_total, int prank, int pworld) {
+                            float* __restrict__ noise, int64_t noise_total, int prank, int pworld, const Prep prep) {
   tc::grid_dep_wait();   /* programmatic dependent launch: the predecessor's results are needed from here on */
- 
+
   const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   const long long done = *step_dev;
   if (i == 0) {
@@ -190,7 +254,8 @@ __global__ void k_step_head(const float4* __restrict__ table, int64_t n_trans, c
     // rank holds only its own user shard (prank / pworld); the Philox stream below always uses the job's rank
     const int64_t p = ((int64_t)done * pworld + prank) * B + i;
     const int64_t t = stream_index(p, n_trans, (int64_t)B * pworld, seed);
-    const float4 a = __ldg(table + 2 * t), b = __ldg(table + 2 * t + 1);
+    float4 a = __ldg(table + 2 * t), b = __ldg(table + 2 * t + 1);
+    if (prep.any()) { a = prep_row0(prep, a); b = prep_row1(prep, b); }   // the table stays raw: scaled at gather
     batch[2 * i] = a;
     batch[2 * i + 1] = b;
     XA[i] = make_float4(a.x, a.y, 0.f, 0.f);
@@ -258,14 +323,20 @@ __device__ __forceinline__ float q_at(const QSrc& s, int net, int r, int o = 0) 
   return v + bias;
 }
 
-__global__ void k_actor_rows(const float4* __restrict__ batch, int B, float4* __restrict__ XA) {
+// Actor input rows of a staged minibatch.  With preprocessing the minibatch is staged in `in` (Handle::batch_in) and
+// its scaled rows are written to `batch` (thread i < B owns half-row 2i, thread B + i half-row 2i + 1); the staged rows
+// stay raw, so replaying phase 4 on one upload scales the same rows again.  Without preprocessing `in` == `batch`
+// and nothing is written there.
+__global__ void k_actor_rows(const float4* in, int B, float4* batch, float4* __restrict__ XA, const Prep prep) {
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= 2 * B) return;
   if (i < B) {
-    const float4 a = batch[2 * i];
+    float4 a = in[2 * i];
+    if (prep.any()) { a = prep_row0(prep, a); batch[2 * i] = a; }
     XA[i] = make_float4(a.x, a.y, 0.f, 0.f);
   } else {
-    const float4 b = batch[2 * (i - B) + 1];
+    float4 b = in[2 * (i - B) + 1];
+    if (prep.any()) { b = prep_row1(prep, b); batch[2 * (i - B) + 1] = b; }
     XA[i] = make_float4(b.x, b.y, 0.f, 0.f);
   }
 }
@@ -1084,7 +1155,7 @@ inline void phase0(Handle* h, cudaStream_t st, BatchSource bs, NoiseSource ns) {
                                                           h->stepinfo, c.beta1, c.beta2, B, h->n, c.rank, c.world_size,
                                                           c.seed, reinterpret_cast<float4*>(h->batch), h->XA, h->noise,
                                                           h->noise_floats, h->table_sharded ? 0 : c.rank,
-                                                          h->table_sharded ? 1 : c.world_size);
+                                                          h->table_sharded ? 1 : c.world_size, h->prep);
     CQL_LAUNCH_CHECK(h);
   } else {
     k_step_begin<<<1, 1, 0, st>>>(h->step_dev, h->stepinfo, c.beta1, c.beta2);
@@ -1094,7 +1165,7 @@ inline void phase0(Handle* h, cudaStream_t st, BatchSource bs, NoiseSource ns) {
       k_sample<<<(B + 127) / 128, 128, 0, st>>>(reinterpret_cast<const float4*>(h->table), h->n_trans, nullptr,
                                                 h->step_dev, 0, B, (int64_t)B * (h->table_sharded ? 1 : c.world_size),
                                                 h->table_sharded ? 0 : c.rank, h->table_sharded ? 1 : c.world_size,
-                                                c.seed, reinterpret_cast<float4*>(h->batch));
+                                                c.seed, reinterpret_cast<float4*>(h->staged_batch()));
       CQL_LAUNCH_CHECK(h);
     }
     if (ns == NoiseSource::Philox) {
@@ -1102,7 +1173,8 @@ inline void phase0(Handle* h, cudaStream_t st, BatchSource bs, NoiseSource ns) {
                                                                     h->step_dev, c.rank);
       CQL_LAUNCH_CHECK(h);
     }
-    k_actor_rows<<<(2 * B + 255) / 256, 256, 0, st>>>(batch4, B, h->XA);
+    k_actor_rows<<<(2 * B + 255) / 256, 256, 0, st>>>(reinterpret_cast<const float4*>(h->staged_batch()), B,
+                                                      reinterpret_cast<float4*>(h->batch), h->XA, h->prep);
     CQL_LAUNCH_CHECK(h);
   }
   {

@@ -15,7 +15,7 @@ from typing import Callable, Dict, Optional, Sequence
 
 import numpy as np
 
-from . import _lib, layout
+from . import _lib, layout, scalers
 
 METRIC_NAMES = ("temp_loss", "temp", "alpha_loss", "alpha", "critic_loss", "actor_loss")
 NOISE_KEYS = ("temp_eps", "alpha_eps_t", "alpha_eps_t1", "alpha_u",
@@ -237,6 +237,34 @@ class CqlEngine:
         """Fill the replay table with a seeded synthetic log of the given shape, generated on the device (stress shape)."""
         self._check(self._lib.cql_synth_table(self._h, int(n_rows), int(n_users), int(n_items), int(seed) & (2**64 - 1)),
                     "cql_synth_table")
+
+    def table_stats(self) -> dict:
+        """Column statistics of the loaded table's one-step rows (``cql_get_table_stats``): float64 arrays ``min``,
+        ``max``, ``mean``, ``m2`` and int64 ``count`` over the columns (obs.x, obs.y, act, rew), and ``rew_available``."""
+        st = _lib.TableStats()
+        self._check(self._lib.cql_get_table_stats(self._h, C.byref(st)), "cql_get_table_stats")
+        out = {k: np.array([getattr(st.col[c], k) for c in range(4)], dtype=np.int64 if k == "count" else np.float64)
+               for k in scalers.STAT_KEYS}
+        out["rew_available"] = bool(st.rew_available)
+        return out
+
+    def set_preprocessing(self, scaler=None, action_scaler=None, reward_scaler=None, stats: Optional[dict] = None) -> dict:
+        """d3rlpy's scalers for every later update and scoring call (``cql_set_preprocessing``).  Each argument is None,
+        a kind name fitted on ``stats`` (default: this engine's ``table_stats()``) or an explicit-parameter dict (see
+        ``scalers``).  All None restores the unscaled path.  -> the explicit parameters applied."""
+        specs = {"scaler": scaler, "action_scaler": action_scaler, "reward_scaler": reward_scaler}
+        if stats is None and any(isinstance(v, str) for v in specs.values()):
+            stats = self.table_stats()
+        params = scalers.resolve(specs, stats)
+        p = scalers.to_struct(params)
+        self._check(self._lib.cql_set_preprocessing(self._h, C.byref(p)), "cql_set_preprocessing")
+        return params
+
+    def get_preprocessing(self) -> dict:
+        """{"scaler", "action_scaler", "reward_scaler"} -> explicit-parameter dict or None."""
+        p = _lib.Preprocessing()
+        self._check(self._lib.cql_get_preprocessing(self._h, C.byref(p)), "cql_get_preprocessing")
+        return scalers.from_struct(p)
 
     @property
     def n_transitions(self) -> int:

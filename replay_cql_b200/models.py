@@ -31,6 +31,15 @@ class CQL(Recommender):
     ``n_steps`` steps of its user's episode and the TD target bootstraps from the state that many steps later with
     discount ``gamma ** k`` (``k`` shorter where the episode ends first).  It is unrelated to ``resume(n_steps=...)`` and
     ``engine.update(n_steps)``, which count update steps.
+
+    ``scaler`` (observations: ``None``, ``"min_max"``, ``"standard"``), ``action_scaler`` (``None``, ``"min_max"``) and
+    ``reward_scaler`` (``None``, ``"min_max"``, ``"standard"``) are d3rlpy's preprocessors, or explicit-parameter dicts
+    (``replay_cql_b200.scalers``).  Names are fitted by ``fit`` on the replay table (all ranks' rows when it is
+    sharded); ``resume`` and ``load`` keep the fitted parameters.  The minibatches and the scored observations are
+    transformed, the replay table stays raw.  With ``score="q"`` the greedy action enters Q in the network's (scaled)
+    action space, where d3rlpy's ``predict_value(x, predict(x))`` round-trips it through the reverse and forward action
+    transforms -- a few ulps of the action apart; ``score="policy"`` returns the reverse-transformed action (rating
+    units).
     """
 
     SHARD_ROWS = 200_000_000      # data-parallel fits shard the replay table by user range from this log size on
@@ -80,8 +89,14 @@ class CQL(Recommender):
         log_every: int = 1000,
         shard_table: Optional[bool] = None,
         n_steps: int = 1,
+        scaler=None,
+        action_scaler=None,
+        reward_scaler=None,
     ):
-        from . import _lib
+        from . import _lib, scalers
+        scaler = scalers.validate("scaler", scaler)
+        action_scaler = scalers.validate("action_scaler", action_scaler)
+        reward_scaler = scalers.validate("reward_scaler", reward_scaler)
         if not isinstance(n_steps, (int, np.integer)) or not 1 <= n_steps <= _lib.MAX_N_STEPS:
             raise ValueError(f"n_steps (the n-step TD horizon) must be an integer in 1..{_lib.MAX_N_STEPS}")
         if soft_q_backup:
@@ -119,6 +134,7 @@ class CQL(Recommender):
         self.log_every = log_every
         self.shard_table = shard_table
         self.n_steps = int(n_steps)
+        self.scaler, self.action_scaler, self.reward_scaler = scaler, action_scaler, reward_scaler
         self.engine: Optional[CqlEngine] = None
         self.last_metrics: Optional[Dict[str, float]] = None
 
@@ -152,6 +168,9 @@ class CQL(Recommender):
             "log_every": self.log_every,
             "shard_table": self.shard_table,
             "n_steps": self.n_steps,
+            "scaler": self.scaler,
+            "action_scaler": self.action_scaler,
+            "reward_scaler": self.reward_scaler,
         }
 
     # ------------------------------------------------------------------ engine
@@ -193,6 +212,7 @@ class CQL(Recommender):
             log = shard_log_by_user(log, rank, world)
         build_mdp_on_device(eng, log, top_k=self.top_k, action_randomization_scale=self.action_randomization_scale)
         eng.set_table_sharded(sharded)
+        self._fit_preprocessing(sharded)
         n_rows = eng.n_transitions
         per_epoch = self.n_steps_per_epoch
         if per_epoch is None:
@@ -203,6 +223,19 @@ class CQL(Recommender):
                                 n_rows, self.batch_size * world)
             return
         self._run_steps(total, per_epoch)
+
+    def _fit_preprocessing(self, sharded: bool) -> None:
+        """Fit the scalers on the table just built (a sharded table: every rank's statistics, all-gathered and combined
+        in rank order, so every rank applies the same parameter bits)."""
+        from . import scalers
+        specs = {"scaler": self.scaler, "action_scaler": self.action_scaler, "reward_scaler": self.reward_scaler}
+        if all(v is None for v in specs.values()):
+            return
+        stats = self.engine.table_stats()
+        if sharded:
+            rows = gather_rows(scalers.stats_to_array(stats)[None, :])
+            stats = scalers.combine([scalers.stats_from_array(r) for r in rows])
+        self.engine.set_preprocessing(**specs, stats=stats)
 
     def _run_steps(self, total: int, per_epoch: Optional[int] = None) -> None:
         """``total`` updates on the engine's replay table, continuing from its step counter (which fixes the position
@@ -394,8 +427,12 @@ class CQL(Recommender):
         n_rows = self.engine.n_transitions if self.save_replay_table else 0
         if n_rows:                                          # [n, 8] rows: obs.x obs.y act rew next.x next.y term discount
             np.save(os.path.join(path, "replay_table.npy"), self.engine.export_transitions())
+        meta = {"fitted": True, "step": step, "format": 2, "replay_rows": int(n_rows)}
+        prep = self.engine.get_preprocessing()
+        if any(v is not None for v in prep.values()):
+            meta["preprocessing"] = prep                    # the fitted parameters; absent = no preprocessing
         with open(os.path.join(path, "meta.json"), "w") as f:
-            json.dump({"fitted": True, "step": step, "format": 2, "replay_rows": int(n_rows)}, f)
+            json.dump(meta, f)
 
     def _load_model(self, path: str) -> None:
         with open(os.path.join(path, "meta.json")) as f:
@@ -406,6 +443,8 @@ class CQL(Recommender):
         eng = self._make_engine()
         eng.set_state(data["state"])
         eng.set_optimizer(data["adam_m"], data["adam_v"], int(meta["step"]))
+        if meta.get("preprocessing"):
+            eng.set_preprocessing(**meta["preprocessing"])
         if meta.get("replay_rows"):
             # verbatim: n-step rows cannot be rebuilt from their columns, and one-step rows come back bit for bit
             eng.set_table_rows(np.load(os.path.join(path, "replay_table.npy")))
