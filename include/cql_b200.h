@@ -265,7 +265,8 @@ int  cql_dp_mode(cql_handle* h, int32_t* fused_out);
 /* For each user: relevance of every candidate item, minus the user's seen
  * items (CSR, sorted item ids per user; seen_indptr may be NULL = no filter),
  * top-k by (relevance desc, item asc).  Rows with fewer than k candidates are
- * padded with item -1 / score -inf.
+ * padded with item -1 / score -inf.  A negative candidate id is skipped: it is
+ * never returned and does not count as a candidate.
  * replaces: CQL._predict per-user loop [EXT; pattern replay/models/neuromf.py:394-438]
  *           + _filter_seen replay/models/base_rec.py:417-464
  *           + get_top_k_recs replay/utils.py:112-127

@@ -158,6 +158,7 @@ __device__ __forceinline__ void fold_block_select(const float* __restrict__ scor
         const float s = score[r];
         if (!(s >= t_lo && s < t_hi)) continue;
         const int item = __ldg(items + i0 + r);
+        if (item < 0) continue;                        // never returned, as in the sequential folds
         if (has_seen && is_seen(sv, item)) continue;
         const int p = atomicAdd(const_cast<int*>(ncand), 1);
         if (p < FB_CAP) { candS[p] = s; candI[p] = item; }
