@@ -10,7 +10,9 @@
  * them with ctypes; INTEGRATION.md shows the stub a RePlay maintainer adds.
  *
  * Conventions: plain pointers and sizes, no C++/torch types.  Every function
- * returns 0 on success, non-zero on error (cql_last_error() has the text).
+ * returns 0 on success, non-zero on error (cql_last_error() has the text):
+ * 3 when an argument, the call sequence or the input data was rejected,
+ * 1 or 2 for a CUDA or other failure.
  * "host" pointers are ordinary (ideally pinned) host memory, "dev" pointers
  * are device memory on the handle's GPU.  One handle per GPU; a handle is not
  * thread-safe.  `stream` is a cudaStream_t passed as void*.  NULL selects the
@@ -95,16 +97,19 @@ int  cql_load_transitions(cql_handle* h, const float* obs, const float* act,
 int64_t cql_num_transitions(const cql_handle* h);
 /* MDP builder on the GPU: interaction log columns (host, input order) -> replay table, one episode per user.
  * order (user, timestamp, input order); reward = 1 for the user's top_k rows by (relevance desc, timestamp desc);
- * terminal = user's last row; action = (float)relevance + noise.  action_noise (host, per ORIGINAL row, already
+ * terminal = user's last row (top_k <= 0 rewards nothing); action = (float)relevance + noise.  action_noise (host, per ORIGINAL row, already
  * scaled; may be NULL => seeded N(0,1)*noise_scale on the device).  Optional host outputs (all NULL or all set):
  * obs_out [n][2], act_out/rew_out/term_out [n] in episode order; order_out [n] = original row of each step.
+ * timestamp holds int64 sort keys: float timestamps go through an order-preserving key on the host first
+ * (replay_cql_b200/frames.py timestamps_to_int64).  A NaN or infinite relevance fails the call (no table is left).
  * replaces: MdpDatasetBuilder.build (two Spark window sorts + orderBy + toPandas) [EXT upstream RePlay CQL wrapper] */
 int  cql_build_mdp(cql_handle* h, const int32_t* user_idx, const int32_t* item_idx, const int64_t* timestamp,
                    const double* relevance, const double* action_noise, int64_t n, int32_t top_k, float noise_scale,
                    float* obs_out, float* act_out, float* rew_out, float* term_out, int64_t* order_out);
 /* The same builder fed in CHUNKS (SURVEY 8f-1: Arrow record batches / Parquet row groups / pandas columns, each in its
  * own dtype, no intermediate frame): cql_mdp_begin announces n rows; cql_mdp_append adds the next `count` values of
- * one column (col: 0 user_idx, 1 item_idx, 2 timestamp, 3 relevance, 4 action noise [optional]; dtype CQL_DT_*; chunks
+ * one column (col: 0 user_idx, 1 item_idx, 2 timestamp, 3 relevance, 4 action noise [optional]; dtype CQL_DT_*,
+ * but only CQL_DT_I32 / CQL_DT_I64 keys for timestamps -- a float timestamp is rejected, not truncated; chunks
  * of a column arrive in row order, columns in any order -- timestamps first lets their sorts overlap the other
  * uploads).  Every chunk goes host -> pinned ring (up to four copy threads) -> device asynchronously.
  * cql_mdp_finish sorts, builds the replay table and ends the session (outputs as for cql_build_mdp).
@@ -229,7 +234,8 @@ int  cql_device_buffer(cql_handle* h, int which, void** dev_ptr, int64_t* n_floa
 
 /* Seen-items CSR of an interaction log, built on the device -- the structure the scorer's lazy seen filter searches
  * (replaces the host-side joins of `_filter_seen`, replay/models/base_rec.py:417-464, for the GPU path).
- * users_host / items_host [n] int32: the log's id columns in any order, duplicates allowed (host memory);
+ * users_host / items_host [n] int32: the log's id columns in any order, duplicates allowed (host memory); rows with
+ * a user outside [0, n_users_dim) or a negative item are dropped (no candidate id is negative: they filter nothing);
  * wanted_host [n_users_dim] uint8 or NULL: keep only rows of users whose flag is non-zero;
  * indptr_dev [n_users_dim + 1] int64 and seen_dev [>= n] int32: device buffers of the caller; on return user u's
  * de-duplicated items, ascending, are seen_dev[indptr_dev[u] .. indptr_dev[u + 1]); *n_seen_out = entries written.

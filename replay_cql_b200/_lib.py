@@ -122,6 +122,10 @@ class CqlLibraryError(RuntimeError):
     """The CUDA library is missing/unloadable, or a call into it failed."""
 
 
+class CqlArgumentError(CqlLibraryError, ValueError):
+    """A call into the library rejected an argument or the call sequence (return code 3)."""
+
+
 def load() -> C.CDLL:
     """Load the C-ABI library (once).  Raises ``CqlLibraryError`` -- never falls back."""
     global _lib
@@ -152,4 +156,5 @@ def load() -> C.CDLL:
 def check(handle, rc: int, what: str) -> None:
     if rc != 0:
         msg = load().cql_last_error(handle)
-        raise CqlLibraryError(f"{what} failed: {msg.decode() if msg else rc}")
+        err = CqlArgumentError if rc == 3 else CqlLibraryError
+        raise err(f"{what} failed: {msg.decode() if msg else rc}")

@@ -261,6 +261,9 @@ int guarded(cql_handle* ch, F&& f) {
     CQL_CUDA(cudaSetDevice(ch->h.cfg.device));
     f();
     return 0;
+  } catch (const ArgError& e) {
+    ch->h.err = e.msg;
+    return 3;
   } catch (const Error& e) {
     ch->h.err = e.msg;
     return 1;
@@ -706,7 +709,6 @@ int cql_mdp_append(cql_handle* ch, int32_t col, int32_t dtype, const void* host_
 int cql_mdp_finish(cql_handle* ch, int32_t top_k, float noise_scale, float* obs_out, float* act_out, float* rew_out,
                    float* term_out, int64_t* order_out) {
   return guarded(ch, [&] {
-    CQL_REQUIRE(top_k >= 0, "cql_mdp_finish: top_k < 0");
     ch->h.launches += mdp_finish(ch->h, top_k, noise_scale, obs_out, act_out, rew_out, term_out, order_out);
     destroy_graph(ch);
   });
@@ -741,7 +743,6 @@ int cql_build_mdp(cql_handle* ch, const int32_t* user_idx, const int32_t* item_i
                   const double* relevance, const double* action_noise, int64_t n, int32_t top_k, float noise_scale,
                   float* obs_out, float* act_out, float* rew_out, float* term_out, int64_t* order_out) {
   return guarded(ch, [&] {
-    CQL_REQUIRE(top_k >= 0, "cql_build_mdp: top_k < 0");
     CQL_CUDA(cudaDeviceSynchronize());
     ch->h.launches += mdp_build_on_device(ch->h, user_idx, item_idx, timestamp, relevance, action_noise, n, top_k,
                                           noise_scale, obs_out, act_out, rew_out, term_out, order_out);

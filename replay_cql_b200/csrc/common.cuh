@@ -37,6 +37,7 @@ __host__ __device__ inline int64_t grad_floats(int C) { return (int64_t)(1 + C) 
 
 // ---------------------------------------------------------------- errors
 struct Error { std::string msg; };
+struct ArgError : Error {};          // a rejected argument or call sequence (CQL_REQUIRE): the C API returns 3
 #define CQL_CUDA(expr)                                                                   \
   do {                                                                                   \
     cudaError_t _e = (expr);                                                             \
@@ -46,7 +47,7 @@ struct Error { std::string msg; };
   } while (0)
 #define CQL_REQUIRE(cond, text)                                                          \
   do {                                                                                   \
-    if (!(cond)) throw ::cql::Error{std::string(text)};                                  \
+    if (!(cond)) throw ::cql::ArgError{{std::string(text)}};                             \
   } while (0)
 
 // ---------------------------------------------------------------- device helpers

@@ -8,6 +8,7 @@
 // row of the user, action = relevance + noise, next_obs = next row of the same user).  Ties keep input order,
 // exactly like the host builder (replay_cql_b200/mdp.py), which the tests hold it bit-exact against.
 #include <algorithm>
+#include <cmath>
 #include <initializer_list>
 #include <vector>
 #include <cstring>
@@ -243,6 +244,8 @@ void cql::mdp_append(Handle& h, int col, int dtype, const void* host, int64_t co
   CQL_REQUIRE(dtype >= CQL_DT_I32 && dtype <= CQL_DT_F64, "cql_mdp_append: dtype must be one of CQL_DT_*");
   CQL_REQUIRE(count >= 0 && m.filled[col] + count <= m.n, "cql_mdp_append: more rows than cql_mdp_begin announced");
   CQL_REQUIRE(host != nullptr || count == 0, "cql_mdp_append: NULL chunk");
+  CQL_REQUIRE(col != 2 || dtype == CQL_DT_I32 || dtype == CQL_DT_I64,
+              "cql_mdp_append: timestamps must be int32 or int64 keys (convert float timestamps to an order-preserving key)");
   if (col == 4 && m.noise == nullptr) {
     m.noise = dmalloc<double>(m.n, m.pool, m.alloc_stream);
     CQL_CUDA(cudaStreamSynchronize(m.alloc_stream));
@@ -345,6 +348,15 @@ int64_t cql::mdp_finish(Handle& h, int top_k, float noise_scale, float* obs_out,
     for (int64_t i = 0; i < n; ++i) order_out[i] = tmp[(size_t)i];
   }
   CQL_CUDA(cudaStreamSynchronize(st));
+  // A NaN or infinite relevance (or action noise) gives a non-finite action, which would make every critic gradient
+  // NaN.  The action column's statistics (table_stats above: count, mean, M2, min, max, copied to the pinned
+  // stats_host before this synchronise) are finite exactly when every action is: no extra device work or copy.
+  const double* act_stats = h.stats_host + 5 * 2;
+  if (!(std::isfinite(act_stats[1]) && std::isfinite(act_stats[2]) && std::isfinite(act_stats[3]) && std::isfinite(act_stats[4]))) {
+    h.stats = cql_table_stats{};                    // no table is left: ensure_table set n_trans = 0
+    h.stats_pending = false;
+    CQL_REQUIRE(false, "cql_mdp_finish: relevance column has a non-finite value (or the action noise has)");
+  }
   h.n_trans = n;
   return m.launches;
 }
@@ -380,7 +392,7 @@ __global__ void k_seen_keys(const int32_t* __restrict__ user, const int32_t* __r
   const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= n) return;
   const int64_t u = user[i];
-  const bool keep = u >= 0 && u < n_users && (wanted == nullptr || wanted[u] != 0);
+  const bool keep = u >= 0 && u < n_users && item[i] >= 0 && (wanted == nullptr || wanted[u] != 0);
   key[i] = keep ? ((unsigned long long)u << 32) | (unsigned int)item[i] : (unsigned long long)n_users << 32;   // dropped rows sort last
 }
 // unique, sorted keys -> seen items + CSR row pointers (a thread fills the pointers of the users between its

@@ -16,6 +16,7 @@ from typing import Callable, Dict, Optional, Sequence
 import numpy as np
 
 from . import _lib, layout, scalers
+from .frames import timestamps_to_int64
 
 METRIC_NAMES = ("temp_loss", "temp", "alpha_loss", "alpha", "critic_loss", "actor_loss")
 NOISE_KEYS = ("temp_eps", "alpha_eps_t", "alpha_eps_t1", "alpha_u",
@@ -185,7 +186,7 @@ class CqlEngine:
         arrays in episode order (for parity tests); otherwise None."""
         user = np.ascontiguousarray(user_idx, dtype=np.int32)
         item = np.ascontiguousarray(item_idx, dtype=np.int32)
-        ts = np.ascontiguousarray(timestamp, dtype=np.int64)
+        ts = np.ascontiguousarray(timestamps_to_int64(timestamp))
         rel = np.ascontiguousarray(relevance, dtype=np.float64)
         n = user.size
         if not (item.size == ts.size == rel.size == n):

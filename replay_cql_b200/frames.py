@@ -61,14 +61,24 @@ def get_ids(data: Any, column: str) -> pd.DataFrame:
     raise ValueError(f"Wrong type {type(data)}")
 
 
-def timestamps_to_int64(col: pd.Series) -> np.ndarray:
-    """Timestamps (datetime64 / numeric) -> int64 preserving order."""
-    if np.issubdtype(col.dtype, np.datetime64):
-        return col.to_numpy().astype("datetime64[ns]").astype(np.int64)
+def timestamps_to_int64(col: Any) -> np.ndarray:
+    """Timestamps (pandas Series or numpy array; datetime64 / numeric) -> int64 keys with the same order and the same
+    ties.  The one place a non-integer timestamp becomes an integer key: every builder (host, device, one-call,
+    chunked) sorts these keys.  Floats map element by element to an order-preserving bit key (-0.0 and +0.0 are one
+    key; NaN raises), so a chunked column converts chunk by chunk."""
+    if isinstance(col, pd.Series) and isinstance(col.dtype, pd.DatetimeTZDtype):
+        col = col.dt.tz_convert("UTC").dt.tz_localize(None)
     if col.dtype == object:
-        return pd.to_datetime(col).to_numpy().astype("datetime64[ns]").astype(np.int64)
-    arr = col.to_numpy()
+        return pd.to_datetime(pd.Series(col)).to_numpy().astype("datetime64[ns]").astype(np.int64)
+    arr = col.to_numpy() if isinstance(col, pd.Series) else np.asarray(col)
+    if np.issubdtype(arr.dtype, np.datetime64):
+        return arr.astype("datetime64[ns]").astype(np.int64)
     if np.issubdtype(arr.dtype, np.integer):
         return arr.astype(np.int64)
-    # float timestamps: order-preserving rank
-    return np.argsort(np.argsort(arr, kind="stable"), kind="stable").astype(np.int64)
+    if not np.issubdtype(arr.dtype, np.floating):
+        raise ValueError(f"unsupported timestamp dtype {arr.dtype}")
+    x = arr.astype(np.float64)
+    if np.isnan(x).any():
+        raise ValueError("timestamp column has a NaN")
+    b = (x + 0.0).view(np.int64)                   # + 0.0: -0.0 -> +0.0
+    return np.where(b >= 0, b, b ^ np.int64(0x7FFF_FFFF_FFFF_FFFF))

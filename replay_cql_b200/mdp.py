@@ -19,6 +19,7 @@ from dataclasses import dataclass
 from typing import Any, Optional
 
 import numpy as np
+from pandas.api import types as pd_api
 
 from .frames import to_pandas, timestamps_to_int64
 
@@ -61,6 +62,8 @@ def build_mdp(log: Any, top_k: int = 10, action_randomization_scale: float = 1e-
         raise ValueError("user_idx/item_idx must be < 2**24 to be exact in float32 observations")
     ts = timestamps_to_int64(pdf["timestamp"])
     rel = pdf["relevance"].to_numpy().astype(np.float64)
+    if not np.isfinite(rel).all():
+        raise ValueError("relevance column has a non-finite value")
     row = np.arange(n, dtype=np.int64)
 
     order = np.lexsort((row, ts, user))                      # (user, timestamp, input order)
@@ -69,7 +72,8 @@ def build_mdp(log: Any, top_k: int = 10, action_randomization_scale: float = 1e-
     if n > 1:
         term[:-1] = (u_sorted[1:] != u_sorted[:-1]).astype(np.float32)
 
-    rank_order = np.lexsort((row, -ts, -rel, user))          # (user, relevance desc, timestamp desc)
+    rank_order = np.lexsort((row, ~ts, -rel, user))          # (user, relevance desc, timestamp desc); ~ts = -ts - 1
+                                                             # reverses every int64, INT64_MIN included
     ur = user[rank_order]
     starts = np.flatnonzero(np.r_[True, ur[1:] != ur[:-1]]) if n else np.zeros(0, dtype=np.int64)
     group_start = np.repeat(starts, np.diff(np.r_[starts, n])) if n else starts
@@ -103,10 +107,15 @@ def to_transitions(mdp: MdpArrays) -> dict:
 
 
 def seen_csr(log: Any, n_users_dim: int):
-    """Per-user sorted, de-duplicated seen items as CSR over user id (for the lazy seen filter)."""
+    """Per-user sorted, de-duplicated seen items as CSR over user id (for the lazy seen filter).  Rows with a negative
+    user or item are dropped (no candidate id is negative, so they filter nothing); a user at or past ``n_users_dim``
+    widens the CSR."""
     pdf = to_pandas(log)
     user = pdf["user_idx"].to_numpy().astype(np.int64)
     item = pdf["item_idx"].to_numpy().astype(np.int64)
+    keep = (user >= 0) & (item >= 0)
+    if not keep.all():
+        user, item = user[keep], item[keep]
     if user.size:
         n_users_dim = max(n_users_dim, int(user.max()) + 1)
     key = user * (2 ** 32) + item
@@ -137,6 +146,12 @@ def _column_chunks(log: Any, name: str):
             t = ch.type
             if pa.types.is_timestamp(t) or pa.types.is_date64(t) or pa.types.is_duration(t):
                 ch, t = ch.view(pa.int64()), pa.int64()              # same buffer, order-preserving for one unit
+            elif pa.types.is_date32(t):
+                ch, t = ch.view(pa.int32()), pa.int32()              # days since the epoch
+            if name == "timestamp" and pa.types.is_floating(t):      # float timestamps: the host's order-preserving key
+                key = timestamps_to_int64(ch.to_numpy(zero_copy_only=False))
+                yield key.ctypes.data, key.dtype, key.size, key
+                continue
             if not (pa.types.is_integer(t) or pa.types.is_floating(t)) or t.bit_width not in (32, 64) or \
                     (pa.types.is_integer(t) and not pa.types.is_signed_integer(t)):
                 ch = ch.cast(pa.float64() if pa.types.is_floating(t) or pa.types.is_decimal(t) else pa.int64())
@@ -147,7 +162,7 @@ def _column_chunks(log: Any, name: str):
         return
     pdf = to_pandas(log)
     ser = pdf[name]
-    if name == "timestamp" and not (np.issubdtype(ser.dtype, np.integer) and ser.dtype.itemsize in (4, 8)):
+    if name == "timestamp" and not (pd_api.is_integer_dtype(ser.dtype) and ser.dtype.itemsize in (4, 8)):
         arr = timestamps_to_int64(ser)
     else:
         arr = ser.to_numpy()
