@@ -16,16 +16,48 @@
 
 using namespace cql;
 
+// A CUDA graph of one update, captured from an enqueue function on first use and again when the stream changes.  A
+// replay counts the launches the capture made.
+struct StepGraph {
+  cudaGraphExec_t exec = nullptr;
+  cudaStream_t stream = nullptr;
+  int64_t launches = 0;
+
+  void reset() {
+    if (exec) cudaGraphExecDestroy(exec);
+    exec = nullptr;
+  }
+  // capture `enqueue` if needed, then replay the graph n times on st
+  template <typename F>
+  void run(Handle& h, cudaStream_t st, int64_t n, F&& enqueue) {
+    if (!exec || stream != st) {
+      reset();
+      cudaGraph_t g = nullptr;
+      const int64_t before = h.launches;
+      CQL_CUDA(cudaStreamBeginCapture(st, cudaStreamCaptureModeThreadLocal));
+      try {
+        enqueue();
+      } catch (...) {
+        cudaStreamEndCapture(st, &g);
+        if (g) cudaGraphDestroy(g);
+        throw;
+      }
+      CQL_CUDA(cudaStreamEndCapture(st, &g));
+      launches = h.launches - before;
+      h.launches = before;
+      CQL_CUDA(cudaGraphInstantiate(&exec, g, 0));
+      CQL_CUDA(cudaGraphDestroy(g));
+      stream = st;
+    }
+    for (int64_t i = 0; i < n; ++i) CQL_CUDA(cudaGraphLaunch(exec, st));
+    h.launches += launches * n;
+  }
+};
+
 struct cql_handle {
   Handle h;
-  // CUDA graph of one sampled update (phases 0-3), captured lazily per stream
-  cudaGraphExec_t graph_exec = nullptr;
-  cudaStream_t graph_stream = nullptr;
-  int64_t graph_launches = 0;
-  // same for the host-minibatch entry (cql_update_batch): [0] Philox noise, [1] caller-provided noise
-  cudaGraphExec_t batch_graph[2] = {nullptr, nullptr};
-  cudaStream_t batch_graph_stream[2] = {nullptr, nullptr};
-  int64_t batch_graph_launches[2] = {0, 0};
+  StepGraph update_graph;            // one sampled update (phases 0-3): cql_update
+  StepGraph batch_graph[2];          // the host-minibatch entry (cql_update_batch): [0] Philox noise, [1] caller-provided noise
   // grow-only device scratch for the host-pointer scoring entry points
   void* sbuf[8] = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr};
   size_t sbuf_bytes[8] = {0, 0, 0, 0, 0, 0, 0, 0};
@@ -34,9 +66,7 @@ struct cql_handle {
   size_t part_elems = 0;
   uint8_t* packed_score = nullptr;   // tf32-packed W2 of actor + critics for the tensor-core scorer
   // cql_update_batches: the bare step (minibatch already on the device) as a graph, pinned staging ring, metrics rows
-  cudaGraphExec_t step_graph = nullptr;
-  cudaStream_t step_graph_stream = nullptr;
-  int64_t step_graph_launches = 0;
+  StepGraph step_graph;
   float* ring = nullptr;             // pinned [8][B*8]
   cudaEvent_t ring_ev[8] = {};
   float* metrics_rows = nullptr;     // pinned [metrics_rows_cap][8]
@@ -84,8 +114,6 @@ void set_kernel_attrs() {
   CQL_CUDA(cudaFuncSetAttribute(k_score_topk, cudaFuncAttributeMaxDynamicSharedMemorySize, score_smem(CQL_MAX_TOPK)));
   CQL_CUDA(cudaFuncSetAttribute(k_score_pairs, cudaFuncAttributeMaxDynamicSharedMemorySize, FWD_SMEM));
   CQL_CUDA(cudaFuncSetAttribute(k_topk_filter_staged, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)TKS_SMEM));
-  CQL_CUDA(cudaFuncSetAttribute(tc::tc_fwd_kernel<true, 2, 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tc::FwdSmem<true, tc::FWD_NPW>::BYTES));
-  CQL_CUDA(cudaFuncSetAttribute(tc::tc_fwd_kernel<true, 3, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tc::FwdSmem<true, tc::FWD_NPW>::BYTES));
   CQL_CUDA(cudaFuncSetAttribute(tc::tc_fwd_kernel<false, 2, 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tc::FwdSmem<false, tc::FWD_NPW>::BYTES));
   CQL_CUDA(cudaFuncSetAttribute(tc::tc_fwd_kernel<false, 3, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tc::FwdSmem<false, tc::FWD_NPW>::BYTES));
   CQL_CUDA(cudaFuncSetAttribute(tc::tc_score_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tc::ScoreSmem::bytes(CQL_MAX_TOPK)));
@@ -114,10 +142,7 @@ void set_kernel_attrs() {
   CQL_CUDA(cudaFuncSetAttribute(tc::tc_bwd1_ts_kernel<3, 1, true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tc::TsCfg::SMEM_BYTES));
   CQL_CUDA(cudaFuncSetAttribute(tc::tc_bwd1_ts_kernel<3, 1, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tc::TsCfg::SMEM_BYTES));
   CQL_CUDA(cudaFuncSetAttribute(tc::tc_bwd1_ts_kernel<2, 2, true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tc::TsCfg::SMEM_BYTES));
-  const int f1 = (int)tc::FwdSmem<true, tc::BWD1_NPW>::BYTES, f0 = (int)tc::FwdSmem<false, tc::BWD1_NPW>::BYTES;
-  CQL_CUDA(cudaFuncSetAttribute(tc::tc_bwd1_kernel<true, 3, 1, true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, f1));
-  CQL_CUDA(cudaFuncSetAttribute(tc::tc_bwd1_kernel<true, 3, 1, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, f1));
-  CQL_CUDA(cudaFuncSetAttribute(tc::tc_bwd1_kernel<true, 2, 2, true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, f1));
+  const int f0 = (int)tc::FwdSmem<false, tc::BWD1_NPW>::BYTES;
   CQL_CUDA(cudaFuncSetAttribute(tc::tc_bwd1_kernel<false, 3, 1, true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, f0));
   CQL_CUDA(cudaFuncSetAttribute(tc::tc_bwd1_kernel<false, 3, 1, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, f0));
   CQL_CUDA(cudaFuncSetAttribute(tc::tc_bwd1_kernel<false, 2, 2, true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, f0));
@@ -224,7 +249,7 @@ void create_impl(const cql_config* cfg, cql_handle* ch) {
       h.packed_bwd2 = h.dalloc<uint8_t>((size_t)(1 + C) * h.packed_net_bytes2);
       h.w2max = h.dalloc<int>((size_t)(2 + 2 * C) * 4);
       h.ap_wmax = h.dalloc<int>((size_t)CQL_MAX_CRITICS * 17);
-      if (const char* sw = std::getenv("CQL_PAIR_SWAP")) h.pair_swap_b = std::atoi(sw);
+      h.pair_swap_b = switches().pair_swap;
     }
     h.slots1 = (f16 ? tc::HCfg::NEW : 4) * h.num_sms;
     h.splits_tc = h.num_sms;
@@ -232,7 +257,6 @@ void create_impl(const cql_config* cfg, cql_handle* ch) {
     h.small2 = h.dalloc<float>((size_t)C * h.splits_tc * SMALL_STRIDE);
     h.pw2_tc = h.dalloc<float>((size_t)(h.num_sms + C) * H * H);
     h.dX_part = h.dalloc<float4>((size_t)C * std::max(slices, 8) * B);
-    h.b2_tickets = h.dalloc<unsigned int>((size_t)CQL_MAX_CRITICS * 64 + 64);
   }
   // scalars start at the configured initial values; networks are set by cql_set_weights
   float sc[SCALAR_SLOT] = {0};
@@ -242,9 +266,9 @@ void create_impl(const cql_config* cfg, cql_handle* ch) {
 }
 
 void destroy_graph(cql_handle* ch) {
-  if (ch->graph_exec) { cudaGraphExecDestroy(ch->graph_exec); ch->graph_exec = nullptr; }
-  for (auto& g : ch->batch_graph) if (g) { cudaGraphExecDestroy(g); g = nullptr; }
-  if (ch->step_graph) { cudaGraphExecDestroy(ch->step_graph); ch->step_graph = nullptr; }
+  ch->update_graph.reset();
+  for (auto& g : ch->batch_graph) g.reset();
+  ch->step_graph.reset();
 }
 
 template <typename F>
@@ -274,10 +298,25 @@ int guarded(cql_handle* ch, F&& f) {
 }
 
 void run_full_step(Handle* h, cudaStream_t st, BatchSource bs, NoiseSource ns) {
-  phase0(h, st, bs, ns);
-  phase1(h, st);
-  phase2(h, st);
-  phase3(h, st);
+  with_precision(h, [&](auto p) {
+    constexpr Prec P = decltype(p)::value;
+    phase0<P>(h, st, bs, ns);
+    phase1<P>(h, st);
+    phase2<P>(h, st);
+    phase3<P>(h, st);
+  });
+}
+
+// a host minibatch (obs [B][2], act, rew, next_obs [B][2], term) -> B rows of the table's format in `rows`; the discount
+// slot holds gamma in n-step mode (these are one-step transitions) and 0 otherwise
+void pack_rows(const Handle& h, const float* obs, const float* act, const float* rew, const float* next_obs,
+               const float* term, float* rows) {
+  const float disc = h.n_steps > 1 ? h.cfg.gamma : 0.f;
+  for (int b = 0; b < h.B; ++b) {
+    float* r = rows + (size_t)b * 8;
+    r[0] = obs[2 * b]; r[1] = obs[2 * b + 1]; r[2] = act[b]; r[3] = rew[b];
+    r[4] = next_obs[2 * b]; r[5] = next_obs[2 * b + 1]; r[6] = term[b]; r[7] = disc;
+  }
 }
 
 // obs scaler on: the candidate items' scaled coordinates (k_scale_items) in scratch slot 7; off: nullptr (the scorers
@@ -434,32 +473,7 @@ void update_staged_batch(cql_handle* ch, const float* noise, float* metrics6, fl
     run_full_step(&h, st, BatchSource::Provided, noise ? NoiseSource::Provided : NoiseSource::Philox);
     CQL_CUDA(cudaMemcpyAsync(h.metrics_host, h.metrics, 8 * sizeof(float), cudaMemcpyDeviceToHost, st));
   };
-  const int gi = noise ? 1 : 0;
-  if (h.timing) {
-    enqueue();
-  } else {
-    if (!ch->batch_graph[gi] || ch->batch_graph_stream[gi] != st) {
-      if (ch->batch_graph[gi]) { cudaGraphExecDestroy(ch->batch_graph[gi]); ch->batch_graph[gi] = nullptr; }
-      cudaGraph_t g = nullptr;
-      const int64_t before = h.launches;
-      CQL_CUDA(cudaStreamBeginCapture(st, cudaStreamCaptureModeThreadLocal));
-      try {
-        enqueue();
-      } catch (...) {
-        cudaStreamEndCapture(st, &g);
-        if (g) cudaGraphDestroy(g);
-        throw;
-      }
-      CQL_CUDA(cudaStreamEndCapture(st, &g));
-      ch->batch_graph_launches[gi] = h.launches - before;
-      h.launches = before;
-      CQL_CUDA(cudaGraphInstantiate(&ch->batch_graph[gi], g, 0));
-      CQL_CUDA(cudaGraphDestroy(g));
-      ch->batch_graph_stream[gi] = st;
-    }
-    CQL_CUDA(cudaGraphLaunch(ch->batch_graph[gi], st));
-    h.launches += ch->batch_graph_launches[gi];
-  }
+  ch->batch_graph[noise ? 1 : 0].run(h, st, 1, enqueue);
   if (grads_out)
     CQL_CUDA(cudaMemcpyAsync(grads_out, h.grads, grad_floats(h.C) * sizeof(float), cudaMemcpyDeviceToHost, st));
   CQL_CUDA(cudaStreamSynchronize(st));
@@ -545,7 +559,7 @@ int cql_set_weights(cql_handle* ch, const float* host_flat, int64_t n) {
     CQL_REQUIRE(host_flat && n == state_floats(ch->h.C), "cql_set_weights: n must equal cql_state_floats()");
     CQL_CUDA(cudaDeviceSynchronize());
     CQL_CUDA(cudaMemcpy(ch->h.params, host_flat, n * sizeof(float), cudaMemcpyHostToDevice));
-    pack_all_weights(&ch->h, ch->h.own_stream);
+    with_precision(&ch->h, [&](auto p) { pack_all_weights<decltype(p)::value>(&ch->h, ch->h.own_stream); });
     CQL_CUDA(cudaStreamSynchronize(ch->h.own_stream));
   });
 }
@@ -783,27 +797,7 @@ int cql_update(cql_handle* ch, int64_t n_steps, float* metrics6, void* stream) {
     CQL_REQUIRE(n_steps >= 0, "cql_update: n_steps < 0");
     CQL_REQUIRE(h.n_trans > 0, "cql_update: no transitions loaded (call cql_load_transitions first)");
     cudaStream_t st = pick_stream(&h, stream);
-    if (!ch->graph_exec || ch->graph_stream != st) {
-      destroy_graph(ch);
-      cudaGraph_t g = nullptr;
-      const int64_t before = h.launches;
-      CQL_CUDA(cudaStreamBeginCapture(st, cudaStreamCaptureModeThreadLocal));
-      try {
-        run_full_step(&h, st, BatchSource::Sampled, NoiseSource::Philox);
-      } catch (...) {
-        cudaStreamEndCapture(st, &g);
-        if (g) cudaGraphDestroy(g);
-        throw;
-      }
-      CQL_CUDA(cudaStreamEndCapture(st, &g));
-      ch->graph_launches = h.launches - before;
-      h.launches = before;
-      CQL_CUDA(cudaGraphInstantiate(&ch->graph_exec, g, 0));
-      CQL_CUDA(cudaGraphDestroy(g));
-      ch->graph_stream = st;
-    }
-    for (int64_t i = 0; i < n_steps; ++i) CQL_CUDA(cudaGraphLaunch(ch->graph_exec, st));
-    h.launches += ch->graph_launches * n_steps;
+    ch->update_graph.run(h, st, n_steps, [&] { run_full_step(&h, st, BatchSource::Sampled, NoiseSource::Philox); });
     if (metrics6) {
       CQL_CUDA(cudaMemcpyAsync(h.metrics_host, h.metrics, 8 * sizeof(float), cudaMemcpyDeviceToHost, st));
       CQL_CUDA(cudaStreamSynchronize(st));
@@ -883,17 +877,15 @@ int cql_timed_update(cql_handle* ch, float* out_ms8, void* stream) {
     cudaStream_t st = pick_stream(&h, stream);
     for (int i = 0; i < 13; ++i)
       if (!h.ev[i]) CQL_CUDA(cudaEventCreate(&h.ev[i]));
-    h.timing = true;
-    g_timing_no_pdl = true;      // events between kernels only separate their durations without PDL overlap
-    try {
+    {
+      // events between kernels only separate their durations without PDL overlap
+      struct TimingScope {
+        Handle& h;
+        explicit TimingScope(Handle& h_) : h(h_) { h.timing = true; h.pdl_off = true; }
+        ~TimingScope() { h.timing = false; h.pdl_off = false; }
+      } timing(h);
       run_full_step(&h, st, BatchSource::Sampled, NoiseSource::Philox);
-    } catch (...) {
-      h.timing = false;
-      g_timing_no_pdl = false;
-      throw;
     }
-    h.timing = false;
-    g_timing_no_pdl = false;
     CQL_CUDA(cudaStreamSynchronize(st));
     auto ms = [&](int a, int b) { float t = 0.f; CQL_CUDA(cudaEventElapsedTime(&t, h.ev[a], h.ev[b])); return t; };
     const float fwd_all = ms(3, 4);           // TIMED_FWD_REPS launches of the critic forward, back to back
@@ -910,13 +902,7 @@ int cql_update_batch(cql_handle* ch, const float* obs, const float* act, const f
     Handle& h = ch->h;
     CQL_REQUIRE(obs && act && rew && next_obs && term, "cql_update_batch: NULL batch pointer");
     cudaStream_t st = pick_stream(&h, stream);
-    const int B = h.B;
-    const float disc = h.n_steps > 1 ? h.cfg.gamma : 0.f;     // one-step transitions: discount gamma in n-step mode
-    for (int b = 0; b < B; ++b) {
-      float* r = h.batch_host + (size_t)b * 8;
-      r[0] = obs[2 * b]; r[1] = obs[2 * b + 1]; r[2] = act[b]; r[3] = rew[b];
-      r[4] = next_obs[2 * b]; r[5] = next_obs[2 * b + 1]; r[6] = term[b]; r[7] = disc;
-    }
+    pack_rows(h, obs, act, rew, next_obs, term, h.batch_host);
     update_staged_batch(ch, noise, metrics6, grads_out, st);
   });
 }
@@ -962,43 +948,20 @@ int cql_update_batches(cql_handle* ch, int64_t n_batches, const float* obs, cons
       CQL_CUDA(cudaMallocHost(&ch->metrics_rows, (size_t)n_batches * 8 * sizeof(float)));
       ch->metrics_rows_cap = n_batches;
     }
-    if (!ch->step_graph || ch->step_graph_stream != st) {          // the step alone: minibatch already in h.batch
-      if (ch->step_graph) { cudaGraphExecDestroy(ch->step_graph); ch->step_graph = nullptr; }
-      cudaGraph_t g = nullptr;
-      const int64_t before = h.launches;
-      CQL_CUDA(cudaStreamBeginCapture(st, cudaStreamCaptureModeThreadLocal));
-      try {
-        run_full_step(&h, st, BatchSource::Provided, NoiseSource::Philox);
-      } catch (...) {
-        cudaStreamEndCapture(st, &g);
-        if (g) cudaGraphDestroy(g);
-        throw;
-      }
-      CQL_CUDA(cudaStreamEndCapture(st, &g));
-      ch->step_graph_launches = h.launches - before;
-      h.launches = before;
-      CQL_CUDA(cudaGraphInstantiate(&ch->step_graph, g, 0));
-      CQL_CUDA(cudaGraphDestroy(g));
-      ch->step_graph_stream = st;
-    }
+    auto step = [&] { run_full_step(&h, st, BatchSource::Provided, NoiseSource::Philox); };   // minibatch already in h.batch
+    ch->step_graph.run(h, st, 0, step);                                   // captured here, replayed in the loop
     // Copies ride on their own stream: minibatch i goes pinned ring -> device ring there (every step, 32 B x B), the
     // compute stream only waits for its event, moves it into h.batch (device to device), replays the step and drops the
     // step's metrics into a device slot, which the copy stream takes to the host (every step).  On one stream each
     // step paid both PCIe copies' start-up latency in series (e2e 0.885 of the HBM-resident rate).
     CQL_CUDA(cudaEventRecord(ch->ev_used[0], st));                        // orders the copy stream behind earlier work on st
     CQL_CUDA(cudaStreamWaitEvent(cs, ch->ev_used[0], 0));
-    const float disc = h.n_steps > 1 ? h.cfg.gamma : 0.f;     // one-step transitions: discount gamma in n-step mode
     for (int64_t i = 0; i < n_batches; ++i) {
       const int slot = (int)(i % RING);
       if (i >= RING) CQL_CUDA(cudaEventSynchronize(ch->ring_ev[slot]));     // that slot's host->device copy has run
       float* stage = ch->ring + (size_t)slot * row_floats;
-      const float *o = obs + (size_t)i * B * 2, *a = act + (size_t)i * B, *r = rew + (size_t)i * B,
-                  *no = next_obs + (size_t)i * B * 2, *t = term + (size_t)i * B;
-      for (int b = 0; b < B; ++b) {
-        float* w = stage + (size_t)b * 8;
-        w[0] = o[2 * b]; w[1] = o[2 * b + 1]; w[2] = a[b]; w[3] = r[b];
-        w[4] = no[2 * b]; w[5] = no[2 * b + 1]; w[6] = t[b]; w[7] = disc;
-      }
+      pack_rows(h, obs + (size_t)i * B * 2, act + (size_t)i * B, rew + (size_t)i * B, next_obs + (size_t)i * B * 2,
+                term + (size_t)i * B, stage);
       float* dslot = ch->dev_ring + (size_t)slot * row_floats;
       if (i >= RING) CQL_CUDA(cudaStreamWaitEvent(cs, ch->ev_used[slot], 0));   // the device slot has been consumed
       CQL_CUDA(cudaMemcpyAsync(dslot, stage, row_floats * sizeof(float), cudaMemcpyHostToDevice, cs));
@@ -1006,8 +969,7 @@ int cql_update_batches(cql_handle* ch, int64_t n_batches, const float* obs, cons
       CQL_CUDA(cudaStreamWaitEvent(st, ch->ring_ev[slot], 0));
       CQL_CUDA(cudaMemcpyAsync(h.staged_batch(), dslot, row_floats * sizeof(float), cudaMemcpyDeviceToDevice, st));
       CQL_CUDA(cudaEventRecord(ch->ev_used[slot], st));
-      CQL_CUDA(cudaGraphLaunch(ch->step_graph, st));
-      h.launches += ch->step_graph_launches;
+      ch->step_graph.run(h, st, 1, step);
       if (i >= RING) CQL_CUDA(cudaStreamWaitEvent(st, ch->ev_met_out[slot], 0));   // the metrics slot has left the device
       CQL_CUDA(cudaMemcpyAsync(ch->dev_metrics + (size_t)slot * 8, h.metrics, 8 * sizeof(float), cudaMemcpyDeviceToDevice, st));
       CQL_CUDA(cudaEventRecord(ch->ev_met[slot], st));
@@ -1031,12 +993,7 @@ int cql_upload_batch(cql_handle* ch, const float* obs, const float* act, const f
     cudaStream_t st = pick_stream(&h, stream);
     const int B = h.B;
     CQL_CUDA(cudaStreamSynchronize(st));      // the staging buffer may still be in flight from the previous step
-    const float disc = h.n_steps > 1 ? h.cfg.gamma : 0.f;     // one-step transitions: discount gamma in n-step mode
-    for (int b = 0; b < B; ++b) {
-      float* r = h.batch_host + (size_t)b * 8;
-      r[0] = obs[2 * b]; r[1] = obs[2 * b + 1]; r[2] = act[b]; r[3] = rew[b];
-      r[4] = next_obs[2 * b]; r[5] = next_obs[2 * b + 1]; r[6] = term[b]; r[7] = disc;
-    }
+    pack_rows(h, obs, act, rew, next_obs, term, h.batch_host);
     CQL_CUDA(cudaMemcpyAsync(h.staged_batch(), h.batch_host, (size_t)B * 8 * sizeof(float), cudaMemcpyHostToDevice, st));
   });
 }
@@ -1045,14 +1002,17 @@ int cql_step_phase(cql_handle* ch, int phase, void* stream) {
   return guarded(ch, [&] {
     Handle& h = ch->h;
     cudaStream_t st = pick_stream(&h, stream);
-    switch (phase) {
-      case 0: phase0(&h, st, BatchSource::Sampled, NoiseSource::Philox); break;
-      case 1: phase1(&h, st); break;
-      case 2: phase2(&h, st); break;
-      case 3: phase3(&h, st); break;
-      case 4: phase0(&h, st, BatchSource::Provided, NoiseSource::Philox); break;   // after cql_upload_batch
-      default: throw Error{"cql_step_phase: phase must be 0..4"};
-    }
+    with_precision(&h, [&](auto p) {
+      constexpr Prec P = decltype(p)::value;
+      switch (phase) {
+        case 0: phase0<P>(&h, st, BatchSource::Sampled, NoiseSource::Philox); break;
+        case 1: phase1<P>(&h, st); break;
+        case 2: phase2<P>(&h, st); break;
+        case 3: phase3<P>(&h, st); break;
+        case 4: phase0<P>(&h, st, BatchSource::Provided, NoiseSource::Philox); break;   // after cql_upload_batch
+        default: throw Error{"cql_step_phase: phase must be 0..4"};
+      }
+    });
   });
 }
 
@@ -1080,8 +1040,8 @@ int cql_dp_attach(cql_handle* ch, int32_t world, int32_t rank, const void* const
     p.epoch = (unsigned long long*)ch->dp_local;
     p.ticket = (unsigned int*)((char*)ch->dp_local + 64);
     p.error = (int*)((char*)ch->dp_local + 128);
-    p.debug = std::getenv("CQL_DP_DEBUG") ? std::atoi(std::getenv("CQL_DP_DEBUG")) : 0;
-    h.dp_fused = world > 1 && ll_room && h.cfg.precision == CQL_PREC_F16X3 && std::getenv("CQL_NO_FUSED_DP") == nullptr;
+    p.debug = switches().dp_debug;
+    h.dp_fused = world > 1 && ll_room && h.cfg.precision == CQL_PREC_F16X3 && !switches().no_fused_dp;
     destroy_graph(ch);
   });
 }

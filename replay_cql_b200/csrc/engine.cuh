@@ -1,5 +1,6 @@
 // engine.cuh -- the per-GPU handle: configuration, HBM-resident state, scratch.
 #pragma once
+#include <cstdlib>
 #include <vector>
 #include <string>
 #include "common.cuh"
@@ -57,6 +58,50 @@ __device__ __forceinline__ float4 prep_row1(const Prep& p, float4 r) {
 
 constexpr int STATS_MAX_BLOCKS = 1024;                               // table_stats (update.cuh)
 constexpr size_t STATS_DEV_DOUBLES = (STATS_MAX_BLOCKS + 1) * 4 * 5;
+
+// A/B switches of the update schedule, read from the environment once per process.  Each selects the path a measurement
+// in DESIGN.md compared against; unset, the library runs its default schedule.
+struct Switches {
+  int skip;                   // CQL_SKIP=<mask>: leave the launches with these bits out (timing experiments; results wrong)
+  bool no_pdl;                // CQL_NO_PDL: no programmatic dependent launch
+  bool no_pair;               // CQL_NO_PAIR: no CTA-pair kernels (forward, bwd1, bwd2)
+  bool no_pair_bwd1;          // CQL_NO_PAIR_BWD1: no CTA-pair bwd1
+  bool no_pair_bwd2;          // CQL_NO_PAIR_BWD2: no CTA-pair bwd2
+  bool no_pair_bwd2_small;    // CQL_NO_PAIR_BWD2_SMALL: the small (actor) bwd2 on one-CTA kernels
+  bool no_small;              // CQL_NO_SMALL: no 32-column work items for the small f16x3 launches
+  bool no_fold;               // CQL_NO_FOLD: separate gradient reduction launch instead of k_adam_pack summing the partials
+  bool no_fused_adam;         // CQL_NO_FUSED_ADAM: k_adam_polyak + pack kernels instead of k_adam_pack (implies CQL_NO_FOLD)
+  bool no_fork;               // CQL_NO_FORK: bwd1 and bwd2 of a job back to back on one stream
+  int big_fork;               // CQL_BIG_FORK=<pairs>: CTA pairs of the big forked bwd1 (0 = serial); -1 = default
+  int h2_cost;                // CQL_H2_COST=<cost>: f16x3 forward's relative cost of an item that stores H2 (0 = default)
+  int pair_swap;              // CQL_PAIR_SWAP=<rank>: cluster rank holding the first half of the CTA-pair operand rows
+  int dp_debug;               // CQL_DP_DEBUG=<mask>: data-parallel exchange timing experiments (dp_peer.cuh; results wrong)
+  bool no_fused_dp;           // CQL_NO_FUSED_DP: data-parallel gradient exchange by cql_dp_allreduce, not inside the kernels
+};
+inline const Switches& switches() {
+  static const Switches s = [] {
+    auto set = [](const char* name) { return std::getenv(name) != nullptr; };
+    auto num = [](const char* name, int unset) { const char* v = std::getenv(name); return v ? std::atoi(v) : unset; };
+    Switches w{};
+    w.skip = num("CQL_SKIP", 0);
+    w.no_pdl = set("CQL_NO_PDL");
+    w.no_pair = set("CQL_NO_PAIR");
+    w.no_pair_bwd1 = set("CQL_NO_PAIR_BWD1");
+    w.no_pair_bwd2 = set("CQL_NO_PAIR_BWD2");
+    w.no_pair_bwd2_small = set("CQL_NO_PAIR_BWD2_SMALL");
+    w.no_small = set("CQL_NO_SMALL");
+    w.no_fold = set("CQL_NO_FOLD");
+    w.no_fused_adam = set("CQL_NO_FUSED_ADAM");
+    w.no_fork = set("CQL_NO_FORK");
+    w.big_fork = num("CQL_BIG_FORK", -1);
+    w.h2_cost = num("CQL_H2_COST", 0);
+    w.pair_swap = num("CQL_PAIR_SWAP", 0);
+    w.dp_debug = num("CQL_DP_DEBUG", 0);
+    w.no_fused_dp = set("CQL_NO_FUSED_DP");
+    return w;
+  }();
+  return s;
+}
 
 struct MdpSession;                   // chunked ingestion session (mdp_gpu.cu)
 // seen-items CSR of a log on the device (mdp_gpu.cu); returns the number of (user, item) entries written
@@ -149,10 +194,7 @@ struct Handle {
   float* small2 = nullptr;         // [C][splits_tc][SMALL_STRIDE] bwd2 partials (b2 | W3 | b3)
   float* pw2_tc = nullptr;         // [C][splits_tc][H*H]
   float4* dX_part = nullptr;       // [C*SLICES][B]
-  unsigned int* b2_tickets = nullptr;   // [C][64] group tickets of the f16x3 bwd2 kernel
   int slots1 = 0, splits_tc = 0, tc_slices = 1;
-  int last_dx_parts = 0;           // parts (nets x column slices) of dX_part written by the last dx launch
-  int last_slots1 = 0, last_splits = 0;   // partial counts of the last weight-gradient backward (summed by k_adam_pack)
   // CTA-pair (cta_group::2) f16x3 kernels: W2 of every slot in the pair layout (mlp_tc_h2.cuh)
   uint8_t* packed_fwd2 = nullptr;  // [(2+2C) slots][H2Cfg::PACKED_NET_BYTES]  B[n][k] = W2[n][k]
   uint8_t* packed_bwd2 = nullptr;  // [(1+C) slots]                           B[n][k] = W2[k][n]
@@ -165,6 +207,7 @@ struct Handle {
 
   // optional event marks for cql_timed_update
   bool timing = false;
+  bool pdl_off = false;            // cql_timed_update: launches without PDL, so the events separate their kernels' durations
   cudaEvent_t ev[16] = {};
 
   MdpSession* mdp = nullptr;       // between cql_mdp_begin and cql_mdp_finish

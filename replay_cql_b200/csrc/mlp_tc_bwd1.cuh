@@ -640,12 +640,10 @@ __device__ __forceinline__ V reduce8(const float* __restrict__ p, int n, size_t 
 
 // block = 32 float4 groups (128 consecutive parameters) x 8 slot-chunks; chunk partials combined through shared
 // memory in chunk order, so the result is independent of scheduling
-// w2_group: the W2 partials were pre-summed in groups of `w2_group` splits by the producing kernel (first slot of
-// every group holds the group's sum); 1 = every split is read
 __global__ void __launch_bounds__(256) k_reduce_grads_tc(const float* __restrict__ small1, int slots1,
                                                          const float* __restrict__ small2, const float* __restrict__ pw2,
                                                          int splits, int in_dim, int out_dim, float* __restrict__ grads,
-                                                         int w2_group = 1, const DpPeer dp = DpPeer{}, int dp_group = 0,
+                                                         const DpPeer dp = DpPeer{}, int dp_group = 0,
                                                          long long dp_off = 0) {
   tc::grid_dep_wait();   /* programmatic dependent launch: the predecessor's results are needed from here on */
  
@@ -660,7 +658,7 @@ __global__ void __launch_bounds__(256) k_reduce_grads_tc(const float* __restrict
     int n = 0;
     size_t stride = 0;
     if (idx >= w2_lo && idx < w2_hi) {
-      base = pw2 + (size_t)net * splits * H * H + (idx - w2_lo); n = (splits + w2_group - 1) / w2_group; stride = (size_t)w2_group * H * H;
+      base = pw2 + (size_t)net * splits * H * H + (idx - w2_lo); n = splits; stride = (size_t)H * H;
     } else if (idx < w2_lo) {
       base = small1 + (size_t)net * slots1 * SMALL_STRIDE + idx; n = slots1; stride = SMALL_STRIDE;
     } else if (idx < total) {         // tail: (idx - H*H) keeps 16-byte alignment; entries past `total` are zero

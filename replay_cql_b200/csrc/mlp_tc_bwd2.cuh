@@ -43,7 +43,6 @@ struct Bwd2Job {
   float* pw2;           // [n_nets][splits][256*256]
   float* small2;        // [n_nets][splits][SMALL_STRIDE]: only b2 | W3 | b3 entries written (same offsets as `small`)
   int rows, n_nets, splits;
-  unsigned int* tickets = nullptr;   // f16x3 kernel: [n_nets][64] group tickets (zero, self-resetting) for the in-kernel partial sums
 };
 
 template <bool TF32, int IN, int OUT>

@@ -756,8 +756,6 @@ __global__ void __launch_bounds__(HCfg::THREADS, 1) tc_bwd1_h_kernel(const Bwd1J
 //   s_A[t] from |W3[:,t]| . max_r |dOut[r,:]|,   s_B[t] from |W1[t,:]| . max_r |x[r,:]| + |b1[t]|
 // with the maxima taken in a pre-pass over the CTA's rows; the partial is unscaled by 1/(s_A[j] s_B[k]) on the way out.
 // A stage holds 32 rows (K = 32 = two MMAs), the same operand bytes as the tf32 kernel's 16 rows.
-constexpr int B2H_GROUP = 4;        // splits per in-kernel partial-sum group
-
 struct B2HCfg {
   static constexpr int ES = 2, EPC = 8, UK = 16;
   static constexpr int RS = 32;                             // rows (K extent) per stage
@@ -1026,34 +1024,6 @@ __global__ void __launch_bounds__(B2HCfg::THREADS, 1) tc_bwd2_h_kernel(const Bwd
   tc_fence_before();
   __syncthreads();
   if (warp == C::PROD_WARPS) tmem_dealloc(tmem, 512);
-  // ---------------- groups of B2H_GROUP splits: the last CTA to finish adds the group's partials (in split order, so the
-  // result does not depend on which CTA is last) into the first member's slot -- the reduction kernel then reads
-  // 4x fewer 256 KB partials
-  if (jb.tickets != nullptr) {
-    __shared__ int is_last;
-    const int g = split / B2H_GROUP, g_lo = g * B2H_GROUP, g_n = min(B2H_GROUP, jb.splits - g_lo);
-    __threadfence();
-    __syncthreads();
-    if (tid == 0) {
-      unsigned int* tk = jb.tickets + net_i * 64 + g;
-      const unsigned int t = atomicAdd(tk, 1u);
-      is_last = (t == (unsigned)g_n - 1) ? 1 : 0;
-      if (is_last) *tk = 0;
-    }
-    __syncthreads();
-    if (is_last && g_n > 1) {
-      __threadfence();
-      float* first = jb.pw2 + ((size_t)net_i * jb.splits + g_lo) * H * H;
-      for (int i = tid * 4; i < H * H; i += C::THREADS * 4) {
-        float4 acc = __ldcg(reinterpret_cast<const float4*>(first + i));
-        for (int m = 1; m < g_n; ++m) {
-          const float4 v = __ldcg(reinterpret_cast<const float4*>(first + (size_t)m * H * H + i));
-          acc.x += v.x; acc.y += v.y; acc.z += v.z; acc.w += v.w;
-        }
-        *reinterpret_cast<float4*>(first + i) = acc;
-      }
-    }
-  }
 }
 
 }  // namespace tc

@@ -7,7 +7,6 @@
 #pragma once
 #include <algorithm>
 #include <utility>
-#include <cstdlib>
 #include "engine.cuh"
 #include "mlp_tc.cuh"
 #include "mlp_tc_ts.cuh"
@@ -758,164 +757,147 @@ __global__ void k_adam_polyak(float* __restrict__ p, float* __restrict__ m, floa
   if (targ) targ[i] = targ[i] * (1.f - tau) + tau * pn;
 }
 
-// ---------------------------------------------------------------- launch helpers
-// Programmatic dependent launch: the kernel may start (barrier init, TMEM allocation) while its predecessor in the
-// stream drains; it executes `griddepcontrol.wait` before touching anything the predecessor wrote.  Only used for
-// kernels that contain that wait (the f16x3 tensor-core kernels).  CQL_NO_PDL=1 switches it off (A/B measurements).
-// cql_timed_update switches PDL off for its one timed step: with PDL a kernel's prologue starts under its predecessor,
-// so a CUDA event recorded between two kernels no longer separates their durations (r01: bwd1 0.118 ms / bwd2 0.003 ms)
-inline bool g_timing_no_pdl = false;
-// CQL_SKIP=<mask>: timing experiments only (results wrong) -- leaves launches out to read their cost on the critical path
-inline bool skip_launch(int bit) {
-  static const int mask = std::getenv("CQL_SKIP") ? std::atoi(std::getenv("CQL_SKIP")) : 0;
-  return (mask & bit) != 0;
-}
+// ---------------------------------------------------------------- launches
+// How a kernel is launched.  pdl: with programmatic dependent launch -- the kernel may start (barrier init, TMEM
+// allocation) while its predecessor in the stream drains; it executes `griddepcontrol.wait` before touching anything the
+// predecessor wrote, and only kernels that contain that wait are launched this way.  skip: the CQL_SKIP bit that leaves
+// the launch out (timing experiments only: results wrong).
+struct LaunchMode { bool pdl; int skip; };
+constexpr LaunchMode PLAIN{false, 0}, PDL{true, 0};
+constexpr LaunchMode pdl_skip(int bit) { return LaunchMode{true, bit}; }
+
+// Every launch of the update goes through here: counted in Handle::launches and error-checked.  PDL is off under
+// CQL_NO_PDL=1 and while Handle::pdl_off is set (cql_timed_update: with PDL a kernel's prologue starts under its
+// predecessor, so a CUDA event recorded between two kernels no longer separates their durations -- r01: bwd1 0.118 ms /
+// bwd2 0.003 ms).
 template <typename... KArgs, typename... Args>
-inline void launch_pdl(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t st, Args&&... args) {
-  static const bool no_pdl_env = std::getenv("CQL_NO_PDL") != nullptr;
-  const bool no_pdl = no_pdl_env || g_timing_no_pdl;
+inline void launch(Handle* h, cudaStream_t st, LaunchMode mode, void (*kernel)(KArgs...), dim3 grid, dim3 block,
+                   size_t smem, Args&&... args) {
+  if (switches().skip & mode.skip) return;
   cudaLaunchConfig_t cfg{};
   cfg.gridDim = grid; cfg.blockDim = block; cfg.dynamicSmemBytes = smem; cfg.stream = st;
   cudaLaunchAttribute attr[1];
   attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
   attr[0].val.programmaticStreamSerializationAllowed = 1;
   cfg.attrs = attr;
-  cfg.numAttrs = no_pdl ? 0 : 1;
+  cfg.numAttrs = mode.pdl && !switches().no_pdl && !h->pdl_off ? 1 : 0;
   CQL_CUDA(cudaLaunchKernelEx(&cfg, kernel, KArgs(std::forward<Args>(args))...));
-}
-
-// same for a kernel compiled with __cluster_dims__(2, 1, 1): grid = 2 x clusters
-template <typename... KArgs, typename... Args>
-inline void launch_pdl_pair(void (*kernel)(KArgs...), int clusters, dim3 block, size_t smem, cudaStream_t st, Args&&... args) {
-  static const bool no_pdl_env = std::getenv("CQL_NO_PDL") != nullptr;
-  const bool no_pdl = no_pdl_env || g_timing_no_pdl;
-  cudaLaunchConfig_t cfg{};
-  cfg.gridDim = dim3(2 * clusters); cfg.blockDim = block; cfg.dynamicSmemBytes = smem; cfg.stream = st;
-  cudaLaunchAttribute attr[1];
-  attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  attr[0].val.programmaticStreamSerializationAllowed = 1;
-  cfg.attrs = attr;
-  cfg.numAttrs = no_pdl ? 0 : 1;
-  CQL_CUDA(cudaLaunchKernelEx(&cfg, kernel, KArgs(std::forward<Args>(args))...));
-}
-
-template <int IN, int OUT>
-inline void launch_fwd(Handle* h, FwdJobs& jobs, cudaStream_t st) {
-  int t = 0;
-  for (int i = 0; i < jobs.n; ++i) {
-    jobs.j[i].tile_begin = t;
-    t += tiles_of(jobs.j[i].rows) * jobs.j[i].n_nets;
-  }
-  jobs.total_tiles = t;
-  if (t == 0) return;
-  mlp_fwd_kernel<IN, OUT><<<t, NT, FWD_SMEM, st>>>(jobs);
   CQL_LAUNCH_CHECK(h);
 }
 
-// ---- tensor-core forward: same job list, W2 from the packed copy, partial sums folded afterwards
-template <bool TF32, int IN, int OUT, bool F16X3 = false>
-inline void launch_fwd_tc(Handle* h, const FwdJobs& jobs, cudaStream_t st, QSrc* defer = nullptr) {
-  using C = std::conditional_t<F16X3, tc::HCfg, tc::Cfg<TF32>>;
-  tc::TcFwdJobs tj{};
-  tj.n = jobs.n;
-  // big launches of the f16x3 path run on CTA pairs (one H1 tile feeds all 256 output columns); CQL_NO_PAIR=1 = A/B switch.
-  // Critics only: the actor has no CTA-pair operand copy (pack_slots, adam_pack), so its forward stays on one-CTA kernels
-  // at any batch size, as its backward does in launch_bwd_tc.
-  bool pair = false;
-  if constexpr (F16X3) {
-    static const bool no_pair = std::getenv("CQL_NO_PAIR") != nullptr;
-    int pair_items = 0;
-    for (int i = 0; i < jobs.n; ++i) pair_items += jobs.j[i].n_nets * ((jobs.j[i].rows + 2 * tc::TM - 1) / (2 * tc::TM));
-    pair = !no_pair && IN == 3 && pair_items >= h->num_sms / 2;
+// ---------------------------------------------------------------- precision
+// cfg.precision as a compile-time parameter of the schedule; with_precision is the one place that maps the one to the other
+enum class Prec { FP32, TF32X3, BF16, F16X3 };
+template <typename F>
+inline void with_precision(const Handle* h, F&& f) {
+  switch (h->cfg.precision) {
+    case CQL_PREC_FP32: f(std::integral_constant<Prec, Prec::FP32>{}); break;
+    case CQL_PREC_TF32X3: f(std::integral_constant<Prec, Prec::TF32X3>{}); break;
+    case CQL_PREC_BF16: f(std::integral_constant<Prec, Prec::BF16>{}); break;
+    case CQL_PREC_F16X3: f(std::integral_constant<Prec, Prec::F16X3>{}); break;
+    default: throw Error{"internal: bad precision"};
   }
-  // small launches (the B-row passes of the actor step: 16-32 work items of 128 columns) run on 32-column work items
-  // instead -- four times as many CTAs, a quarter of the operand load each; CQL_NO_SMALL=1 = A/B switch
-  bool small = false;
-  if constexpr (F16X3) {
-    static const bool no_small = std::getenv("CQL_NO_SMALL") != nullptr;
-    int items128 = 0;
-    for (int i = 0; i < jobs.n; ++i) items128 += jobs.j[i].n_nets * tc::HCfg::SLICES * ((jobs.j[i].rows + tc::TM - 1) / tc::TM);
-    small = !pair && !no_small && items128 * 2 <= h->num_sms;
-  }
-  const int n_slices = small ? tc::HCfgS::SLICES : C::SLICES;
-  const int n_parts = pair ? tc::H2Cfg::PARTS : n_slices;       // layer-3 partial sums per row
-  size_t part_off = 0;
-  int items = 0;
-  float* part_of[4] = {nullptr, nullptr, nullptr, nullptr};
-  for (int i = 0; i < jobs.n; ++i) {
-    const FwdJob& j = jobs.j[i];
-    const int slot = (int)((j.params - h->params) / NET_STRIDE);
-    tj.item_begin[i] = items;
-    items += j.n_nets * n_slices * ((j.rows + tc::TM - 1) / tc::TM);
-    part_of[i] = h->part + part_off;
-    part_off += (size_t)j.n_nets * n_parts * j.rows * OUT;
-    tj.j[i] = tc::TcFwdJob{j.X, j.params,
-                           pair ? h->packed_fwd2 + (size_t)slot * h->packed_net_bytes2 : h->packed_fwd + (size_t)slot * h->packed_net_bytes,
-                           part_of[i], j.h2, j.rows, j.n_nets};
-  }
-  tj.item_begin[jobs.n] = items;
-  { static const char* hc = std::getenv("CQL_H2_COST"); if (hc) tj.h2_cost = std::atoi(hc); }   // tuning knob
-  CQL_REQUIRE(part_off <= h->part_floats, "internal: partial-sum scratch too small");
-  if (items == 0) return;
-  const int grid = items < h->num_sms ? items : h->num_sms;
-  if constexpr (F16X3) {
-    if (pair) launch_pdl_pair(tc::tc_fwd_h2_kernel<IN, OUT>, h->num_sms / 2, dim3(tc::H2Cfg::THREADS), tc::H2Cfg::SMEM_BYTES, st, tj, h->pair_swap_b);
-    else if (small) launch_pdl(tc::tc_fwd_h_kernel<IN, OUT, tc::HCfgS>, dim3(grid), dim3(tc::HCfgS::THREADS), tc::HCfgS::SMEM_BYTES, st, tj);
-    else launch_pdl(tc::tc_fwd_h_kernel<IN, OUT>, dim3(grid), dim3(tc::HCfg::THREADS), tc::HCfg::SMEM_BYTES, st, tj);
-  } else if constexpr (TF32)
-    tc::tc_fwd_ts_kernel<IN, OUT><<<grid, tc::TsCfg::THREADS, tc::TsCfg::SMEM_BYTES, st>>>(tj);
-  else
-    tc::tc_fwd_kernel<TF32, IN, OUT><<<grid, tc::Pipe<TF32, tc::FWD_NPW>::THREADS, tc::FwdSmem<TF32, tc::FWD_NPW>::BYTES, st>>>(tj);
-  CQL_LAUNCH_CHECK(h);
-  if (defer != nullptr && F16X3) {       // the consumers add the partial sums themselves (q_at): no summation launch
-    for (int i = 0; i < jobs.n; ++i) defer[i] = QSrc{part_of[i], jobs.j[i].params, n_parts, jobs.j[i].rows, IN, OUT};
-    return;
-  }
-  if (defer != nullptr)
-    for (int i = 0; i < jobs.n; ++i) defer[i] = QSrc{jobs.j[i].out, jobs.j[i].params, 0, jobs.j[i].rows, IN, OUT};
-  tc::SumJobs sj{};
-  sj.n = jobs.n;
-  int max_n = 0;
-  for (int i = 0; i < jobs.n; ++i) {
-    const FwdJob& j = jobs.j[i];
-    sj.j[i] = {part_of[i], j.params, j.out, j.rows, j.n_nets};
-    max_n = std::max(max_n, j.n_nets * j.rows * OUT);
-  }
-  launch_pdl(tc::k_sum_partials_multi<IN, OUT>, dim3(dim3((max_n + 255) / 256, jobs.n)), dim3(256), 0, st, sj, n_parts);
-  CQL_LAUNCH_CHECK(h);
 }
+// the tensor-core kernel configuration of a precision (f16x3: fp16 hi/lo split; tf32x3 and bf16: mlp_tc.cuh)
+template <Prec P>
+using TcCfg = std::conditional_t<P == Prec::F16X3, tc::HCfg, tc::Cfg<P != Prec::BF16>>;
 
-// defer[i] (optional, one per job) tells the consumer kernels where job i's outputs are (see QSrc)
-template <int IN, int OUT>
-inline void launch_fwd_any(Handle* h, FwdJobs& jobs, cudaStream_t st, QSrc* defer = nullptr) {
-  if (h->cfg.precision == CQL_PREC_TF32X3) launch_fwd_tc<true, IN, OUT>(h, jobs, st, defer);
-  else if (h->cfg.precision == CQL_PREC_F16X3) launch_fwd_tc<true, IN, OUT, true>(h, jobs, st, defer);
-  else if (h->cfg.precision == CQL_PREC_BF16) launch_fwd_tc<false, IN, OUT>(h, jobs, st, defer);
-  else {
-    launch_fwd<IN, OUT>(h, jobs, st);
-    if (defer != nullptr)
-      for (int i = 0; i < jobs.n; ++i) defer[i] = QSrc{jobs.j[i].out, jobs.j[i].params, 0, jobs.j[i].rows, IN, OUT};
+// The critic forward over a job list (fp32: CUDA cores; else tensor cores, W2 from the packed copy).  src[i] tells the
+// consumer kernels where job i's outputs are (see QSrc): f16x3 leaves the layer-3 partial sums to them (q_at); tf32x3
+// and bf16 sum the partials in one more launch.
+template <Prec P, int IN, int OUT>
+inline void launch_fwd(Handle* h, FwdJobs& jobs, cudaStream_t st, QSrc* src) {
+  if constexpr (P == Prec::FP32) {
+    int t = 0;
+    for (int i = 0; i < jobs.n; ++i) {
+      jobs.j[i].tile_begin = t;
+      t += tiles_of(jobs.j[i].rows) * jobs.j[i].n_nets;
+    }
+    jobs.total_tiles = t;
+    if (t > 0) launch(h, st, PLAIN, mlp_fwd_kernel<IN, OUT>, dim3(t), dim3(NT), FWD_SMEM, jobs);
+    for (int i = 0; i < jobs.n; ++i) src[i] = QSrc{jobs.j[i].out, jobs.j[i].params, 0, jobs.j[i].rows, IN, OUT};
+  } else {
+    constexpr bool F16X3 = P == Prec::F16X3;
+    const Switches& sw = switches();
+    tc::TcFwdJobs tj{};
+    tj.n = jobs.n;
+    // big launches of the f16x3 path run on CTA pairs (one H1 tile feeds all 256 output columns).  Critics only: the
+    // actor has no CTA-pair operand copy (pack_slots, adam_pack), so its forward stays on one-CTA kernels at any batch
+    // size, as its backward does in launch_bwd.
+    int pair_items = 0, items128 = 0;
+    for (int i = 0; i < jobs.n; ++i) {
+      pair_items += jobs.j[i].n_nets * ((jobs.j[i].rows + 2 * tc::TM - 1) / (2 * tc::TM));
+      items128 += jobs.j[i].n_nets * tc::HCfg::SLICES * ((jobs.j[i].rows + tc::TM - 1) / tc::TM);
+    }
+    const bool pair = F16X3 && !sw.no_pair && IN == 3 && pair_items >= h->num_sms / 2;
+    // small launches (the B-row passes of the actor step: 16-32 work items of 128 columns) run on 32-column work items
+    // instead -- four times as many CTAs, a quarter of the operand load each
+    const bool small = F16X3 && !pair && !sw.no_small && items128 * 2 <= h->num_sms;
+    const int n_slices = small ? tc::HCfgS::SLICES : TcCfg<P>::SLICES;
+    const int n_parts = pair ? tc::H2Cfg::PARTS : n_slices;       // layer-3 partial sums per row
+    size_t part_off = 0;
+    int items = 0;
+    float* part_of[4] = {nullptr, nullptr, nullptr, nullptr};
+    for (int i = 0; i < jobs.n; ++i) {
+      const FwdJob& j = jobs.j[i];
+      const int slot = (int)((j.params - h->params) / NET_STRIDE);
+      tj.item_begin[i] = items;
+      items += j.n_nets * n_slices * ((j.rows + tc::TM - 1) / tc::TM);
+      part_of[i] = h->part + part_off;
+      part_off += (size_t)j.n_nets * n_parts * j.rows * OUT;
+      tj.j[i] = tc::TcFwdJob{j.X, j.params,
+                             pair ? h->packed_fwd2 + (size_t)slot * h->packed_net_bytes2 : h->packed_fwd + (size_t)slot * h->packed_net_bytes,
+                             part_of[i], j.h2, j.rows, j.n_nets};
+    }
+    tj.item_begin[jobs.n] = items;
+    tj.h2_cost = sw.h2_cost;
+    CQL_REQUIRE(part_off <= h->part_floats, "internal: partial-sum scratch too small");
+    if (items == 0) return;
+    const int grid = items < h->num_sms ? items : h->num_sms;
+    if constexpr (F16X3) {
+      if (pair)
+        launch(h, st, PDL, tc::tc_fwd_h2_kernel<IN, OUT>, dim3(2 * (h->num_sms / 2)), dim3(tc::H2Cfg::THREADS),
+               tc::H2Cfg::SMEM_BYTES, tj, h->pair_swap_b);
+      else if (small)
+        launch(h, st, PDL, tc::tc_fwd_h_kernel<IN, OUT, tc::HCfgS>, dim3(grid), dim3(tc::HCfgS::THREADS), tc::HCfgS::SMEM_BYTES, tj);
+      else
+        launch(h, st, PDL, tc::tc_fwd_h_kernel<IN, OUT>, dim3(grid), dim3(tc::HCfg::THREADS), tc::HCfg::SMEM_BYTES, tj);
+      for (int i = 0; i < jobs.n; ++i) src[i] = QSrc{part_of[i], jobs.j[i].params, n_parts, jobs.j[i].rows, IN, OUT};
+    } else {
+      if constexpr (P == Prec::TF32X3)
+        launch(h, st, PLAIN, tc::tc_fwd_ts_kernel<IN, OUT>, dim3(grid), dim3(tc::TsCfg::THREADS), tc::TsCfg::SMEM_BYTES, tj);
+      else
+        launch(h, st, PLAIN, tc::tc_fwd_kernel<false, IN, OUT>, dim3(grid), dim3(tc::Pipe<false, tc::FWD_NPW>::THREADS),
+               tc::FwdSmem<false, tc::FWD_NPW>::BYTES, tj);
+      tc::SumJobs sj{};
+      sj.n = jobs.n;
+      int max_n = 0;
+      for (int i = 0; i < jobs.n; ++i) {
+        const FwdJob& j = jobs.j[i];
+        sj.j[i] = {part_of[i], j.params, j.out, j.rows, j.n_nets};
+        max_n = std::max(max_n, j.n_nets * j.rows * OUT);
+        src[i] = QSrc{j.out, j.params, 0, j.rows, IN, OUT};
+      }
+      launch(h, st, PDL, tc::k_sum_partials_multi<IN, OUT>, dim3((max_n + 255) / 256, jobs.n), dim3(256), 0, sj, n_parts);
+    }
   }
 }
 
 // refresh the packed (tensor-core operand layout) copies of W2 -- forward orientation for every listed slot,
-// plus W2^T for the trainable ones (slot <= C) -- in ONE launch
+// plus W2^T for the trainable ones (slot <= C) -- in ONE launch (f16x3: one more for the critics' CTA-pair layout)
+template <Prec P>
 inline void pack_slots(Handle* h, const int* slots, int n_slots, cudaStream_t st) {
-  if (h->cfg.precision == CQL_PREC_FP32 || n_slots == 0) return;
-  tc::PackJobs jobs{}, jobs_h{};      // jobs_h: forward copies in the fp16 hi|lo layout (f16x3 mode)
-  const bool f16 = h->cfg.precision == CQL_PREC_F16X3;
+  if (P == Prec::FP32 || n_slots == 0) return;
+  tc::PackJobs jobs{};
   for (int i = 0; i < n_slots; ++i) {
     const int slot = slots[i];
     const bool is_actor = slot == slot_actor() || slot == slot_targ_actor(h->C);
     const int in_dim = is_actor ? 2 : 3;
-    tc::PackJobs& fj = f16 ? jobs_h : jobs;
-    fj.j[fj.n++] = {h->net_params(slot), h->packed_fwd + (size_t)slot * h->packed_net_bytes, in_dim, 0};
-    tc::PackJobs& bj = f16 ? jobs_h : jobs;
-    if (slot <= h->C) bj.j[bj.n++] = {h->net_params(slot), h->packed_bwd + (size_t)slot * h->packed_net_bytes_bwd, in_dim, 1};
+    jobs.j[jobs.n++] = {h->net_params(slot), h->packed_fwd + (size_t)slot * h->packed_net_bytes, in_dim, 0};
+    if (slot <= h->C) jobs.j[jobs.n++] = {h->net_params(slot), h->packed_bwd + (size_t)slot * h->packed_net_bytes_bwd, in_dim, 1};
   }
-  if (jobs_h.n) {
-    launch_pdl(tc::k_pack_multi_h, dim3(dim3(H * 32 / 256, jobs_h.n)), dim3(256), 0, st, jobs_h, 2);
-    CQL_LAUNCH_CHECK(h);
+  if constexpr (P == Prec::F16X3) {    // the fp16 hi|lo layout
+    launch(h, st, PDL, tc::k_pack_multi_h, dim3(H * 32 / 256, jobs.n), dim3(256), 0, jobs, 2);
     tc::PackJobs jp{};                // the same operands in the CTA-pair layout
     for (int i = 0; i < n_slots; ++i) {
       const int slot = slots[i];
@@ -924,163 +906,203 @@ inline void pack_slots(Handle* h, const int* slots, int n_slots, cudaStream_t st
       jp.j[jp.n++] = {h->net_params(slot), h->packed_fwd2 + (size_t)slot * h->packed_net_bytes2, 3, 0};
       if (slot <= h->C) jp.j[jp.n++] = {h->net_params(slot), h->packed_bwd2 + (size_t)slot * h->packed_net_bytes2, 3, 1};
     }
-    if (jp.n) {
-      launch_pdl(tc::k_pack_pair_h, dim3(dim3(H * 32 / 256, jp.n)), dim3(256), 0, st, jp, 2);
-      CQL_LAUNCH_CHECK(h);
-    }
-  }
-  if (jobs.n == 0) return;
-  if (h->cfg.precision != CQL_PREC_BF16) {
-    const int chunks = H * (H / tc::Cfg<true>::EPC);
-    tc::k_pack_multi<true><<<dim3((chunks + 255) / 256, jobs.n), 256, 0, st>>>(jobs);
+    if (jp.n) launch(h, st, PDL, tc::k_pack_pair_h, dim3(H * 32 / 256, jp.n), dim3(256), 0, jp, 2);
   } else {
-    const int chunks = H * (H / tc::Cfg<false>::EPC);
-    tc::k_pack_multi<false><<<dim3((chunks + 255) / 256, jobs.n), 256, 0, st>>>(jobs);
+    constexpr bool TF32 = P == Prec::TF32X3;
+    const int chunks = H * (H / tc::Cfg<TF32>::EPC);
+    launch(h, st, PLAIN, tc::k_pack_multi<TF32>, dim3((chunks + 255) / 256, jobs.n), dim3(256), 0, jobs);
   }
-  CQL_LAUNCH_CHECK(h);
 }
-inline void pack_weights(Handle* h, int slot, int n_slots, int /*in_dim*/, cudaStream_t st) {
+template <Prec P>
+inline void pack_weights(Handle* h, int slot, int n_slots, cudaStream_t st) {
   int slots[8];
   for (int i = 0; i < n_slots; ++i) slots[i] = slot + i;
-  pack_slots(h, slots, n_slots, st);
+  pack_slots<P>(h, slots, n_slots, st);
+}
+
+template <Prec P>
+inline void pack_all_weights(Handle* h, cudaStream_t st) {
+  if constexpr (P == Prec::F16X3)
+    launch(h, st, PLAIN, tc::k_w2max_init, dim3(2 + 2 * h->C), dim3(256), 0, h->params, 2 + 2 * h->C, h->w2max);
+  pack_weights<P>(h, slot_actor(), 1, st);
+  pack_weights<P>(h, slot_critic(0), h->C, st);
+  pack_weights<P>(h, slot_targ_actor(h->C), 1, st);
+  pack_weights<P>(h, slot_targ_critic(h->C, 0), h->C, st);
 }
 
 // f16x3 at world size 1: k_adam_pack sums the backward's gradient partials itself and the weight-gradient bwd1 kernels
 // zero their own partial slots -- no k_reduce_grads_tc launch and no memset node per gradient group, so every edge of
 // the backward chain is a programmatic one.  Data-parallel runs keep the separate reduction: it is where their gradient
-// exchange starts (phase A of dp_peer.cuh, or the exchange between cql_step_phase calls).  CQL_NO_FOLD=1 = A/B switch.
+// exchange starts (phase A of dp_peer.cuh, or the exchange between cql_step_phase calls).
+template <Prec P>
 inline bool fold_grads(const Handle* h) {
-  static const bool no_fold = std::getenv("CQL_NO_FOLD") != nullptr || std::getenv("CQL_NO_FUSED_ADAM") != nullptr;
-  return !no_fold && h->cfg.precision == CQL_PREC_F16X3 && h->cfg.world_size <= 1 && h->dp.world <= 1;
+  const Switches& sw = switches();
+  return P == Prec::F16X3 && !sw.no_fold && !sw.no_fused_adam && h->cfg.world_size <= 1 && h->dp.world <= 1;
 }
 
-// ---- tensor-core backward of one job: bwd1 (dH1, dW1, db1, dx) + bwd2 (dW2, db2, dW3, db3) + reduce
-template <bool TF32, int IN, int OUT, bool WGRADS, bool DX, bool F16X3 = false>
-inline void launch_bwd_tc(Handle* h, const BwdJob& jb, float* grads_out, cudaStream_t st, int mark_mid = -1, int mark_end = -1) {
-  using C = std::conditional_t<F16X3, tc::HCfg, tc::Cfg<TF32>>;
-  const int slot = (int)((jb.params - h->params) / NET_STRIDE);
-  const int tiles = (jb.rows + tc::TM - 1) / tc::TM;
-  const int items = jb.n_nets * C::SLICES * tiles;
-  // big launches of the f16x3 path run on CTA pairs (mlp_tc_h2.cuh): one dZ2 tile feeds all 256 columns of dH1
-  bool pair = false;
-  if constexpr (F16X3) {
-    static const bool no_pair = std::getenv("CQL_NO_PAIR") != nullptr || std::getenv("CQL_NO_PAIR_BWD1") != nullptr;
-    pair = !no_pair && IN == 3 && jb.n_nets * ((jb.rows + 2 * tc::TM - 1) / (2 * tc::TM)) >= h->num_sms / 2;
-  }
-  bool small = false;
-  if constexpr (F16X3) {
-    static const bool no_small = std::getenv("CQL_NO_SMALL") != nullptr;
-    small = !pair && !no_small && items * 2 <= h->num_sms;
-  }
-  const int n_slices = small ? tc::HCfgS::SLICES : C::SLICES;
-  const int items_s = jb.n_nets * n_slices * tiles;
-  // The big launch's bwd1 and bwd2 are independent too and run SIDE BY SIDE: bwd1 on 30 of the 74 CTA pairs, bwd2 on the
-  // other 44 (22 splits per critic).  Back to back on all SMs each, the fixed cost of either kernel -- prologue,
-  // accumulator dump (half as many dW2 partials now), tail -- was serial: with the main loop skipped bwd2 still took
-  // 16 of its 44 us.  Measured sweep of the bwd1 share (pairs -> us per update): 74 (serial) 222.4, 46 238, 42 229,
-  // 38 222.5, 34 216.5, 32 213.1, 30 212.7, 28 212.9, 26 219, 22 230.  CQL_BIG_FORK=<pairs> overrides (0 = serial).
-  static const bool no_fork = std::getenv("CQL_NO_FORK") != nullptr;      // A/B switch for measurements
-  static const int big_fork = std::getenv("CQL_BIG_FORK") ? std::atoi(std::getenv("CQL_BIG_FORK")) : -1;
-  const int fork_pairs = big_fork >= 0 ? big_fork : (h->num_sms / 2) * 30 / 74;
-  const int clusters1 = (pair && WGRADS && fork_pairs > 0 && fork_pairs < h->num_sms / 2 && !no_fork && !h->timing && h->side_stream != nullptr)
-                            ? fork_pairs : h->num_sms / 2;
-  const int grid1 = pair ? 2 * clusters1 : (items_s < h->num_sms ? items_s : h->num_sms);
-  h->last_dx_parts = jb.n_nets * (pair ? (int)tc::H2Cfg::PARTS : n_slices);
-  const int slots1 = (F16X3 ? 2 : 4) * grid1;      // f16x3: one slot per (CTA, epilogue group)
-  const bool fold = F16X3 && WGRADS && fold_grads(h);
-  if (WGRADS && !fold) CQL_CUDA(cudaMemsetAsync(h->small1, 0, (size_t)jb.n_nets * slots1 * SMALL_STRIDE * sizeof(float), st));
-  tc::Bwd1Job j1{jb.X, jb.dOut, jb.h2, jb.params,
-                 pair ? h->packed_bwd2 + (size_t)slot * h->packed_net_bytes2 : h->packed_bwd + (size_t)slot * h->packed_net_bytes_bwd,
-                 h->small1, DX ? h->dX_part : nullptr, jb.rows, jb.n_nets, slots1};
-  j1.q_part = jb.q_part; j1.q_parts = jb.q_parts; j1.dq_scale = jb.dq_scale;
-  j1.zero_small1 = fold ? 1 : 0;
-  // bwd1 and bwd2 of one job are independent (both only read X, dOut, H2).  For the small jobs (the actor's B rows:
-  // a few dozen CTAs each) they run side by side on a forked branch -- the fork/join is captured into the step graph.
-  constexpr int RS2 = F16X3 ? tc::B2HCfg::RS : tc::B2Cfg<TF32>::RS;
-  const int n_stage = (jb.rows + RS2 - 1) / RS2;
-  int splits = h->num_sms / jb.n_nets;
-  if (splits > n_stage) splits = n_stage;      // (fewer, longer splits for the small jobs were measured: slower)
-  if (splits > h->splits_tc) splits = h->splits_tc;
-  if (splits < 1) splits = 1;
-  bool pair2 = false;                            // dW2 on CTA pairs (A operand in tensor memory): the big launches
-  if constexpr (F16X3) {
-    static const bool no_pair2 = std::getenv("CQL_NO_PAIR") != nullptr || std::getenv("CQL_NO_PAIR_BWD2") != nullptr;
-    static const bool no_pair2_small = std::getenv("CQL_NO_PAIR_BWD2_SMALL") != nullptr;
-    pair2 = !no_pair2 && (pair || !no_pair2_small);     // also the small (actor) launch: a pair CTA dumps half an accumulator
-    if (pair2) splits = std::max(1, std::min(n_stage, (h->num_sms / 2) / jb.n_nets));
-    if (pair2 && pair && clusters1 < h->num_sms / 2) splits = std::max(1, (h->num_sms / 2 - clusters1) / jb.n_nets);
-  }
-  const bool fork = WGRADS && !no_fork && !h->timing && h->side_stream != nullptr &&
-                    grid1 + (pair2 ? 2 : 1) * splits * jb.n_nets <= h->num_sms;
-  cudaStream_t st2 = st;
-  if (fork) {
-    CQL_CUDA(cudaEventRecord(h->ev_fork, st));
-    CQL_CUDA(cudaStreamWaitEvent(h->side_stream, h->ev_fork, 0));
-    st2 = h->side_stream;
-  }
-  if constexpr (F16X3) {
-    if (pair) launch_pdl_pair(tc::tc_bwd1_h2_kernel<IN, OUT, WGRADS, DX>, clusters1, dim3(tc::H2Cfg::THREADS), tc::H2B1Cfg::SMEM_BYTES, st, j1, h->pair_swap_b);
-    else if (small) launch_pdl(tc::tc_bwd1_h_kernel<IN, OUT, WGRADS, DX, tc::HCfgS>, dim3(grid1), dim3(tc::HCfgS::THREADS), tc::HCfgS::SMEM_BYTES, st, j1);
-    else launch_pdl(tc::tc_bwd1_h_kernel<IN, OUT, WGRADS, DX>, dim3(grid1), dim3(tc::HCfg::THREADS), tc::HCfg::SMEM_BYTES, st, j1);
-  } else if constexpr (TF32)
-    tc::tc_bwd1_ts_kernel<IN, OUT, WGRADS, DX><<<grid1, tc::TsCfg::THREADS, tc::TsCfg::SMEM_BYTES, st>>>(j1);
-  else
-    tc::tc_bwd1_kernel<TF32, IN, OUT, WGRADS, DX><<<grid1, tc::Pipe<TF32, tc::BWD1_NPW>::THREADS, tc::FwdSmem<TF32, tc::BWD1_NPW>::BYTES, st>>>(j1);
-  CQL_LAUNCH_CHECK(h);
-  if (mark_mid >= 0) mark(h, st, mark_mid);
-  if (!WGRADS) return;
-  tc::Bwd2Job j2{jb.X, jb.dOut, jb.h2, jb.params, h->pw2_tc, h->small2, jb.rows, jb.n_nets, splits};
-  constexpr bool GROUP_SUM = false;   // in-kernel group sums of the dW2 partials: measured slower (one CTA re-reads 1 MB at the tail)
-  if (F16X3 && GROUP_SUM) j2.tickets = h->b2_tickets;
-  if constexpr (F16X3) {
-    if (pair2) {
-      static const bool no_pdl_env = std::getenv("CQL_NO_PDL") != nullptr;
-      cudaLaunchConfig_t cfg{};
-      cfg.gridDim = dim3(2 * splits, jb.n_nets); cfg.blockDim = dim3(tc::B2PCfg::THREADS); cfg.dynamicSmemBytes = tc::B2PCfg::BYTES; cfg.stream = st2;
-      cudaLaunchAttribute attr[1];
-      attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-      attr[0].val.programmaticStreamSerializationAllowed = 1;
-      cfg.attrs = attr;
-      cfg.numAttrs = (no_pdl_env || g_timing_no_pdl) ? 0 : 1;
-      CQL_CUDA(cudaLaunchKernelEx(&cfg, tc::tc_bwd2_h2_kernel<IN, OUT>, j2));
-    } else {
-      launch_pdl(tc::tc_bwd2_h_kernel<IN, OUT>, dim3(splits, jb.n_nets), dim3(tc::B2HCfg::THREADS), tc::B2HCfg::BYTES, st2, j2);
-    }
-  } else
-    tc::tc_bwd2_kernel<TF32, IN, OUT><<<dim3(splits, jb.n_nets), tc::B2_THREADS, tc::B2Cfg<TF32>::BYTES, st2>>>(j2);
-  CQL_LAUNCH_CHECK(h);
-  if (fork) {
-    CQL_CUDA(cudaEventRecord(h->ev_join, st2));
-    CQL_CUDA(cudaStreamWaitEvent(st, h->ev_join, 0));
-  }
-  if (mark_end >= 0) mark(h, st, mark_end);
-  if (fold) {                          // summed by the group's k_adam_pack
-    h->last_slots1 = slots1;
-    h->last_splits = splits;
-    return;
-  }
-  if (!skip_launch(64))
-    launch_pdl(tc::k_reduce_grads_tc, dim3(dim3((NET_STRIDE / 4 + 31) / 32, jb.n_nets)), dim3(256), 0, st, h->small1, slots1, h->small2, h->pw2_tc,
-                                                                                  splits, IN, OUT, grads_out,
-                                                                                  (F16X3 && GROUP_SUM) ? tc::B2H_GROUP : 1,
-                                                                                  h->dp_fused ? h->dp : DpPeer{}, IN == 3 ? 1 : 2,
-                                                                                  (long long)(IN == 3 ? NET_STRIDE : 0));
-  CQL_LAUNCH_CHECK(h);
+// The backward jobs of an update.  The critic and actor jobs are built in one phase and their gradients consumed by the
+// optimizer step of the next, which re-derives the job's BwdPlan from the same job.
+inline BwdJob critic_bwd_job(Handle* h) {
+  return BwdJob{h->XC, h->dQ, h->h2C, h->net_params(slot_critic(0)), h->smallC, nullptr, h->pw2C, h->B * (3 * h->n + 1),
+                h->C, h->splitsC};
 }
+inline BwdJob actor_bwd_job(Handle* h) {
+  return BwdJob{h->XA, h->dOutA, h->h2A, h->net_params(slot_actor()), h->smallA, nullptr, h->pw2A, h->B, 1, h->splitsA};
+}
+
+// Launch geometry of one backward job and the partial counts its consumers sum: k_reduce_grads_tc or k_adam_pack
+// (slots1 bwd1 partials, splits bwd2 partials per net) and k_actor_dout (dx_parts partials of dx).  A function of the
+// job and the handle alone.
+struct BwdPlan {
+  bool pair = false, small = false, pair2 = false, fork = false, fold = false;
+  int clusters1 = 0, grid1 = 0, slots1 = 0, splits = 0;
+  const float4* dx = nullptr;
+  int dx_parts = 0;
+};
+template <Prec P, int IN, int OUT, bool WGRADS, bool DX>
+inline BwdPlan bwd_plan(const Handle* h, const BwdJob& jb) {
+  BwdPlan p{};
+  if constexpr (P == Prec::FP32) {
+    p.splits = jb.splits;
+    p.dx = jb.dX;
+    p.dx_parts = jb.n_nets;            // parts = critics (x column slices)
+  } else {
+    constexpr bool F16X3 = P == Prec::F16X3;
+    const Switches& sw = switches();
+    const int tiles = (jb.rows + tc::TM - 1) / tc::TM;
+    const int items = jb.n_nets * TcCfg<P>::SLICES * tiles;
+    // big launches of the f16x3 path run on CTA pairs (mlp_tc_h2.cuh): one dZ2 tile feeds all 256 columns of dH1
+    p.pair = F16X3 && !sw.no_pair && !sw.no_pair_bwd1 && IN == 3 &&
+             jb.n_nets * ((jb.rows + 2 * tc::TM - 1) / (2 * tc::TM)) >= h->num_sms / 2;
+    p.small = F16X3 && !p.pair && !sw.no_small && items * 2 <= h->num_sms;
+    const int n_slices = p.small ? tc::HCfgS::SLICES : TcCfg<P>::SLICES;
+    const int items_s = jb.n_nets * n_slices * tiles;
+    // The big launch's bwd1 and bwd2 are independent too and run SIDE BY SIDE: bwd1 on 30 of the 74 CTA pairs, bwd2 on
+    // the other 44 (22 splits per critic).  Back to back on all SMs each, the fixed cost of either kernel -- prologue,
+    // accumulator dump (half as many dW2 partials now), tail -- was serial: with the main loop skipped bwd2 still took
+    // 16 of its 44 us.  Measured sweep of the bwd1 share (pairs -> us per update): 74 (serial) 222.4, 46 238, 42 229,
+    // 38 222.5, 34 216.5, 32 213.1, 30 212.7, 28 212.9, 26 219, 22 230.  CQL_BIG_FORK=<pairs> overrides (0 = serial).
+    const bool may_fork = WGRADS && !sw.no_fork && !h->timing && h->side_stream != nullptr;
+    const int fork_pairs = sw.big_fork >= 0 ? sw.big_fork : (h->num_sms / 2) * 30 / 74;
+    p.clusters1 = (p.pair && may_fork && fork_pairs > 0 && fork_pairs < h->num_sms / 2) ? fork_pairs : h->num_sms / 2;
+    p.grid1 = p.pair ? 2 * p.clusters1 : (items_s < h->num_sms ? items_s : h->num_sms);
+    p.slots1 = (F16X3 ? 2 : 4) * p.grid1;      // f16x3: one slot per (CTA, epilogue group)
+    p.dx = h->dX_part;
+    p.dx_parts = jb.n_nets * (p.pair ? (int)tc::H2Cfg::PARTS : n_slices);
+    p.fold = WGRADS && fold_grads<P>(h);
+    // bwd1 and bwd2 of one job are independent (both only read X, dOut, H2).  For the small jobs (the actor's B rows:
+    // a few dozen CTAs each) they run side by side on a forked branch -- the fork/join is captured into the step graph.
+    constexpr int RS2 = F16X3 ? tc::B2HCfg::RS : tc::B2Cfg<P != Prec::BF16>::RS;
+    const int n_stage = (jb.rows + RS2 - 1) / RS2;
+    int splits = h->num_sms / jb.n_nets;
+    if (splits > n_stage) splits = n_stage;      // (fewer, longer splits for the small jobs were measured: slower)
+    if (splits > h->splits_tc) splits = h->splits_tc;
+    if (splits < 1) splits = 1;
+    if constexpr (F16X3) {                       // dW2 on CTA pairs (A operand in tensor memory): the big launches
+      p.pair2 = !sw.no_pair && !sw.no_pair_bwd2 && (p.pair || !sw.no_pair_bwd2_small);   // also the small (actor)
+      if (p.pair2) splits = std::max(1, std::min(n_stage, (h->num_sms / 2) / jb.n_nets));   // launch: a pair CTA dumps
+      if (p.pair2 && p.pair && p.clusters1 < h->num_sms / 2)                                // half an accumulator
+        splits = std::max(1, (h->num_sms / 2 - p.clusters1) / jb.n_nets);
+    }
+    p.splits = splits;
+    p.fork = may_fork && p.grid1 + (p.pair2 ? 2 : 1) * splits * jb.n_nets <= h->num_sms;
+  }
+  return p;
+}
+
+// event marks of cql_timed_update inside a backward job (-1: none): mid after bwd1, end after bwd2, done after the job
+// (fp32 records `done` ahead of its reduction launch, so the actor-backward duration leaves that launch out there)
+struct BwdMarks { int mid = -1, end = -1, done = -1; };
+
+// The backward of one job: bwd1 (dH1, dW1, db1, dx), with WGRADS bwd2 (dW2, db2, dW3, db3) and the reduction of their
+// partials into grads_out -- unless k_adam_pack sums them (plan.fold).
+template <Prec P, int IN, int OUT, bool WGRADS, bool DX>
+inline BwdPlan launch_bwd(Handle* h, const BwdJob& jb, float* grads_out, cudaStream_t st, BwdMarks mk = {}) {
+  auto mark_at = [&](int i) { if (i >= 0) mark(h, st, i); };
+  const BwdPlan p = bwd_plan<P, IN, OUT, WGRADS, DX>(h, jb);
+  if constexpr (P == Prec::FP32) {
+    launch(h, st, PLAIN, mlp_bwd1_kernel<IN, OUT, WGRADS, DX>, dim3(tiles_of(jb.rows) * jb.n_nets), dim3(NT), BWD1_SMEM, jb);
+    mark_at(mk.mid);
+    if (!WGRADS) return p;
+    launch(h, st, PLAIN, mlp_bwd2_kernel<IN, OUT>, dim3(4, jb.splits, jb.n_nets), dim3(NT), BWD2_SMEM, jb);
+    mark_at(mk.end);
+    mark_at(mk.done);
+    launch(h, st, PLAIN, k_reduce_grads, dim3((NET_STRIDE + 255) / 256, jb.n_nets), dim3(256), 0, jb.small, jb.pw2, IN, OUT,
+           tiles_of(jb.rows), jb.splits, grads_out);
+  } else {
+    constexpr bool F16X3 = P == Prec::F16X3;
+    const int slot = (int)((jb.params - h->params) / NET_STRIDE);
+    if (WGRADS && !p.fold) CQL_CUDA(cudaMemsetAsync(h->small1, 0, (size_t)jb.n_nets * p.slots1 * SMALL_STRIDE * sizeof(float), st));
+    tc::Bwd1Job j1{jb.X, jb.dOut, jb.h2, jb.params,
+                   p.pair ? h->packed_bwd2 + (size_t)slot * h->packed_net_bytes2 : h->packed_bwd + (size_t)slot * h->packed_net_bytes_bwd,
+                   h->small1, DX ? h->dX_part : nullptr, jb.rows, jb.n_nets, p.slots1};
+    j1.q_part = jb.q_part; j1.q_parts = jb.q_parts; j1.dq_scale = jb.dq_scale;
+    j1.zero_small1 = p.fold ? 1 : 0;
+    cudaStream_t st2 = st;
+    if (p.fork) {
+      CQL_CUDA(cudaEventRecord(h->ev_fork, st));
+      CQL_CUDA(cudaStreamWaitEvent(h->side_stream, h->ev_fork, 0));
+      st2 = h->side_stream;
+    }
+    if constexpr (F16X3) {
+      if (p.pair)
+        launch(h, st, PDL, tc::tc_bwd1_h2_kernel<IN, OUT, WGRADS, DX>, dim3(2 * p.clusters1), dim3(tc::H2Cfg::THREADS),
+               tc::H2B1Cfg::SMEM_BYTES, j1, h->pair_swap_b);
+      else if (p.small)
+        launch(h, st, PDL, tc::tc_bwd1_h_kernel<IN, OUT, WGRADS, DX, tc::HCfgS>, dim3(p.grid1), dim3(tc::HCfgS::THREADS),
+               tc::HCfgS::SMEM_BYTES, j1);
+      else
+        launch(h, st, PDL, tc::tc_bwd1_h_kernel<IN, OUT, WGRADS, DX>, dim3(p.grid1), dim3(tc::HCfg::THREADS), tc::HCfg::SMEM_BYTES, j1);
+    } else if constexpr (P == Prec::TF32X3) {
+      launch(h, st, PLAIN, tc::tc_bwd1_ts_kernel<IN, OUT, WGRADS, DX>, dim3(p.grid1), dim3(tc::TsCfg::THREADS), tc::TsCfg::SMEM_BYTES, j1);
+    } else {
+      launch(h, st, PLAIN, tc::tc_bwd1_kernel<false, IN, OUT, WGRADS, DX>, dim3(p.grid1), dim3(tc::Pipe<false, tc::BWD1_NPW>::THREADS),
+             tc::FwdSmem<false, tc::BWD1_NPW>::BYTES, j1);
+    }
+    mark_at(mk.mid);
+    if (!WGRADS) return p;
+    tc::Bwd2Job j2{jb.X, jb.dOut, jb.h2, jb.params, h->pw2_tc, h->small2, jb.rows, jb.n_nets, p.splits};
+    if constexpr (F16X3) {
+      if (p.pair2)
+        launch(h, st2, PDL, tc::tc_bwd2_h2_kernel<IN, OUT>, dim3(2 * p.splits, jb.n_nets), dim3(tc::B2PCfg::THREADS), tc::B2PCfg::BYTES, j2);
+      else
+        launch(h, st2, PDL, tc::tc_bwd2_h_kernel<IN, OUT>, dim3(p.splits, jb.n_nets), dim3(tc::B2HCfg::THREADS), tc::B2HCfg::BYTES, j2);
+    } else {
+      constexpr bool TF32 = P == Prec::TF32X3;
+      launch(h, st2, PLAIN, tc::tc_bwd2_kernel<TF32, IN, OUT>, dim3(p.splits, jb.n_nets), dim3(tc::B2_THREADS), tc::B2Cfg<TF32>::BYTES, j2);
+    }
+    if (p.fork) {
+      CQL_CUDA(cudaEventRecord(h->ev_join, st2));
+      CQL_CUDA(cudaStreamWaitEvent(st, h->ev_join, 0));
+    }
+    mark_at(mk.end);
+    if (!p.fold)
+      launch(h, st, pdl_skip(64), tc::k_reduce_grads_tc, dim3((NET_STRIDE / 4 + 31) / 32, jb.n_nets), dim3(256), 0, h->small1,
+             p.slots1, h->small2, h->pw2_tc, p.splits, IN, OUT, grads_out, h->dp_fused ? h->dp : DpPeer{}, IN == 3 ? 1 : 2,
+             (long long)(IN == 3 ? NET_STRIDE : 0));
+    mark_at(mk.done);
+  }
+  return p;
+}
+
+// the networks one optimizer step updates: the critics or the actor, each with its Polyak-averaged target copy
+struct NetGroup { int first_slot, n_nets, in_dim, out_dim; float lr; };
+inline NetGroup critic_group(const Handle* h) { return NetGroup{slot_critic(0), h->C, 3, 1, h->cfg.critic_lr}; }
+inline NetGroup actor_group(const Handle* h) { return NetGroup{slot_actor(), 1, 2, 2, h->cfg.actor_lr}; }
 
 // f16x3: Adam + Polyak + every operand copy of W2 (network and target, both orientations, both layouts) in one launch
-inline void adam_pack(Handle* h, int first_slot, int n_nets, int in_dim, int out_dim, float lr, cudaStream_t st, bool last = false) {
+inline void adam_pack(Handle* h, const NetGroup& g, const BwdPlan& plan, cudaStream_t st, bool last) {
   const cql_config& c = h->cfg;
+  const bool critic = g.in_dim == 3;
   tc::AdamPackJobs j{};
-  j.in_dim = in_dim; j.out_dim = out_dim;
-  j.lr = lr; j.beta1 = c.beta1; j.beta2 = c.beta2; j.eps = c.adam_eps; j.tau = c.tau;
+  j.in_dim = g.in_dim; j.out_dim = g.out_dim;
+  j.lr = g.lr; j.beta1 = c.beta1; j.beta2 = c.beta2; j.eps = c.adam_eps; j.tau = c.tau;
   j.step_inc = last ? h->step_dev : nullptr;
   j.dp = h->dp_fused ? h->dp : DpPeer{};
-  j.dp_group = in_dim == 3 ? 1 : 2;
-  j.dp_off = (long long)first_slot * NET_STRIDE;       // staging layout = gradient buffer layout [actor | critics | scalars]
-  for (int i = 0; i < n_nets; ++i) {
-    const int slot = first_slot + i, tslot = slot + 1 + h->C;       // [actor | critics | targ_actor | targ_critics]
-    const bool critic = in_dim == 3;
+  j.dp_group = critic ? 1 : 2;
+  j.dp_off = (long long)g.first_slot * NET_STRIDE;       // staging layout = gradient buffer layout [actor | critics | scalars]
+  for (int i = 0; i < g.n_nets; ++i) {
+    const int slot = g.first_slot + i, tslot = slot + 1 + h->C;       // [actor | critics | targ_actor | targ_critics]
     tc::AdamPackNet& n = j.n[i];
     n.p = h->net_params(slot);
     n.m = h->adam_m + (size_t)slot * NET_STRIDE;
@@ -1095,39 +1117,34 @@ inline void adam_pack(Handle* h, int first_slot, int n_nets, int in_dim, int out
     n.tfwd2 = critic ? h->packed_fwd2 + (size_t)tslot * h->packed_net_bytes2 : nullptr;
     n.w2max = h->w2max + slot * 4;
   }
-  const bool fold = fold_grads(h);
-  if (fold) {                          // the partials of this group's backward (launch_bwd_tc)
+  if (plan.fold) {                     // the partials of this group's backward (launch_bwd)
     j.small1 = h->small1; j.small2 = h->small2; j.pw2 = h->pw2_tc;
-    j.slots1 = h->last_slots1; j.splits = h->last_splits;
+    j.slots1 = plan.slots1; j.splits = plan.splits;
     j.wmax_acc = h->ap_wmax;
   }
-  const int blocks = tc::AP_W2_BLOCKS + (fold ? tc::ap_small_blocks(in_dim, out_dim) : 1);
-  if (!skip_launch(128))
-    launch_pdl(tc::k_adam_pack, dim3(blocks, n_nets), dim3(1024), 0, st, j, h->stepinfo);
-  CQL_LAUNCH_CHECK(h);
+  const int blocks = tc::AP_W2_BLOCKS + (plan.fold ? tc::ap_small_blocks(g.in_dim, g.out_dim) : 1);
+  launch(h, st, pdl_skip(128), tc::k_adam_pack, dim3(blocks, g.n_nets), dim3(1024), 0, j, h->stepinfo);
 }
 
-inline void pack_all_weights(Handle* h, cudaStream_t st) {
-  if (h->cfg.precision == CQL_PREC_F16X3) {
-    tc::k_w2max_init<<<2 + 2 * h->C, 256, 0, st>>>(h->params, 2 + 2 * h->C, h->w2max);
-    CQL_LAUNCH_CHECK(h);
+// Adam + Polyak of one group and the refresh of its packed W2 copies; `last`: the update's final launch, which also counts
+// the step.  plan: the group's backward (launch_bwd), whose partials f16x3 sums here.
+template <Prec P>
+inline void optimizer_step(Handle* h, const NetGroup& g, const BwdPlan& plan, cudaStream_t st, bool last) {
+  if (P == Prec::F16X3 && !switches().no_fused_adam) {
+    adam_pack(h, g, plan, st, last);
+    return;
   }
-  pack_weights(h, slot_actor(), 1, 2, st);
-  pack_weights(h, slot_critic(0), h->C, 3, st);
-  pack_weights(h, slot_targ_actor(h->C), 1, 2, st);
-  pack_weights(h, slot_targ_critic(h->C, 0), h->C, 3, st);
-}
-
-template <int IN, int OUT, bool WGRADS, bool DX>
-inline void launch_bwd1(Handle* h, const BwdJob& jb, cudaStream_t st) {
-  mlp_bwd1_kernel<IN, OUT, WGRADS, DX><<<tiles_of(jb.rows) * jb.n_nets, NT, BWD1_SMEM, st>>>(jb);
-  CQL_LAUNCH_CHECK(h);
-}
-
-template <int IN, int OUT>
-inline void launch_bwd2(Handle* h, const BwdJob& jb, cudaStream_t st) {
-  mlp_bwd2_kernel<IN, OUT><<<dim3(4, jb.splits, jb.n_nets), NT, BWD2_SMEM, st>>>(jb);
-  CQL_LAUNCH_CHECK(h);
+  const cql_config& c = h->cfg;
+  const int64_t cnt = (int64_t)g.n_nets * NET_STRIDE, off = (int64_t)g.first_slot * NET_STRIDE;
+  const int tslot = g.first_slot + 1 + h->C;
+  launch(h, st, PDL, k_adam_polyak, dim3((int)((cnt + 255) / 256)), dim3(256), 0, h->net_params(g.first_slot), h->adam_m + off,
+         h->adam_v + off, h->grads + off, h->net_params(tslot), cnt, g.lr, c.beta1, c.beta2, c.adam_eps, c.tau, h->stepinfo);
+  int slots[2 * CQL_MAX_CRITICS], n = 0;
+  for (int i = 0; i < g.n_nets; ++i) slots[n++] = g.first_slot + i;
+  if (g.in_dim == 3)                   // the target critics' forward (TD target) reads the packed copy; the target actor's none
+    for (int i = 0; i < g.n_nets; ++i) slots[n++] = tslot + i;
+  pack_slots<P>(h, slots, n, st);
+  if (last) launch(h, st, PDL, k_step_end, dim3(1), dim3(1), 0, h->step_dev);
 }
 
 inline LossConsts loss_consts(const Handle* h) {
@@ -1141,6 +1158,7 @@ enum class BatchSource { Sampled, Provided };
 enum class NoiseSource { Philox, Provided };
 
 // phase 0: (sample, noise,) shared actor forward, all critic forwards, scalar gradients
+template <Prec P>
 inline void phase0(Handle* h, cudaStream_t st, BatchSource bs, NoiseSource ns) {
   NvtxRange nvtx("cql.update.phase0: sample, actor forward, critic forwards, temp/alpha gradients");
   const int B = h->B, C = h->C, n3 = 3 * h->n;
@@ -1150,32 +1168,23 @@ inline void phase0(Handle* h, cudaStream_t st, BatchSource bs, NoiseSource ns) {
   if (bs == BatchSource::Sampled && ns == NoiseSource::Philox) {
     CQL_REQUIRE(h->n_trans > 0, "cql_update: no transitions loaded (call cql_load_transitions first)");
     const int64_t nthr = h->noise_floats > B ? h->noise_floats : B;
-    if (!skip_launch(256))
-      launch_pdl(k_step_head, dim3((int)((nthr + 255) / 256)), dim3(256), 0, st, reinterpret_cast<const float4*>(h->table), h->n_trans, h->step_dev,
-                                                          h->stepinfo, c.beta1, c.beta2, B, h->n, c.rank, c.world_size,
-                                                          c.seed, reinterpret_cast<float4*>(h->batch), h->XA, h->noise,
-                                                          h->noise_floats, h->table_sharded ? 0 : c.rank,
-                                                          h->table_sharded ? 1 : c.world_size, h->prep);
-    CQL_LAUNCH_CHECK(h);
+    launch(h, st, pdl_skip(256), k_step_head, dim3((int)((nthr + 255) / 256)), dim3(256), 0, reinterpret_cast<const float4*>(h->table),
+           h->n_trans, h->step_dev, h->stepinfo, c.beta1, c.beta2, B, h->n, c.rank, c.world_size, c.seed,
+           reinterpret_cast<float4*>(h->batch), h->XA, h->noise, h->noise_floats, h->table_sharded ? 0 : c.rank,
+           h->table_sharded ? 1 : c.world_size, h->prep);
   } else {
-    k_step_begin<<<1, 1, 0, st>>>(h->step_dev, h->stepinfo, c.beta1, c.beta2);
-    CQL_LAUNCH_CHECK(h);
+    launch(h, st, PLAIN, k_step_begin, dim3(1), dim3(1), 0, h->step_dev, h->stepinfo, c.beta1, c.beta2);
     if (bs == BatchSource::Sampled) {
       CQL_REQUIRE(h->n_trans > 0, "cql_update: no transitions loaded (call cql_load_transitions first)");
-      k_sample<<<(B + 127) / 128, 128, 0, st>>>(reinterpret_cast<const float4*>(h->table), h->n_trans, nullptr,
-                                                h->step_dev, 0, B, (int64_t)B * (h->table_sharded ? 1 : c.world_size),
-                                                h->table_sharded ? 0 : c.rank, h->table_sharded ? 1 : c.world_size,
-                                                c.seed, reinterpret_cast<float4*>(h->staged_batch()));
-      CQL_LAUNCH_CHECK(h);
+      launch(h, st, PLAIN, k_sample, dim3((B + 127) / 128), dim3(128), 0, reinterpret_cast<const float4*>(h->table), h->n_trans,
+             nullptr, h->step_dev, 0, B, (int64_t)B * (h->table_sharded ? 1 : c.world_size), h->table_sharded ? 0 : c.rank,
+             h->table_sharded ? 1 : c.world_size, c.seed, reinterpret_cast<float4*>(h->staged_batch()));
     }
-    if (ns == NoiseSource::Philox) {
-      k_noise<<<(int)((h->noise_floats + 255) / 256), 256, 0, st>>>(h->noise, h->noise_floats, B, h->n, c.seed,
-                                                                    h->step_dev, c.rank);
-      CQL_LAUNCH_CHECK(h);
-    }
-    k_actor_rows<<<(2 * B + 255) / 256, 256, 0, st>>>(reinterpret_cast<const float4*>(h->staged_batch()), B,
-                                                      reinterpret_cast<float4*>(h->batch), h->XA, h->prep);
-    CQL_LAUNCH_CHECK(h);
+    if (ns == NoiseSource::Philox)
+      launch(h, st, PLAIN, k_noise, dim3((int)((h->noise_floats + 255) / 256)), dim3(256), 0, h->noise, h->noise_floats, B, h->n,
+             c.seed, h->step_dev, c.rank);
+    launch(h, st, PLAIN, k_actor_rows, dim3((2 * B + 255) / 256), dim3(256), 0, reinterpret_cast<const float4*>(h->staged_batch()),
+           B, reinterpret_cast<float4*>(h->batch), h->XA, h->prep);
   }
   {
     FwdJobs jobs{};
@@ -1184,13 +1193,11 @@ inline void phase0(Handle* h, cudaStream_t st, BatchSource bs, NoiseSource ns) {
     jobs.j[1] = FwdJob{h->XA + B, h->net_params(slot_actor()), h->outA + 2 * (size_t)B, nullptr, B, 1, 0};
     mark(h, st, 1);
     QSrc srcA[2];
-    launch_fwd_any<2, 2>(h, jobs, st, srcA);
+    launch_fwd<P, 2, 2>(h, jobs, st, srcA);
     mark(h, st, 2);
-    if (!skip_launch(1))
-      launch_pdl(k_prep, dim3((B * 64 + 255) / 256), dim3(256), 0, st, batch4, srcA[0], srcA[1], h->outA, h->noise, B, h->n, c.squash, h->XAl,
-               h->offAl, h->XC, h->offC, h->XT, h->XP, reinterpret_cast<float4*>(h->perb));
+    launch(h, st, pdl_skip(1), k_prep, dim3((B * 64 + 255) / 256), dim3(256), 0, batch4, srcA[0], srcA[1], h->outA, h->noise, B,
+           h->n, c.squash, h->XAl, h->offAl, h->XC, h->offC, h->XT, h->XP, reinterpret_cast<float4*>(h->perb));
   }
-  CQL_LAUNCH_CHECK(h);
   {
     FwdJobs jobs{};
     jobs.n = 3;
@@ -1204,140 +1211,68 @@ inline void phase0(Handle* h, cudaStream_t st, BatchSource bs, NoiseSource ns) {
     // (the repeats are launched the way the step graph launches this kernel -- with programmatic dependent launch -- so a
     //  repeat's prologue overlaps its predecessor's drain exactly as it overlaps k_prep's in the product schedule; the
     //  events on either side still separate the four launches from their neighbours)
+    const bool pdl_off = h->pdl_off;
     for (int rep = 0; rep < (h->timing ? TIMED_FWD_REPS : 1); ++rep) {
-      const bool saved = g_timing_no_pdl;
-      if (rep > 0) g_timing_no_pdl = false;
-      launch_fwd_any<3, 1>(h, jobs, st, srcQ);
-      g_timing_no_pdl = saved;
+      h->pdl_off = pdl_off && rep == 0;
+      launch_fwd<P, 3, 1>(h, jobs, st, srcQ);
     }
+    h->pdl_off = pdl_off;
     mark(h, st, 4);
     // (the last block of k_lse also sums the pair values and publishes the two scalar gradients: the former k_scalar_reduce)
     const int64_t so = scalars_off(C);
     ScalarReduceArgs ra{reinterpret_cast<const float4*>(h->perb), h->scalars(), h->adam_m + so, h->adam_v + so, h->g_scalars(),
                         h->loss_sums, h->metrics, reinterpret_cast<unsigned int*>(h->loss_sums + 15), h->dp_fused ? h->dp : DpPeer{}};
-    if (!skip_launch(2))
-      launch_pdl(k_lse, dim3((C * B * 32 + 255) / 256), dim3(256), 0, st, batch4, srcQ[0], h->offAl, srcQ[1], h->offC, srcQ[2], loss_consts(h),
-               h->dQ, reinterpret_cast<PairVals*>(h->pairv), ra);
-    CQL_LAUNCH_CHECK(h);
+    launch(h, st, pdl_skip(2), k_lse, dim3((C * B * 32 + 255) / 256), dim3(256), 0, batch4, srcQ[0], h->offAl, srcQ[1], h->offC,
+           srcQ[2], loss_consts(h), h->dQ, reinterpret_cast<PairVals*>(h->pairv), ra);
   }
 }
 
 // phase 1: temp/alpha Adam, critic backward -> critic gradients
+template <Prec P>
 inline void phase1(Handle* h, cudaStream_t st) {
   NvtxRange nvtx("cql.update.phase1: temp/alpha Adam, critic backward");
-  const int B = h->B, C = h->C, n3 = 3 * h->n, rows = B * (n3 + 1);
+  const int B = h->B, C = h->C, rows = B * (3 * h->n + 1);
   const int64_t so = scalars_off(C);
-  if (!skip_launch(8))
-    launch_pdl(k_scalar_adam_dq, dim3((int)(((int64_t)C * rows + 255) / 256)), dim3(256), 0, st, h->scalars(), h->adam_m + so, h->adam_v + so,
-             h->g_scalars(), h->stepinfo, loss_consts(h), h->loss_sums, h->metrics, reinterpret_cast<const PairVals*>(h->pairv), h->dQ,
-             h->dp_fused ? h->dp : DpPeer{}, (long long)(1 + C) * NET_STRIDE);
-  CQL_LAUNCH_CHECK(h);
-  BwdJob jb{h->XC, h->dQ, h->h2C, h->net_params(slot_critic(0)), h->smallC, nullptr, h->pw2C, rows, C, h->splitsC};
+  launch(h, st, pdl_skip(8), k_scalar_adam_dq, dim3((int)(((int64_t)C * rows + 255) / 256)), dim3(256), 0, h->scalars(),
+         h->adam_m + so, h->adam_v + so, h->g_scalars(), h->stepinfo, loss_consts(h), h->loss_sums, h->metrics,
+         reinterpret_cast<const PairVals*>(h->pairv), h->dQ, h->dp_fused ? h->dp : DpPeer{}, (long long)(1 + C) * NET_STRIDE);
   mark(h, st, 5);
-  if (h->cfg.precision != CQL_PREC_FP32) {
-    if (h->cfg.precision == CQL_PREC_F16X3) launch_bwd_tc<true, 3, 1, true, false, true>(h, jb, h->g_critics(), st, 6, 7);
-    else if (h->cfg.precision != CQL_PREC_BF16) launch_bwd_tc<true, 3, 1, true, false>(h, jb, h->g_critics(), st, 6, 7);
-    else launch_bwd_tc<false, 3, 1, true, false>(h, jb, h->g_critics(), st, 6, 7);
-    return;
-  }
-  launch_bwd1<3, 1, true, false>(h, jb, st);
-  mark(h, st, 6);
-  launch_bwd2<3, 1>(h, jb, st);
-  mark(h, st, 7);
-  k_reduce_grads<<<dim3((NET_STRIDE + 255) / 256, C), 256, 0, st>>>(h->smallC, h->pw2C, 3, 1, tiles_of(rows),
-                                                                   h->splitsC, h->g_critics());
-  CQL_LAUNCH_CHECK(h);
+  launch_bwd<P, 3, 1, true, false>(h, critic_bwd_job(h), h->g_critics(), st, BwdMarks{6, 7, -1});
 }
 
 // phase 2: critic Adam + Polyak, actor loss through the updated critics -> actor gradients
+template <Prec P>
 inline void phase2(Handle* h, cudaStream_t st) {
   NvtxRange nvtx("cql.update.phase2: critic Adam + Polyak + pack, actor step forward/backward");
   const int B = h->B, C = h->C;
-  const cql_config& c = h->cfg;
-  static const bool no_fused_adam = std::getenv("CQL_NO_FUSED_ADAM") != nullptr;      // A/B switch
-  if (h->cfg.precision == CQL_PREC_F16X3 && !no_fused_adam) {
-    adam_pack(h, slot_critic(0), C, 3, 1, c.critic_lr, st);
-  } else {
-    const int64_t cnt = (int64_t)C * NET_STRIDE;
-    launch_pdl(k_adam_polyak, dim3((int)((cnt + 255) / 256)), dim3(256), 0, st,
-        h->net_params(slot_critic(0)), h->adam_m + (size_t)NET_STRIDE, h->adam_v + (size_t)NET_STRIDE, h->g_critics(),
-        h->net_params(slot_targ_critic(C, 0)), cnt, c.critic_lr, c.beta1, c.beta2, c.adam_eps, c.tau, h->stepinfo);
-    CQL_LAUNCH_CHECK(h);
-    int slots[2 * CQL_MAX_CRITICS];
-    for (int i = 0; i < C; ++i) { slots[i] = slot_critic(i); slots[C + i] = slot_targ_critic(C, i); }
-    pack_slots(h, slots, 2 * C, st);
-  }
-  bool fold_dq = false;
-  QSrc srcP_keep{};
-  {
-    FwdJobs jobs{};
-    jobs.n = 1;
-    jobs.j[0] = FwdJob{h->XP, h->net_params(slot_critic(0)), h->QP, h->h2P, B, C, 0};
-    mark(h, st, 8);
-    QSrc srcP[1];
-    launch_fwd_any<3, 1>(h, jobs, st, srcP);
-    mark(h, st, 9);
-    fold_dq = h->cfg.precision == CQL_PREC_F16X3 && srcP[0].n_parts > 0;
-    srcP_keep = srcP[0];
-    if (!fold_dq) {        // (f16x3: the dx-only bwd1 below takes dQ from the partial sums itself, k_actor_dout the metric)
-      if (!skip_launch(16))
-        launch_pdl(k_actor_dq, dim3(1), dim3(1024), 0, st, srcP[0], reinterpret_cast<const float4*>(h->perb), h->scalars(), B, C, h->dQP,
-                 h->metrics);
-      CQL_LAUNCH_CHECK(h);
-    }
-  }
-  {
-    BwdJob jb{h->XP, h->dQP, h->h2P, h->net_params(slot_critic(0)), nullptr, h->dXP, nullptr, B, C, 1};
-    if (fold_dq) { jb.q_part = srcP_keep.q; jb.q_parts = srcP_keep.n_parts; jb.dq_scale = -1.f / (float)B; }
-    if (h->cfg.precision == CQL_PREC_F16X3) launch_bwd_tc<true, 3, 1, false, true, true>(h, jb, nullptr, st);
-    else if (h->cfg.precision == CQL_PREC_TF32X3) launch_bwd_tc<true, 3, 1, false, true>(h, jb, nullptr, st);
-    else if (h->cfg.precision == CQL_PREC_BF16) launch_bwd_tc<false, 3, 1, false, true>(h, jb, nullptr, st);
-    else launch_bwd1<3, 1, false, true>(h, jb, st);
-  }
-  const bool tcm = h->cfg.precision != CQL_PREC_FP32;
-  if (!skip_launch(32))
-    launch_pdl(k_actor_dout, dim3((B + 127) / 128), dim3(128), 0, st, h->outA, h->noise + B + 6 * (int64_t)B * h->n,
-                                                tcm ? h->dX_part : h->dXP, h->scalars(), B,
-                                                tcm ? h->last_dx_parts : C, c.squash, h->dOutA,
-                                                fold_dq ? srcP_keep : QSrc{}, reinterpret_cast<const float4*>(h->perb), C,
-                                                h->actor_part, reinterpret_cast<unsigned int*>(h->loss_sums + 14), h->metrics);
-  CQL_LAUNCH_CHECK(h);
-  BwdJob ja{h->XA, h->dOutA, h->h2A, h->net_params(slot_actor()), h->smallA, nullptr, h->pw2A, B, 1, h->splitsA};
+  optimizer_step<P>(h, critic_group(h), bwd_plan<P, 3, 1, true, false>(h, critic_bwd_job(h)), st, false);
+  FwdJobs jobs{};
+  jobs.n = 1;
+  jobs.j[0] = FwdJob{h->XP, h->net_params(slot_critic(0)), h->QP, h->h2P, B, C, 0};
+  mark(h, st, 8);
+  QSrc srcP;
+  launch_fwd<P, 3, 1>(h, jobs, st, &srcP);
+  mark(h, st, 9);
+  // the forward left partial sums (f16x3): the dx-only bwd1 below takes dQ from them itself, k_actor_dout the metric
+  const bool fold_dq = srcP.n_parts > 0;
+  const float4* perb = reinterpret_cast<const float4*>(h->perb);
+  if (!fold_dq)
+    launch(h, st, pdl_skip(16), k_actor_dq, dim3(1), dim3(1024), 0, srcP, perb, h->scalars(), B, C, h->dQP, h->metrics);
+  BwdJob jd{h->XP, h->dQP, h->h2P, h->net_params(slot_critic(0)), nullptr, h->dXP, nullptr, B, C, 1};
+  if (fold_dq) { jd.q_part = srcP.q; jd.q_parts = srcP.n_parts; jd.dq_scale = -1.f / (float)B; }
+  const BwdPlan dx = launch_bwd<P, 3, 1, false, true>(h, jd, nullptr, st);
+  launch(h, st, pdl_skip(32), k_actor_dout, dim3((B + 127) / 128), dim3(128), 0, h->outA, h->noise + B + 6 * (int64_t)B * h->n,
+         dx.dx, h->scalars(), B, dx.dx_parts, h->cfg.squash, h->dOutA, fold_dq ? srcP : QSrc{}, perb, C, h->actor_part,
+         reinterpret_cast<unsigned int*>(h->loss_sums + 14), h->metrics);
   mark(h, st, 10);
-  if (tcm) {
-    if (h->cfg.precision == CQL_PREC_F16X3) launch_bwd_tc<true, 2, 2, true, false, true>(h, ja, h->g_actor(), st);
-    else if (h->cfg.precision != CQL_PREC_BF16) launch_bwd_tc<true, 2, 2, true, false>(h, ja, h->g_actor(), st);
-    else launch_bwd_tc<false, 2, 2, true, false>(h, ja, h->g_actor(), st);
-    mark(h, st, 11);
-    return;
-  }
-  launch_bwd1<2, 2, true, false>(h, ja, st);
-  launch_bwd2<2, 2>(h, ja, st);
-  mark(h, st, 11);
-  k_reduce_grads<<<dim3((NET_STRIDE + 255) / 256, 1), 256, 0, st>>>(h->smallA, h->pw2A, 2, 2, tiles_of(B), h->splitsA,
-                                                                   h->g_actor());
-  CQL_LAUNCH_CHECK(h);
+  launch_bwd<P, 2, 2, true, false>(h, actor_bwd_job(h), h->g_actor(), st, BwdMarks{-1, -1, 11});
 }
 
 // phase 3: actor Adam + Polyak of the target policy, step counter
+template <Prec P>
 inline void phase3(Handle* h, cudaStream_t st) {
   NvtxRange nvtx("cql.update.phase3: actor Adam + Polyak + pack");
-  const cql_config& c = h->cfg;
-  static const bool no_fused_adam = std::getenv("CQL_NO_FUSED_ADAM") != nullptr;      // A/B switch
-  if (h->cfg.precision == CQL_PREC_F16X3 && !no_fused_adam) {
-    adam_pack(h, slot_actor(), 1, 2, 2, c.actor_lr, st, /*last=*/true);      // also counts the step
-    mark(h, st, 12);
-    return;
-  } else {
-    launch_pdl(k_adam_polyak, dim3((NET_STRIDE + 255) / 256), dim3(256), 0, st, h->net_params(slot_actor()), h->adam_m, h->adam_v,
-                                                           h->g_actor(), h->net_params(slot_targ_actor(h->C)),
-                                                           (int64_t)NET_STRIDE, c.actor_lr, c.beta1, c.beta2, c.adam_eps,
-                                                           c.tau, h->stepinfo);
-    CQL_LAUNCH_CHECK(h);
-    pack_weights(h, slot_actor(), 1, 2, st);
-  }
-  launch_pdl(k_step_end, dim3(1), dim3(1), 0, st, h->step_dev);
-  CQL_LAUNCH_CHECK(h);
+  optimizer_step<P>(h, actor_group(h), bwd_plan<P, 2, 2, true, false>(h, actor_bwd_job(h)), st, true);
   mark(h, st, 12);
 }
 

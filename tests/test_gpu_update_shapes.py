@@ -1,7 +1,7 @@
 """GPU parity of the CQL update at the batch sizes, critic counts and action-sample counts the API accepts.
 
 ``cql_create`` takes batch_size 1..2^20, n_critics 1..4 and n_action_samples 1..10.  In ``f16x3`` the shape decides which
-kernel runs each hidden-layer contraction (``launch_fwd_tc`` / ``launch_bwd_tc`` in ``csrc/update.cuh``): "pair" (CTA pairs,
+kernel runs each hidden-layer contraction (``launch_fwd`` / ``bwd_plan`` in ``csrc/update.cuh``): "pair" (CTA pairs,
 ``*_h2_kernel``, when ``n_nets * ceil(rows/256) >= num_sms/2``), "small" (32-column work items, ``HCfgS``) or "regular"
 (``*_h_kernel``).  The row count of each launch also sets the tails: ``rows mod 128`` / ``rows mod 256`` (a CTA pair whose
 second CTA has no rows or one row), ``B mod 32`` (the warp partials of ``k_actor_dout``) and the ``3n + 1`` lanes per batch
