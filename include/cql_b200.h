@@ -313,6 +313,31 @@ int  cql_rank_metrics(cql_handle* h, const int32_t* rec_items, int64_t n_users, 
                       const int32_t* users, const int64_t* gt_indptr, const int32_t* gt_items,
                       const int32_t* ks, int32_t n_ks, double* out_means, void* stream);
 
+/* ---- offline evaluation ------------------------------------------------ */
+/* d3rlpy's offline scorers (DESIGN.md section 1) over the loaded one-step replay table, as float64 SUMS and counts so
+ * that the results of several table shards can be combined.  An episode ends at a terminal row or at the end of the
+ * table; d3rlpy's 1024-transition windows restart the advantage recursion.  Per row, in float32 as the update forms them
+ * (scalers applied: s and s' observation-scaled, a action-scaled into Q, r reward-scaled in the target; the greedy action
+ * tanh(mu(x)) enters Q in network space): Q(s,a) = mean_i Q_i(s, a), V(x) = mean_i Q_i(x, tanh(mu(x))), sigma(x) =
+ * population std of the Q_i(x, tanh(mu(x))).  return_threshold: episodes whose float64 sum of RAW rewards is >= it are
+ * successes (soft OPC); NaN = no soft OPC (success sums 0).  Rejected (3) when no table is loaded or n_steps > 1.
+ * Synchronises `stream`.
+ * replaces: d3rlpy.metrics.scorer td_error_scorer, discounted_sum_of_advantage_scorer, average_value_estimation_scorer,
+ *           value_estimation_std_scorer, initial_state_value_estimation_scorer, soft_opc_scorer,
+ *           continuous_action_diff_scorer [EXT d3rlpy 1.x metrics/scorer.py] */
+typedef struct cql_offline_sums {
+  double td_error;              /* sum over rows of (Q(s,a) - y)^2, y = r' + gamma * V(s') * (1 - term) (one-step) */
+  double discounted_advantage;  /* sum over rows of the windowed discounted advantage sum A_t (adv = Q(s,a) - V(s)) */
+  double value;                 /* sum over rows of V(s) */
+  double value_std;             /* sum over rows of sigma(s) */
+  double initial_value;         /* sum over episodes of V(s_0) */
+  double action_diff;           /* sum over rows of (a - reverse(tanh(mu(s))))^2, a raw */
+  double success_q;             /* sum of Q(s,a) over the rows of successful episodes */
+  double all_q;                 /* sum of Q(s,a) over all rows */
+  int64_t n_rows, n_episodes, n_success_rows;
+} cql_offline_sums;
+int  cql_offline_eval(cql_handle* h, float return_threshold, cql_offline_sums* out, void* stream);
+
 /* Measurement aid: runs ONE sampled update with CUDA events around the heavy launches and
  * returns their durations in milliseconds (synchronises).  out_ms[0] = critic forward (alpha +
  * critic + target rows), [1] = critic backward-1, [2] = critic backward-2 (dW2), [3] = whole

@@ -62,6 +62,17 @@ class Preprocessing(C.Structure):
     ]
 
 
+class OfflineSums(C.Structure):
+    """Mirror of ``struct cql_offline_sums``."""
+
+    _fields_ = [
+        ("td_error", C.c_double), ("discounted_advantage", C.c_double), ("value", C.c_double),
+        ("value_std", C.c_double), ("initial_value", C.c_double), ("action_diff", C.c_double),
+        ("success_q", C.c_double), ("all_q", C.c_double),
+        ("n_rows", C.c_int64), ("n_episodes", C.c_int64), ("n_success_rows", C.c_int64),
+    ]
+
+
 _P = C.c_void_p
 _F = C.POINTER(C.c_float)
 _I32 = C.POINTER(C.c_int32)
@@ -112,6 +123,7 @@ SIGNATURES = {
     "cql_mdp_append": (C.c_int, [_P, C.c_int32, C.c_int32, _P, C.c_int64]),
     "cql_mdp_finish": (C.c_int, [_P, C.c_int32, C.c_float, _P, _P, _P, _P, _P]),
     "cql_selftest_umma": (C.c_int, [_P, C.c_int, _P, _P, C.c_int, C.c_int, _P]),
+    "cql_offline_eval": (C.c_int, [_P, C.c_float, C.POINTER(OfflineSums), _P]),
     "cql_launch_count": (C.c_int64, [_P]),
 }
 

@@ -13,6 +13,7 @@
 #include "metrics.cuh"
 #include "dp_peer.cuh"
 #include "mma_bench.cuh"
+#include "offline_eval.cuh"
 
 using namespace cql;
 
@@ -1245,6 +1246,19 @@ int cql_topk_filter_dev(cql_handle* ch, const float* scores_dev, int64_t n_users
         scores_dev, n_items, users_dev, items_dev, seen_indptr, seen_items, k, out_scores, out_items);
     CQL_LAUNCH_CHECK(&h);
     if (!stream) CQL_CUDA(cudaStreamSynchronize(st));
+  });
+}
+
+int cql_offline_eval(cql_handle* ch, float return_threshold, cql_offline_sums* out, void* stream) {
+  return guarded(ch, [&] {
+    NvtxRange nvtx("cql_offline_eval");
+    Handle& h = ch->h;
+    CQL_REQUIRE(out != nullptr, "cql_offline_eval: NULL output");
+    CQL_REQUIRE(h.n_trans > 0, "cql_offline_eval: no replay table loaded (build or load one, or evaluate a log)");
+    CQL_REQUIRE(h.n_steps == 1, "cql_offline_eval: the table holds n-step rows (n_steps > 1); evaluate one-step rows");
+    double s[OE_SUMS];
+    with_precision(&h, [&](auto p) { offline_eval<decltype(p)::value>(&h, return_threshold, s, pick_stream(&h, stream)); });
+    *out = cql_offline_sums{s[0], s[1], s[2], s[3], s[4], s[5], s[6], s[7], h.n_trans, (int64_t)s[8], (int64_t)s[9]};
   });
 }
 

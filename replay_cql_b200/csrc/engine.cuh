@@ -1,5 +1,6 @@
 // engine.cuh -- the per-GPU handle: configuration, HBM-resident state, scratch.
 #pragma once
+#include <algorithm>
 #include <cstdlib>
 #include <vector>
 #include <string>
@@ -273,6 +274,38 @@ void expand_n_steps(Handle& h, const float* one_step, int64_t n, cudaStream_t st
 // synchronisation; cql_get_table_stats reads them).  rew_ok = false: the reward slot holds n-step returns, the reward
 // statistics are marked unavailable.  Returns the launches it made (capi.cu).
 int table_stats(Handle& h, const float* rows, int64_t n, bool rew_ok, cudaStream_t st);
+
+// Call scratch comes from the stream-ordered pool (cudaMallocAsync), which keeps up to 4 GB cached between calls:
+// the ~1.9 GB of cudaMalloc / cudaFree pairs per 20 M-row ingestion session synchronise the device and made ingestion
+// (and `fit`) wall clocks erratic on shared hosts -- 0.05 .. 1.2 s for the same call (r02 bench lines).
+inline void keep_pool_cached() {
+  static unsigned long long done_mask = 0;          // per device (engines on several GPUs may live in one process)
+  int dev = 0;
+  if (cudaGetDevice(&dev) != cudaSuccess || dev < 0 || dev >= 64 || (done_mask >> dev) & 1ull) return;
+  done_mask |= 1ull << dev;
+  cudaMemPool_t mp = nullptr;
+  unsigned long long keep = 4ull << 30;
+  if (cudaDeviceGetDefaultMemPool(&mp, dev) == cudaSuccess)
+    cudaMemPoolSetAttribute(mp, cudaMemPoolAttrReleaseThreshold, &keep);
+}
+
+// device scratch from the stream-ordered pool, released on every exit path: cudaMalloc / cudaFree pairs per call
+// synchronise the device and made `predict` wall clocks erratic (0.05 .. 1.4 s for the same ML-1M call)
+struct DevTmp {
+  cudaStream_t st;
+  std::vector<void*> p;
+  explicit DevTmp(cudaStream_t s) : st(s) { keep_pool_cached(); }
+  ~DevTmp() { for (void* x : p) cudaFreeAsync(x, st); }
+  DevTmp(const DevTmp&) = delete;
+  DevTmp& operator=(const DevTmp&) = delete;
+  template <typename T>
+  T* get(size_t count) {
+    void* q = nullptr;
+    CQL_CUDA(cudaMallocAsync(&q, std::max<size_t>(1, count) * sizeof(T), st));
+    p.push_back(q);
+    return (T*)q;
+  }
+};
 
 inline void mark(Handle* h, cudaStream_t st, int i) {
   if (h->timing) CQL_CUDA(cudaEventRecord(h->ev[i], st));

@@ -71,20 +71,8 @@ __global__ void k_emit(const uint32_t* __restrict__ order, const int32_t* __rest
   if (obs_o) { obs_o[2 * i] = uf; obs_o[2 * i + 1] = itf; act_o[i] = act; rew_o[i] = rw; term_o[i] = last ? 1.f : 0.f; }
 }
 
-// Session scratch comes from the stream-ordered pool (cudaMallocAsync), which keeps up to 4 GB cached between calls:
-// the ~1.9 GB of cudaMalloc / cudaFree pairs per 20 M-row session synchronise the device and made ingestion (and `fit`)
-// wall clocks erratic on shared hosts -- 0.05 .. 1.2 s for the same call (r02 bench lines).  The caller synchronises
-// `st` before the pointers are used on another stream.
-inline void keep_pool_cached() {
-  static unsigned long long done_mask = 0;          // per device (engines on several GPUs may live in one process)
-  int dev = 0;
-  if (cudaGetDevice(&dev) != cudaSuccess || dev < 0 || dev >= 64 || (done_mask >> dev) & 1ull) return;
-  done_mask |= 1ull << dev;
-  cudaMemPool_t mp = nullptr;
-  unsigned long long keep = 4ull << 30;
-  if (cudaDeviceGetDefaultMemPool(&mp, dev) == cudaSuccess)
-    cudaMemPoolSetAttribute(mp, cudaMemPoolAttrReleaseThreshold, &keep);
-}
+// Session scratch comes from the stream-ordered pool (keep_pool_cached, engine.cuh); the caller synchronises `st`
+// before the pointers are used on another stream.
 template <typename T>
 T* dmalloc(size_t n, std::vector<void*>& pool, cudaStream_t st) {
   keep_pool_cached();
@@ -407,22 +395,6 @@ __global__ void k_seen_emit(const unsigned long long* __restrict__ key, int64_t 
   if (i == num - 1 && u < n_users)
     for (int64_t x = u + 1; x <= n_users; ++x) indptr[x] = num;
 }
-// device scratch from the stream-ordered pool, released on every exit path: cudaMalloc / cudaFree pairs per call
-// synchronise the device and made `predict` wall clocks erratic (0.05 .. 1.4 s for the same ML-1M call); the pool keeps
-// its memory cached between calls (keep_pool_cached)
-struct DevTmp {
-  cudaStream_t st;
-  std::vector<void*> p;
-  explicit DevTmp(cudaStream_t s) : st(s) { keep_pool_cached(); }
-  ~DevTmp() { for (void* x : p) cudaFreeAsync(x, st); }
-  template <typename T>
-  T* get(size_t count) {
-    void* q = nullptr;
-    CQL_CUDA(cudaMallocAsync(&q, count * sizeof(T), st));
-    p.push_back(q);
-    return (T*)q;
-  }
-};
 }  // namespace
 
 int64_t cql::seen_csr_on_device(Handle& h, const int32_t* users_h, const int32_t* items_h, int64_t n, int64_t n_users,

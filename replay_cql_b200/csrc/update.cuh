@@ -804,9 +804,10 @@ using TcCfg = std::conditional_t<P == Prec::F16X3, tc::HCfg, tc::Cfg<P != Prec::
 
 // The critic forward over a job list (fp32: CUDA cores; else tensor cores, W2 from the packed copy).  src[i] tells the
 // consumer kernels where job i's outputs are (see QSrc): f16x3 leaves the layer-3 partial sums to them (q_at); tf32x3
-// and bf16 sum the partials in one more launch.
+// and bf16 sum the partials in one more launch.  `part` / `part_floats`: scratch for those partials other than the
+// update's own (Handle::part), for a caller whose row counts are not the update's (cql_offline_eval).
 template <Prec P, int IN, int OUT>
-inline void launch_fwd(Handle* h, FwdJobs& jobs, cudaStream_t st, QSrc* src) {
+inline void launch_fwd(Handle* h, FwdJobs& jobs, cudaStream_t st, QSrc* src, float* part = nullptr, size_t part_floats = 0) {
   if constexpr (P == Prec::FP32) {
     int t = 0;
     for (int i = 0; i < jobs.n; ++i) {
@@ -843,7 +844,7 @@ inline void launch_fwd(Handle* h, FwdJobs& jobs, cudaStream_t st, QSrc* src) {
       const int slot = (int)((j.params - h->params) / NET_STRIDE);
       tj.item_begin[i] = items;
       items += j.n_nets * n_slices * ((j.rows + tc::TM - 1) / tc::TM);
-      part_of[i] = h->part + part_off;
+      part_of[i] = (part ? part : h->part) + part_off;
       part_off += (size_t)j.n_nets * n_parts * j.rows * OUT;
       tj.j[i] = tc::TcFwdJob{j.X, j.params,
                              pair ? h->packed_fwd2 + (size_t)slot * h->packed_net_bytes2 : h->packed_fwd + (size_t)slot * h->packed_net_bytes,
@@ -851,7 +852,7 @@ inline void launch_fwd(Handle* h, FwdJobs& jobs, cudaStream_t st, QSrc* src) {
     }
     tj.item_begin[jobs.n] = items;
     tj.h2_cost = sw.h2_cost;
-    CQL_REQUIRE(part_off <= h->part_floats, "internal: partial-sum scratch too small");
+    CQL_REQUIRE(part_off <= (part ? part_floats : h->part_floats), "internal: partial-sum scratch too small");
     if (items == 0) return;
     const int grid = items < h->num_sms ? items : h->num_sms;
     if constexpr (F16X3) {

@@ -25,6 +25,26 @@ PRECISIONS = {"fp32": _lib.PREC_FP32, "tf32x3": _lib.PREC_TF32X3, "bf16": _lib.P
               "f16x3": _lib.PREC_F16X3}
 SQUASH = {"eps": _lib.SQUASH_EPS, "softplus": _lib.SQUASH_SOFTPLUS}
 SCORE_MODES = {"q": _lib.SCORE_Q, "policy": _lib.SCORE_POLICY}
+OFFLINE_SUM_KEYS = tuple(name for name, _ in _lib.OfflineSums._fields_)
+
+
+def offline_scores(sums: Dict[str, float], soft_opc: bool) -> Dict[str, float]:
+    """Sums and counts of ``CqlEngine.offline_metrics`` (one table, or several shards added up) -> d3rlpy's offline
+    scorer values (DESIGN.md section 1): means over rows, ``initial_state_value_estimation`` over episodes, ``soft_opc``
+    (only when ``soft_opc``) NaN when no episode reached the return threshold.  Unlike d3rlpy's scorers, which negate the
+    "smaller is better" ones, every value is the plain mean."""
+    n, n_ep, n_ok = sums["n_rows"], sums["n_episodes"], sums["n_success_rows"]
+    out = {
+        "td_error": sums["td_error"] / n,
+        "discounted_sum_of_advantage": sums["discounted_advantage"] / n,
+        "average_value_estimation": sums["value"] / n,
+        "value_estimation_std": sums["value_std"] / n,
+        "initial_state_value_estimation": sums["initial_value"] / n_ep,
+        "continuous_action_diff": sums["action_diff"] / n,
+    }
+    if soft_opc:
+        out["soft_opc"] = sums["success_q"] / n_ok - sums["all_q"] / n if n_ok else float("nan")
+    return out
 
 
 @dataclass
@@ -455,6 +475,19 @@ class CqlEngine:
         ptr, n = self.device_buffer(_lib.BUF_METRICS)
         t = torch.as_tensor(_DevView(ptr, n), device=f"cuda:{self.device}").cpu().numpy()
         return dict(zip(METRIC_NAMES, map(float, t[:6])))
+
+    # ------------------------------------------------------------------ offline evaluation
+    def offline_metrics(self, return_threshold: Optional[float] = None, stream: int | None = None) -> Dict[str, float]:
+        """d3rlpy's offline scorers over the loaded one-step replay table (``cql_offline_eval``) as float64 sums and
+        int counts (keys ``OFFLINE_SUM_KEYS``; ``offline_scores`` turns them into the metric values).  Episodes whose
+        raw return is >= ``return_threshold`` (float32) feed the soft-OPC sums; None leaves them 0.  Weights, Adam
+        state, step counter, table and captured update graphs are untouched."""
+        thr = float("nan") if return_threshold is None else float(return_threshold)
+        if return_threshold is not None and not np.isfinite(thr):
+            raise ValueError("return_threshold must be a finite number or None")
+        out = _lib.OfflineSums()
+        self._check(self._lib.cql_offline_eval(self._h, thr, C.byref(out), stream), "cql_offline_eval")
+        return {k: (int if k.startswith("n_") else float)(getattr(out, k)) for k in OFFLINE_SUM_KEYS}
 
     # ------------------------------------------------------------------ scoring
     def score_topk(self, users, items, k: int, seen_indptr=None, seen_items=None, mode: str = "q"):

@@ -7,6 +7,7 @@ Keeps the wrapper's public contract (SURVEY.md Appendix B, section 8b): ``fit(lo
 """
 from __future__ import annotations
 
+import dataclasses
 import json
 import os
 from typing import Any, Dict, Optional
@@ -14,7 +15,7 @@ from typing import Any, Dict, Optional
 import numpy as np
 import pandas as pd
 
-from .engine import CqlEngine, CqlHyperParams
+from .engine import OFFLINE_SUM_KEYS, CqlEngine, CqlHyperParams, offline_scores
 from .mdp import build_mdp_on_device, seen_csr
 from .parallel import GradAllReducer, dist_info, gather_rows, shard_range
 from .recommender import Recommender, _rec_frame, get_top_k_recs
@@ -212,6 +213,7 @@ class CQL(Recommender):
             log = shard_log_by_user(log, rank, world)
         build_mdp_on_device(eng, log, top_k=self.top_k, action_randomization_scale=self.action_randomization_scale)
         eng.set_table_sharded(sharded)
+        self._table_sharded = sharded
         self._fit_preprocessing(sharded)
         n_rows = eng.n_transitions
         per_epoch = self.n_steps_per_epoch
@@ -410,6 +412,64 @@ class CQL(Recommender):
             pos = top.groupby("user_idx").cumcount().to_numpy()
             table[row, pos] = top["item_idx"].to_numpy().astype(np.int32)
         return self.engine.rank_metrics(table, users, gt_ptr, gt_items, ks)
+
+    def offline_metrics(self, log: Any = None, return_threshold: Optional[float] = None) -> Dict[str, float]:
+        """d3rlpy's offline scorers (``d3rlpy.metrics.scorer``, DESIGN.md section 1) of the current networks on the GPU:
+        ``td_error``, ``discounted_sum_of_advantage``, ``average_value_estimation``, ``value_estimation_std``,
+        ``initial_state_value_estimation``, ``continuous_action_diff`` and, with ``return_threshold``, ``soft_opc``.
+
+        ``log=None`` evaluates the fitted replay table (it must be one-step: ``n_steps = 1``, and present: a model loaded
+        without ``save_replay_table`` has none).  With a ``log`` (anything ``fit`` accepts) the one-step rows are built
+        by the same MDP builder (``top_k``, ``action_randomization_scale``) on a short-lived evaluation engine holding
+        this model's networks and scalers.  Data parallel: each rank evaluates its own user range (of the log, or of a
+        sharded table) and the sums are combined in rank order; a replicated table is evaluated whole on every rank.
+        Nothing of the model changes: ``fit -> offline_metrics -> resume`` equals ``fit -> resume``."""
+        if self.engine is None:
+            raise AttributeError("CQL model is not fitted or loaded")
+        if return_threshold is not None:
+            if isinstance(return_threshold, bool) or not isinstance(return_threshold, (int, float, np.integer, np.floating)) \
+                    or not np.isfinite(float(return_threshold)):
+                raise ValueError("return_threshold must be a finite number or None")
+            return_threshold = float(return_threshold)
+        eng = self.engine
+        rank, world, local_rank = dist_info()
+        if log is None:
+            if eng.hp.n_steps > 1:
+                raise ValueError("offline_metrics: the replay table holds n-step rows (n_steps > 1) -- pass the log to "
+                                 "evaluate its one-step transitions")
+            if eng.n_transitions == 0:
+                raise ValueError("offline_metrics: the model holds no replay table (e.g. loaded from a checkpoint saved "
+                                 "without save_replay_table) -- pass the log")
+            sums = eng.offline_metrics(return_threshold)
+            sharded = world > 1 and getattr(self, "_table_sharded", False)
+        else:
+            n_log = int(log.num_rows) if hasattr(log, "num_rows") else len(log)
+            if n_log == 0:
+                raise ValueError("offline_metrics: empty log")
+            sharded = world > 1
+            if sharded:
+                from .mdp import shard_log_by_user
+                log = shard_log_by_user(log, rank, world)
+            n_local = int(log.num_rows) if hasattr(log, "num_rows") else len(log)
+            sums = {k: 0 for k in OFFLINE_SUM_KEYS}
+            if n_local:
+                ev = CqlEngine(dataclasses.replace(eng.hp, n_steps=1), device=local_rank, rank=rank, world_size=world)
+                try:
+                    ev.set_state(eng.get_state())
+                    prep = eng.get_preprocessing()
+                    if any(v is not None for v in prep.values()):
+                        ev.set_preprocessing(**prep)
+                    build_mdp_on_device(ev, log, top_k=self.top_k, action_randomization_scale=self.action_randomization_scale)
+                    sums = ev.offline_metrics(return_threshold)
+                finally:
+                    ev.close()
+        if sharded:
+            parts = gather_rows(np.array([[sums[k] for k in OFFLINE_SUM_KEYS]], dtype=np.float64))
+            total = np.zeros(len(OFFLINE_SUM_KEYS), dtype=np.float64)
+            for row in parts:                               # rank order: every rank adds the same values in the same order
+                total = total + row
+            sums = {k: (int(v) if k.startswith("n_") else float(v)) for k, v in zip(OFFLINE_SUM_KEYS, total)}
+        return offline_scores(sums, return_threshold is not None)
 
     def _default_criterion(self):
         """``optimize`` trials score NDCG@k on the GPU (``cql_rank_metrics``) instead of the pandas criterion."""
