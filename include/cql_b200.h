@@ -34,7 +34,8 @@ extern "C" {
 #define CQL_HIDDEN 256          /* d3rlpy default encoder: [256, 256] */
 #define CQL_OBS_DIM 2           /* (user_idx, item_idx) */
 #define CQL_ACT_DIM 1           /* relevance */
-#define CQL_MAX_CRITICS 4
+#define CQL_MAX_CRITICS 10        /* largest critic ensemble (n_critics) */
+#define CQL_MAX_ACTION_SAMPLES 32 /* most policy / uniform action samples per state (n_action_samples) */
 #define CQL_MAX_TOPK 1024
 #define CQL_MAX_N_STEPS 64      /* longest n-step TD horizon (cql_set_n_steps) */
 
@@ -53,7 +54,7 @@ typedef struct cql_config {
   int32_t device;               /* CUDA ordinal */
   int32_t batch_size;           /* B (per GPU) */
   int32_t n_critics;            /* C, 1..CQL_MAX_CRITICS */
-  int32_t n_action_samples;     /* n, 1..10 */
+  int32_t n_action_samples;     /* n, 1..CQL_MAX_ACTION_SAMPLES */
   int32_t precision;            /* CQL_PREC_* */
   int32_t squash;               /* CQL_SQUASH_* */
   int32_t rank, world_size;     /* data-parallel position (sampling streams only; no comms inside) */

@@ -20,6 +20,8 @@ SCORE_Q, SCORE_POLICY = 0, 1
 BUF_SCALAR_GRADS, BUF_CRITIC_GRADS, BUF_ACTOR_GRADS, BUF_METRICS, BUF_PARAMS, BUF_ALL_GRADS = range(6)
 MAX_TOPK = 1024
 MAX_N_STEPS = 64                                     # CQL_MAX_N_STEPS: longest n-step TD horizon
+MAX_CRITICS = 10                                     # CQL_MAX_CRITICS: largest critic ensemble (n_critics)
+MAX_ACTION_SAMPLES = 32                              # CQL_MAX_ACTION_SAMPLES: most action samples (n_action_samples)
 DT_I32, DT_I64, DT_F32, DT_F64 = 0, 1, 2, 3          # cql_mdp_append chunk dtypes
 SCALER_NONE, SCALER_MIN_MAX, SCALER_STANDARD = 0, 1, 2   # cql_preprocessing kinds
 

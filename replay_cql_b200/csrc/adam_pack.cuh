@@ -52,6 +52,8 @@ struct AdamPackJobs {
   int slots1, splits;
   int* wmax_acc;            // [CQL_MAX_CRITICS][16] layer maxima across the small-tensor CTAs, then [CQL_MAX_CRITICS] tickets
 };
+// passed by value as a kernel parameter (4 KB is the limit every CUDA 12 toolkit and driver accepts)
+static_assert(sizeof(AdamPackJobs) <= 4096, "AdamPackJobs must fit the kernel-parameter space");
 
 __device__ __forceinline__ float adam_one(float& p, float& m, float& v, float g, float step_size, float bc2s, float beta1,
                                           float beta2, float eps) {

@@ -153,39 +153,11 @@ void set_kernel_attrs() {
   CQL_CUDA(cudaFuncSetAttribute(tc::tc_bwd2_kernel<false, 2, 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tc::B2Cfg<false>::BYTES));
 }
 
-void create_impl(const cql_config* cfg, cql_handle* ch) {
-  Handle& h = ch->h;
-  CQL_REQUIRE(cfg != nullptr, "cql_create: cfg is NULL");
-  CQL_REQUIRE(cfg->struct_size == (int32_t)sizeof(cql_config), "cql_create: cql_config size mismatch (ABI)");
-  CQL_REQUIRE(cfg->batch_size >= 1 && cfg->batch_size <= (1 << 20), "cql_create: batch_size out of range");
-  CQL_REQUIRE(cfg->n_critics >= 1 && cfg->n_critics <= CQL_MAX_CRITICS, "cql_create: n_critics must be 1..4");
-  CQL_REQUIRE(cfg->n_action_samples >= 1 && cfg->n_action_samples <= 10, "cql_create: n_action_samples must be 1..10");
-  CQL_REQUIRE(cfg->precision == CQL_PREC_FP32 || cfg->precision == CQL_PREC_TF32X3 || cfg->precision == CQL_PREC_BF16 ||
-                  cfg->precision == CQL_PREC_F16X3,
-              "cql_create: bad precision");
-  CQL_REQUIRE(cfg->squash == CQL_SQUASH_EPS || cfg->squash == CQL_SQUASH_SOFTPLUS, "cql_create: bad squash");
-  CQL_REQUIRE(cfg->world_size >= 1 && cfg->rank >= 0 && cfg->rank < cfg->world_size, "cql_create: bad rank/world_size");
-  int ndev = 0;
-  cudaError_t e = cudaGetDeviceCount(&ndev);
-  if (e != cudaSuccess || ndev == 0)
-    throw Error{std::string("cql_create: no CUDA device available (") + cudaGetErrorString(e) +
-                "); this library has no CPU fallback"};
-  CQL_REQUIRE(cfg->device >= 0 && cfg->device < ndev, "cql_create: device ordinal out of range");
-  CQL_CUDA(cudaSetDevice(cfg->device));
-  cudaDeviceProp prop{};
-  CQL_CUDA(cudaGetDeviceProperties(&prop, cfg->device));
-  CQL_REQUIRE(prop.major >= 10, "cql_create: built for sm_100a (B200); found an older GPU");
-  h.cfg = *cfg;
-  h.num_sms = prop.multiProcessorCount;
-  h.B = cfg->batch_size; h.n = cfg->n_action_samples; h.C = cfg->n_critics;
+// Every device buffer of the update, from (B, C, n, precision) alone.  With h.plan_bytes set nothing is allocated: the
+// call only adds up the bytes (cql_create's sizing pass).
+void alloc_device_state(Handle& h) {
+  const cql_config* cfg = &h.cfg;
   const int B = h.B, n = h.n, C = h.C, n3 = 3 * n;
-  h.rsA = n3; h.rsC = n3 + 1;
-  CQL_CUDA(cudaStreamCreateWithFlags(&h.own_stream, cudaStreamNonBlocking));
-  CQL_CUDA(cudaStreamCreateWithFlags(&h.side_stream, cudaStreamNonBlocking));
-  CQL_CUDA(cudaEventCreateWithFlags(&h.ev_fork, cudaEventDisableTiming));
-  CQL_CUDA(cudaEventCreateWithFlags(&h.ev_join, cudaEventDisableTiming));
-  set_kernel_attrs();
-
   const int64_t S = state_floats(C);
   h.params = h.dalloc<float>(S);
   h.adam_m = h.dalloc<float>(S);
@@ -196,14 +168,10 @@ void create_impl(const cql_config* cfg, cql_handle* ch) {
   h.stepinfo = h.dalloc<StepInfo>(1);
   h.metrics = h.dalloc<float>(8);
   h.stats_dev = h.dalloc<double>(STATS_DEV_DOUBLES);
-  CQL_CUDA(cudaMallocHost(&h.stats_host, 4 * 5 * sizeof(double)));
-  CQL_CUDA(cudaMallocHost(&h.metrics_host, 8 * sizeof(float)));
   h.batch = h.dalloc<float>((size_t)B * 8);
   h.batch_in = h.dalloc<float>((size_t)B * 8);
-  CQL_CUDA(cudaMallocHost(&h.batch_host, (size_t)B * 8 * sizeof(float)));
   h.noise_floats = 2 * (int64_t)B + 6 * (int64_t)B * n;
   h.noise = h.dalloc<float>(h.noise_floats);
-  CQL_CUDA(cudaMallocHost(&h.noise_host, h.noise_floats * sizeof(float)));
   const int tB = tiles_of(B), rowsC = B * (n3 + 1), tC = tiles_of(rowsC);
   h.XA = h.dalloc<float4>(2 * (size_t)B);
   h.outA = h.dalloc<float>(4 * (size_t)B);
@@ -259,6 +227,64 @@ void create_impl(const cql_config* cfg, cql_handle* ch) {
     h.pw2_tc = h.dalloc<float>((size_t)(h.num_sms + C) * H * H);
     h.dX_part = h.dalloc<float4>((size_t)C * std::max(slices, 8) * B);
   }
+}
+
+void create_impl(const cql_config* cfg, cql_handle* ch) {
+  Handle& h = ch->h;
+  CQL_REQUIRE(cfg != nullptr, "cql_create: cfg is NULL");
+  CQL_REQUIRE(cfg->struct_size == (int32_t)sizeof(cql_config), "cql_create: cql_config size mismatch (ABI)");
+  CQL_REQUIRE(cfg->batch_size >= 1 && cfg->batch_size <= (1 << 20), "cql_create: batch_size out of range");
+  CQL_REQUIRE(cfg->n_critics >= 1 && cfg->n_critics <= CQL_MAX_CRITICS,
+              "cql_create: n_critics must be 1.." + std::to_string(CQL_MAX_CRITICS) + " (CQL_MAX_CRITICS)");
+  CQL_REQUIRE(cfg->n_action_samples >= 1 && cfg->n_action_samples <= CQL_MAX_ACTION_SAMPLES,
+              "cql_create: n_action_samples must be 1.." + std::to_string(CQL_MAX_ACTION_SAMPLES) + " (CQL_MAX_ACTION_SAMPLES)");
+  CQL_REQUIRE(cfg->precision == CQL_PREC_FP32 || cfg->precision == CQL_PREC_TF32X3 || cfg->precision == CQL_PREC_BF16 ||
+                  cfg->precision == CQL_PREC_F16X3,
+              "cql_create: bad precision");
+  CQL_REQUIRE(cfg->squash == CQL_SQUASH_EPS || cfg->squash == CQL_SQUASH_SOFTPLUS, "cql_create: bad squash");
+  CQL_REQUIRE(cfg->world_size >= 1 && cfg->rank >= 0 && cfg->rank < cfg->world_size, "cql_create: bad rank/world_size");
+  int ndev = 0;
+  cudaError_t e = cudaGetDeviceCount(&ndev);
+  if (e != cudaSuccess || ndev == 0)
+    throw Error{std::string("cql_create: no CUDA device available (") + cudaGetErrorString(e) +
+                "); this library has no CPU fallback"};
+  CQL_REQUIRE(cfg->device >= 0 && cfg->device < ndev, "cql_create: device ordinal out of range");
+  CQL_CUDA(cudaSetDevice(cfg->device));
+  cudaDeviceProp prop{};
+  CQL_CUDA(cudaGetDeviceProperties(&prop, cfg->device));
+  CQL_REQUIRE(prop.major >= 10, "cql_create: built for sm_100a (B200); found an older GPU");
+  h.cfg = *cfg;
+  h.num_sms = prop.multiProcessorCount;
+  h.B = cfg->batch_size; h.n = cfg->n_action_samples; h.C = cfg->n_critics;
+  h.rsA = 3 * h.n; h.rsC = 3 * h.n + 1;
+  CQL_CUDA(cudaStreamCreateWithFlags(&h.own_stream, cudaStreamNonBlocking));
+  CQL_CUDA(cudaStreamCreateWithFlags(&h.side_stream, cudaStreamNonBlocking));
+  CQL_CUDA(cudaEventCreateWithFlags(&h.ev_fork, cudaEventDisableTiming));
+  CQL_CUDA(cudaEventCreateWithFlags(&h.ev_join, cudaEventDisableTiming));
+  set_kernel_attrs();
+
+  // every device buffer of the handle, sized BEFORE anything is allocated: a configuration that cannot fit is rejected
+  // here (code 3, with the requirement), not by a failed cudaMalloc halfway through the buffers
+  size_t need = 0;
+  h.plan_bytes = &need;
+  alloc_device_state(h);
+  h.plan_bytes = nullptr;
+  size_t free_b = 0, total_b = 0;
+  CQL_CUDA(cudaMemGetInfo(&free_b, &total_b));
+  if (need > free_b) {
+    char msg[320];
+    snprintf(msg, sizeof msg,
+             "cql_create: batch_size %d, n_critics %d, n_action_samples %d (precision %d) need %.2f GiB of device memory "
+             "for the update's buffers; the device has %.2f GiB free of %.2f GiB",
+             cfg->batch_size, cfg->n_critics, cfg->n_action_samples, cfg->precision, need / 1073741824.0,
+             free_b / 1073741824.0, total_b / 1073741824.0);
+    throw ArgError{{msg}};
+  }
+  alloc_device_state(h);
+  CQL_CUDA(cudaMallocHost(&h.stats_host, 4 * 5 * sizeof(double)));
+  CQL_CUDA(cudaMallocHost(&h.metrics_host, 8 * sizeof(float)));
+  CQL_CUDA(cudaMallocHost(&h.batch_host, (size_t)h.B * 8 * sizeof(float)));
+  CQL_CUDA(cudaMallocHost(&h.noise_host, h.noise_floats * sizeof(float)));
   // scalars start at the configured initial values; networks are set by cql_set_weights
   float sc[SCALAR_SLOT] = {0};
   sc[0] = logf(cfg->initial_temperature);
@@ -513,13 +539,20 @@ int cql_create(const cql_config* cfg, cql_handle** out) {
   if (!out) { g_create_error = "cql_create: out is NULL"; return 1; }
   *out = nullptr;
   cql_handle* ch = new cql_handle();
+  int rc = 0;
   try {
     create_impl(cfg, ch);
+  } catch (const ArgError& e) {
+    g_create_error = e.msg;
+    rc = 3;
   } catch (const Error& e) {
     g_create_error = e.msg;
+    rc = 1;
+  }
+  if (rc != 0) {
     ch->h.free_all();
     delete ch;
-    return 1;
+    return rc;
   }
   *out = ch;
   return 0;

@@ -214,9 +214,14 @@ struct Handle {
   MdpSession* mdp = nullptr;       // between cql_mdp_begin and cql_mdp_finish
   uint8_t* mdp_ring = nullptr;     // pinned staging ring of the ingestion sessions
   std::vector<void*> allocs;
+  size_t* plan_bytes = nullptr;    // cql_create's sizing pass: dalloc adds the bytes here and allocates nothing
 
   template <typename T>
   T* dalloc(size_t count) {
+    if (plan_bytes) {              // (rounded to cudaMalloc's 256-byte alignment: a lower bound of what it will take)
+      *plan_bytes += (count * sizeof(T) + 255) / 256 * 256;
+      return nullptr;
+    }
     void* p = nullptr;
     CQL_CUDA(cudaMalloc(&p, count * sizeof(T)));
     CQL_CUDA(cudaMemset(p, 0, count * sizeof(T)));

@@ -82,7 +82,7 @@ __global__ void k_pack_w2(const float* __restrict__ params, int in_dim, int n_ne
 
 // several networks / orientations in ONE launch (after an Adam step: critics fwd + critics^T + targets fwd)
 struct PackJobs {
-  struct J { const float* net; uint8_t* dst; int in_dim, transpose; } j[12];
+  struct J { const float* net; uint8_t* dst; int in_dim, transpose; } j[3 * CQL_MAX_CRITICS];   // C critics (2 orientations) + C targets
   int n;
 };
 template <bool TF32>

@@ -462,6 +462,31 @@ __device__ __forceinline__ float warp_lse_v(float v, int cnt, int lane, float& m
   return m + logf(s);
 }
 
+// The same over a row of up to 32 * T values (3n + 1 > 32: n_action_samples 11..CQL_MAX_ACTION_SAMPLES), lane l holding
+// values l, l + 32, ..., l + 32 (T - 1) (value j < cnt valid).  Fixed order: each lane takes the max of its values, then
+// the sum of their exponentials, in t order; warp_max / warp_sum combine the lanes in their fixed butterfly -- the
+// same row always gives the same bits.  w_out[t] = softmax weight of value l + 32 t.
+template <int T>
+__device__ __forceinline__ float warp_lse_strided(const float (&v)[T], int cnt, int lane, float (&w_out)[T]) {
+  float m = -INFINITY;
+#pragma unroll
+  for (int t = 0; t < T; ++t)
+    if (lane + 32 * t < cnt) m = fmaxf(m, v[t]);
+  m = warp_max(m);
+  float e[T], s = 0.f;
+#pragma unroll
+  for (int t = 0; t < T; ++t) {
+    e[t] = lane + 32 * t < cnt ? expf(v[t] - m) : 0.f;
+    s += e[t];
+  }
+  s = warp_sum(s);
+#pragma unroll
+  for (int t = 0; t < T; ++t) w_out[t] = e[t] / s;
+  return m + logf(s);
+}
+// values per lane in k_lse's wide path: 3n + 1 <= 32 * LSE_STRIDE for every n the API accepts
+constexpr int LSE_STRIDE = (3 * CQL_MAX_ACTION_SAMPLES + 1 + 31) / 32;
+
 struct ScalarReduceArgs {
   const float4* perb; const float* scalars; const float* sc_m; const float* sc_v;
   float* g_scalars; float* sums; float* metrics; unsigned int* ticket;
@@ -469,6 +494,9 @@ struct ScalarReduceArgs {
 };
 __device__ void scalar_reduce_tail(const PairVals* __restrict__ pairv, const LossConsts& k, const ScalarReduceArgs& a);
 
+// WIDE = false: 3n + 1 <= 32 (n_action_samples <= 10), lane i holds row i, lane 3n the data row.  WIDE = true: up to
+// 3 * CQL_MAX_ACTION_SAMPLES + 1 rows, lane l holds rows l, l + 32, ... (warp_lse_strided); the data row is row 3n.
+template <bool WIDE>
 __global__ void __launch_bounds__(256) k_lse(const float4* __restrict__ batch, const QSrc srcAl,
                                              const float* __restrict__ offAl, const QSrc srcC,
                                              const float* __restrict__ offC, const QSrc srcT, LossConsts k,
@@ -479,15 +507,37 @@ __global__ void __launch_bounds__(256) k_lse(const float4* __restrict__ batch, c
   if (p < k.C * k.B) {
     const int c = p / k.B, b = p % k.B;
     const int n3 = 3 * k.n, rsC = n3 + 1;
-    float m, w;
     PairVals pv;
-    const float va = lane < n3 ? q_at(srcAl, c, b * n3 + lane) - offAl[(int64_t)b * n3 + lane] : 0.f;
-    pv.lse_a = warp_lse_v(va, n3, lane, m, w);
-    const float qc = lane < rsC ? q_at(srcC, c, b * rsC + lane) : 0.f;       // lane n3 = the data row (s, a)
-    const float vc = lane < n3 ? qc - offC[(int64_t)b * rsC + lane] : 0.f;
-    pv.lse_c = warp_lse_v(vc, n3, lane, m, w);
-    if (lane < n3) dQ[((int64_t)c * k.B + b) * rsC + lane] = w;
-    const float qd = __shfl_sync(0xffffffffu, qc, n3 & 31);
+    float qd;
+    if constexpr (!WIDE) {
+      float m, w;
+      const float va = lane < n3 ? q_at(srcAl, c, b * n3 + lane) - offAl[(int64_t)b * n3 + lane] : 0.f;
+      pv.lse_a = warp_lse_v(va, n3, lane, m, w);
+      const float qc = lane < rsC ? q_at(srcC, c, b * rsC + lane) : 0.f;       // lane n3 = the data row (s, a)
+      const float vc = lane < n3 ? qc - offC[(int64_t)b * rsC + lane] : 0.f;
+      pv.lse_c = warp_lse_v(vc, n3, lane, m, w);
+      if (lane < n3) dQ[((int64_t)c * k.B + b) * rsC + lane] = w;
+      qd = __shfl_sync(0xffffffffu, qc, n3 & 31);
+    } else {
+      float va[LSE_STRIDE], qc[LSE_STRIDE], vc[LSE_STRIDE], w[LSE_STRIDE];
+#pragma unroll
+      for (int t = 0; t < LSE_STRIDE; ++t) {
+        const int j = lane + 32 * t;
+        va[t] = j < n3 ? q_at(srcAl, c, b * n3 + j) - offAl[(int64_t)b * n3 + j] : 0.f;
+        qc[t] = j < rsC ? q_at(srcC, c, b * rsC + j) : 0.f;
+        vc[t] = j < n3 ? qc[t] - offC[(int64_t)b * rsC + j] : 0.f;
+      }
+      pv.lse_a = warp_lse_strided(va, n3, lane, w);
+      pv.lse_c = warp_lse_strided(vc, n3, lane, w);
+#pragma unroll
+      for (int t = 0; t < LSE_STRIDE; ++t)
+        if (lane + 32 * t < n3) dQ[((int64_t)c * k.B + b) * rsC + lane + 32 * t] = w[t];
+      float qdt = qc[0];                        // the data row: row n3 = lane n3 % 32 of stride n3 / 32
+#pragma unroll
+      for (int t = 1; t < LSE_STRIDE; ++t)
+        if (t == n3 / 32) qdt = qc[t];
+      qd = __shfl_sync(0xffffffffu, qdt, n3 & 31);
+    }
     if (lane == 0) {
       float qt = q_at(srcT, 0, b);
       for (int c2 = 1; c2 < k.C; ++c2) qt = fminf(qt, q_at(srcT, c2, b));
@@ -916,7 +966,7 @@ inline void pack_slots(Handle* h, const int* slots, int n_slots, cudaStream_t st
 }
 template <Prec P>
 inline void pack_weights(Handle* h, int slot, int n_slots, cudaStream_t st) {
-  int slots[8];
+  int slots[CQL_MAX_CRITICS];
   for (int i = 0; i < n_slots; ++i) slots[i] = slot + i;
   pack_slots<P>(h, slots, n_slots, st);
 }
@@ -1223,8 +1273,8 @@ inline void phase0(Handle* h, cudaStream_t st, BatchSource bs, NoiseSource ns) {
     const int64_t so = scalars_off(C);
     ScalarReduceArgs ra{reinterpret_cast<const float4*>(h->perb), h->scalars(), h->adam_m + so, h->adam_v + so, h->g_scalars(),
                         h->loss_sums, h->metrics, reinterpret_cast<unsigned int*>(h->loss_sums + 15), h->dp_fused ? h->dp : DpPeer{}};
-    launch(h, st, pdl_skip(2), k_lse, dim3((C * B * 32 + 255) / 256), dim3(256), 0, batch4, srcQ[0], h->offAl, srcQ[1], h->offC,
-           srcQ[2], loss_consts(h), h->dQ, reinterpret_cast<PairVals*>(h->pairv), ra);
+    launch(h, st, pdl_skip(2), 3 * h->n + 1 <= 32 ? &k_lse<false> : &k_lse<true>, dim3((C * B * 32 + 255) / 256), dim3(256), 0,
+           batch4, srcQ[0], h->offAl, srcQ[1], h->offC, srcQ[2], loss_consts(h), h->dQ, reinterpret_cast<PairVals*>(h->pairv), ra);
   }
 }
 

@@ -72,6 +72,17 @@ class CqlHyperParams:
     seed: int = 12345
     n_steps: int = 1           # n-step TD horizon of the replay table and the TD target (d3rlpy ``n_steps``)
 
+    def __post_init__(self):
+        check_ensemble(self.n_critics, self.n_action_samples)
+
+
+def check_ensemble(n_critics, n_action_samples) -> None:
+    """``ValueError`` unless 1 <= n_critics <= ``MAX_CRITICS`` and 1 <= n_action_samples <= ``MAX_ACTION_SAMPLES``."""
+    if not isinstance(n_critics, (int, np.integer)) or not 1 <= n_critics <= _lib.MAX_CRITICS:
+        raise ValueError(f"n_critics must be an integer in 1..{_lib.MAX_CRITICS}")
+    if not isinstance(n_action_samples, (int, np.integer)) or not 1 <= n_action_samples <= _lib.MAX_ACTION_SAMPLES:
+        raise ValueError(f"n_action_samples must be an integer in 1..{_lib.MAX_ACTION_SAMPLES}")
+
 
 def _ptr(arr: Optional[np.ndarray]):
     return None if arr is None else arr.ctypes.data_as(C.c_void_p)
@@ -121,7 +132,8 @@ class CqlEngine:
         if rc != 0:
             msg = self._lib.cql_last_error(None)
             self._h = None
-            raise _lib.CqlLibraryError(f"cql_create failed: {msg.decode() if msg else rc}")
+            err = _lib.CqlArgumentError if rc == 3 else _lib.CqlLibraryError
+            raise err(f"cql_create failed: {msg.decode() if msg else rc}")
         self.device, self.rank, self.world_size = device, rank, world_size
         self.n_state = int(self._lib.cql_state_floats(self._h))
         assert self.n_state == layout.state_floats(self.hp.n_critics)

@@ -15,7 +15,7 @@ from typing import Any, Dict, Optional
 import numpy as np
 import pandas as pd
 
-from .engine import OFFLINE_SUM_KEYS, CqlEngine, CqlHyperParams, offline_scores
+from .engine import OFFLINE_SUM_KEYS, CqlEngine, CqlHyperParams, check_ensemble, offline_scores
 from .mdp import build_mdp_on_device, seen_csr
 from .parallel import GradAllReducer, dist_info, gather_rows, shard_range
 from .recommender import Recommender, _rec_frame, get_top_k_recs
@@ -100,6 +100,7 @@ class CQL(Recommender):
         reward_scaler = scalers.validate("reward_scaler", reward_scaler)
         if not isinstance(n_steps, (int, np.integer)) or not 1 <= n_steps <= _lib.MAX_N_STEPS:
             raise ValueError(f"n_steps (the n-step TD horizon) must be an integer in 1..{_lib.MAX_N_STEPS}")
+        check_ensemble(n_critics, n_action_samples)
         if soft_q_backup:
             raise ValueError("soft_q_backup=True is not supported (d3rlpy default False is restated)")
         if not use_gpu:
