@@ -8,7 +8,6 @@
 #include "score.cuh"
 #include "tc_selftest.cuh"
 #include "score_tc.cuh"
-#include "score_tc_h.cuh"
 #include "topk_staged.cuh"
 #include "metrics.cuh"
 #include "dp_peer.cuh"
@@ -55,17 +54,28 @@ struct StepGraph {
   }
 };
 
+// grow-only device scratch of the host-pointer entry points: one buffer per slot, shared by the entry points
+enum ScratchSlot : int {
+  SCR_IN_A = 0,       // users (scoring), recommended lists (metrics)
+  SCR_IN_B = 1,       // items (scoring), users (metrics)
+  SCR_OUT_A = 2,      // top-k items (scoring), per-user metrics
+  SCR_OUT_B = 3,      // top-k or pair scores (scoring), metric means
+  SCR_CSR_PTR = 4,    // upload_csr: indptr
+  SCR_CSR_ITEMS = 5,  // upload_csr: items
+  SCR_ITEM_X = 7,     // scaled_items
+  SCR_SLOTS = 8
+};
+
 struct cql_handle {
   Handle h;
   StepGraph update_graph;            // one sampled update (phases 0-3): cql_update
   StepGraph batch_graph[2];          // the host-minibatch entry (cql_update_batch): [0] Philox noise, [1] caller-provided noise
-  // grow-only device scratch for the host-pointer scoring entry points
-  void* sbuf[8] = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr};
-  size_t sbuf_bytes[8] = {0, 0, 0, 0, 0, 0, 0, 0};
-  float* part_s = nullptr;
+  void* sbuf[SCR_SLOTS] = {};
+  size_t sbuf_bytes[SCR_SLOTS] = {};
+  float* part_s = nullptr;           // grow_partials
   int* part_i = nullptr;
   size_t part_elems = 0;
-  uint8_t* packed_score = nullptr;   // tf32-packed W2 of actor + critics for the tensor-core scorer
+  uint8_t* packed_score = nullptr;   // W2 of actor + critics in the tensor-core scorer's operand layout (pack_score_w2)
   // cql_update_batches: the bare step (minibatch already on the device) as a graph, pinned staging ring, metrics rows
   StepGraph step_graph;
   float* ring = nullptr;             // pinned [8][B*8]
@@ -92,7 +102,7 @@ int64_t mdp_build_on_device(Handle& h, const int32_t* user_h, const int32_t* ite
 
 namespace {
 
-void* scratch(cql_handle* ch, int slot, size_t bytes) {
+void* scratch(cql_handle* ch, ScratchSlot slot, size_t bytes) {
   if (bytes > ch->sbuf_bytes[slot]) {
     if (ch->sbuf[slot]) CQL_CUDA(cudaFree(ch->sbuf[slot]));
     ch->sbuf[slot] = nullptr;
@@ -117,8 +127,8 @@ void set_kernel_attrs() {
   CQL_CUDA(cudaFuncSetAttribute(k_topk_filter_staged, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)TKS_SMEM));
   CQL_CUDA(cudaFuncSetAttribute(tc::tc_fwd_kernel<false, 2, 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tc::FwdSmem<false, tc::FWD_NPW>::BYTES));
   CQL_CUDA(cudaFuncSetAttribute(tc::tc_fwd_kernel<false, 3, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tc::FwdSmem<false, tc::FWD_NPW>::BYTES));
-  CQL_CUDA(cudaFuncSetAttribute(tc::tc_score_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tc::ScoreSmem::bytes(CQL_MAX_TOPK)));
-  CQL_CUDA(cudaFuncSetAttribute(tc::tc_score_h_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tc::ScoreSmemH::bytes(CQL_MAX_TOPK)));
+  CQL_CUDA(cudaFuncSetAttribute(tc::tc_score_kernel<tc::SplitTf32>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tc::ScoreSmem<tc::SplitTf32::Cfg>::bytes(CQL_MAX_TOPK)));
+  CQL_CUDA(cudaFuncSetAttribute(tc::tc_score_kernel<tc::SplitF16>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tc::ScoreSmem<tc::SplitF16::Cfg>::bytes(CQL_MAX_TOPK)));
   CQL_CUDA(cudaFuncSetAttribute(tc::tc_bwd2_h_kernel<3, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tc::B2HCfg::BYTES));
   CQL_CUDA(cudaFuncSetAttribute(tc::tc_bwd2_h_kernel<2, 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tc::B2HCfg::BYTES));
   CQL_CUDA(cudaFuncSetAttribute(tc::tc_bwd2_h2_kernel<3, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tc::B2PCfg::BYTES));
@@ -351,10 +361,79 @@ void pack_rows(const Handle& h, const float* obs, const float* act, const float*
 const float* scaled_items(cql_handle* ch, const int32_t* items, int64_t I, cudaStream_t st) {
   Handle* h = &ch->h;
   if (!h->prep.obs[1].on) return nullptr;
-  float* out = static_cast<float*>(scratch(ch, 7, (size_t)I * sizeof(float)));
+  float* out = static_cast<float*>(scratch(ch, SCR_ITEM_X, (size_t)I * sizeof(float)));
   k_scale_items<<<(unsigned)((I + 255) / 256), 256, 0, st>>>(items, I, h->prep.obs[1], out);
   CQL_LAUNCH_CHECK(h);
   return out;
+}
+
+// grow-only partial top-k lists ([users][chunks][k]) of a scoring launch that splits users into chunks
+void grow_partials(cql_handle* ch, size_t need) {
+  if (need <= ch->part_elems) return;
+  if (ch->part_s) CQL_CUDA(cudaFree(ch->part_s));
+  if (ch->part_i) CQL_CUDA(cudaFree(ch->part_i));
+  ch->part_s = nullptr; ch->part_i = nullptr; ch->part_elems = 0;
+  CQL_CUDA(cudaMalloc(&ch->part_s, need * sizeof(float)));
+  CQL_CUDA(cudaMalloc(&ch->part_i, need * sizeof(int)));
+  ch->part_elems = need;
+}
+
+// a host CSR over user ids in the CSR scratch slots: indptr up to the largest id in `users`, then the items it spans.
+// `fn` and `items_arg` name the entry point and its items argument in error messages.
+struct DevCsr {
+  int64_t* indptr = nullptr;
+  int32_t* items = nullptr;
+};
+DevCsr upload_csr(cql_handle* ch, const char* fn, const int32_t* users, int64_t n_users, const int64_t* indptr,
+                  const int32_t* items, const char* items_arg, cudaStream_t st) {
+  int32_t mx = 0;
+  for (int64_t i = 0; i < n_users; ++i) {
+    CQL_REQUIRE(users[i] >= 0, std::string(fn) + ": negative user id");
+    mx = std::max(mx, users[i]);
+  }
+  const int64_t np = (int64_t)mx + 2, n = indptr[np - 1];
+  CQL_REQUIRE(n == 0 || items, std::string(fn) + ": " + items_arg + " is NULL");
+  DevCsr d;
+  d.indptr = (int64_t*)scratch(ch, SCR_CSR_PTR, (size_t)np * 8);
+  d.items = (int32_t*)scratch(ch, SCR_CSR_ITEMS, (size_t)std::max<int64_t>(1, n) * 4);
+  CQL_CUDA(cudaMemcpyAsync(d.indptr, indptr, (size_t)np * 8, cudaMemcpyHostToDevice, st));
+  if (n) CQL_CUDA(cudaMemcpyAsync(d.items, items, (size_t)n * 4, cudaMemcpyHostToDevice, st));
+  return d;
+}
+
+// the tensor-core scorer's copy of the actor's and critics' W2 (actor first, one packed net per slot) in the operand
+// layout of split S
+template <class S>
+void pack_score_w2(cql_handle* ch, cudaStream_t st) {
+  Handle* h = &ch->h;
+  constexpr size_t NET_BYTES = S::Cfg::PACKED_NET_BYTES;
+  if (!ch->packed_score) CQL_CUDA(cudaMalloc(&ch->packed_score, (size_t)(1 + h->C) * NET_BYTES));
+  if constexpr (S::TF32) {
+    const int chunks16 = H * (H / S::Cfg::EPC);
+    tc::k_pack_w2<true, false><<<dim3((chunks16 + 255) / 256, 1), 256, 0, st>>>(h->net_params(slot_actor()), 2, 1, ch->packed_score);
+    CQL_LAUNCH_CHECK(h);
+    tc::k_pack_w2<true, false><<<dim3((chunks16 + 255) / 256, h->C), 256, 0, st>>>(h->net_params(slot_critic(0)), 3, h->C,
+                                                                                   ch->packed_score + NET_BYTES);
+    CQL_LAUNCH_CHECK(h);
+  } else {
+    tc::PackJobs pj{};
+    pj.j[pj.n++] = {h->net_params(slot_actor()), ch->packed_score, 2, 0};
+    for (int c = 0; c < h->C; ++c) pj.j[pj.n++] = {h->net_params(slot_critic(c)), ch->packed_score + (size_t)(1 + c) * NET_BYTES, 3, 0};
+    tc::k_pack_multi_h<<<dim3(H * 32 / 256, pj.n), 256, 0, st>>>(pj, 2);
+    CQL_LAUNCH_CHECK(h);
+  }
+}
+
+// the tensor-core scorer in split S over a's (user, chunk) blocks; a.packed and a.item_x are filled in here
+template <class S>
+void score_tc(cql_handle* ch, tc::ScoreTcArgs a, cudaStream_t st) {
+  Handle* h = &ch->h;
+  pack_score_w2<S>(ch, st);
+  a.packed = ch->packed_score;
+  a.item_x = scaled_items(ch, a.items, a.n_items, st);
+  const int grid = (int)std::min<int64_t>(a.n_users * a.chunks, h->num_sms);
+  tc::tc_score_kernel<S><<<grid, S::Cfg::THREADS, tc::ScoreSmem<typename S::Cfg>::bytes(a.k), st>>>(a);
+  CQL_LAUNCH_CHECK(h);
 }
 
 void score_topk_dev_impl(cql_handle* ch, const int32_t* users, int64_t U, const int32_t* items, int64_t I,
@@ -374,49 +453,19 @@ void score_topk_dev_impl(cql_handle* ch, const int32_t* users, int64_t U, const 
     return;
   }
   if (h->cfg.precision != CQL_PREC_FP32) {   // tensor-core scorer, FP32-grade: fp16 hi/lo split (f16x3) or tf32 split (other modes)
-    using TC = tc::Cfg<true>;
-    const bool f16 = h->cfg.precision == CQL_PREC_F16X3;
-    if (!ch->packed_score)
-      CQL_CUDA(cudaMalloc(&ch->packed_score, (size_t)(1 + h->C) * std::max<size_t>(TC::PACKED_NET_BYTES, tc::HCfg::PACKED_NET_BYTES)));
-    if (f16) {
-      tc::PackJobs pj{};
-      pj.j[pj.n++] = {h->net_params(slot_actor()), ch->packed_score, 2, 0};
-      for (int c = 0; c < h->C; ++c)
-        pj.j[pj.n++] = {h->net_params(slot_critic(c)), ch->packed_score + (size_t)(1 + c) * tc::HCfg::PACKED_NET_BYTES, 3, 0};
-      tc::k_pack_multi_h<<<dim3(H * 32 / 256, pj.n), 256, 0, st>>>(pj, 2);
-      CQL_LAUNCH_CHECK(h);
-    } else {
-      const int chunks16 = H * (H / TC::EPC);
-      tc::k_pack_w2<true, false><<<dim3((chunks16 + 255) / 256, 1), 256, 0, st>>>(h->net_params(slot_actor()), 2, 1, ch->packed_score);
-      CQL_LAUNCH_CHECK(h);
-      tc::k_pack_w2<true, false><<<dim3((chunks16 + 255) / 256, h->C), 256, 0, st>>>(h->net_params(slot_critic(0)), 3, h->C,
-                                                                                     ch->packed_score + TC::PACKED_NET_BYTES);
-      CQL_LAUNCH_CHECK(h);
-    }
     const int64_t tiles128 = (I + tc::TM - 1) / tc::TM;
     const int chunks = (int)((tiles128 + tc::SC_CH - 1) / tc::SC_CH);
-    const size_t need = (size_t)U * chunks * k;
     float* ps = out_scores;
     int* pi = out_items;
     if (chunks > 1) {
-      if (need > ch->part_elems) {
-        if (ch->part_s) CQL_CUDA(cudaFree(ch->part_s));
-        if (ch->part_i) CQL_CUDA(cudaFree(ch->part_i));
-        ch->part_s = nullptr; ch->part_i = nullptr; ch->part_elems = 0;
-        CQL_CUDA(cudaMalloc(&ch->part_s, need * sizeof(float)));
-        CQL_CUDA(cudaMalloc(&ch->part_i, need * sizeof(int)));
-        ch->part_elems = need;
-      }
+      grow_partials(ch, (size_t)U * chunks * k);
       ps = ch->part_s;
       pi = ch->part_i;
     }
-    tc::ScoreTcArgs a{h->params, ch->packed_score, users, items, seen_indptr, seen_items, U, I, h->C, k, mode, chunks, ps, pi,
-                      scaled_items(ch, items, I, st), h->prep};
-    const int64_t n_blocks = U * chunks;
-    const int grid = (int)std::min<int64_t>(n_blocks, h->num_sms);
-    if (f16) tc::tc_score_h_kernel<<<grid, tc::HCfg4::THREADS, tc::ScoreSmemH::bytes(k), st>>>(a);
-    else tc::tc_score_kernel<<<grid, tc::TsCfg::THREADS, tc::ScoreSmem::bytes(k), st>>>(a);
-    CQL_LAUNCH_CHECK(h);
+    const tc::ScoreTcArgs a{h->params, nullptr, users, items, seen_indptr, seen_items, U, I, h->C, k, mode, chunks, ps, pi,
+                            nullptr, h->prep};
+    if (h->cfg.precision == CQL_PREC_F16X3) score_tc<tc::SplitF16>(ch, a, st);
+    else score_tc<tc::SplitTf32>(ch, a, st);
     if (chunks > 1) {
       const int wpb = 4;
       k_topk_merge<<<(unsigned)((U + wpb - 1) / wpb), wpb * 32, wpb * 2 * k * sizeof(float), st>>>(ps, pi, U, chunks, k,
@@ -448,15 +497,7 @@ void score_topk_dev_impl(cql_handle* ch, const int32_t* users, int64_t U, const 
       s.part_s = out_scores + u0 * k;
       s.part_i = out_items + u0 * k;
     } else {
-      const size_t need = (size_t)nu * chunks * k;
-      if (need > ch->part_elems) {
-        if (ch->part_s) CQL_CUDA(cudaFree(ch->part_s));
-        if (ch->part_i) CQL_CUDA(cudaFree(ch->part_i));
-        ch->part_s = nullptr; ch->part_i = nullptr; ch->part_elems = 0;
-        CQL_CUDA(cudaMalloc(&ch->part_s, need * sizeof(float)));
-        CQL_CUDA(cudaMalloc(&ch->part_i, need * sizeof(int)));
-        ch->part_elems = need;
-      }
+      grow_partials(ch, (size_t)nu * chunks * k);
       s.part_s = ch->part_s;
       s.part_i = ch->part_i;
     }
@@ -563,7 +604,7 @@ void cql_destroy(cql_handle* ch) {
   cudaSetDevice(ch->h.cfg.device);
   cudaDeviceSynchronize();
   destroy_graph(ch);
-  for (int i = 0; i < 8; ++i) if (ch->sbuf[i]) cudaFree(ch->sbuf[i]);
+  for (int i = 0; i < SCR_SLOTS; ++i) if (ch->sbuf[i]) cudaFree(ch->sbuf[i]);
   if (ch->part_s) cudaFree(ch->part_s);
   if (ch->part_i) cudaFree(ch->part_i);
   if (ch->packed_score) cudaFree(ch->packed_score);
@@ -1157,31 +1198,15 @@ int cql_score_topk(cql_handle* ch, const int32_t* users, int64_t n_users, const 
     CQL_REQUIRE(k >= 1 && k <= CQL_MAX_TOPK, "cql_score_topk: k must be 1..1024");
     if (n_users == 0) return;
     cudaStream_t st = pick_stream(&ch->h, stream);
-    int32_t* d_users = (int32_t*)scratch(ch, 0, (size_t)n_users * 4);
-    int32_t* d_items = (int32_t*)scratch(ch, 1, (size_t)std::max<int64_t>(1, n_items) * 4);
-    int32_t* d_oi = (int32_t*)scratch(ch, 2, (size_t)n_users * k * 4);
-    float* d_os = (float*)scratch(ch, 3, (size_t)n_users * k * 4);
+    int32_t* d_users = (int32_t*)scratch(ch, SCR_IN_A, (size_t)n_users * 4);
+    int32_t* d_items = (int32_t*)scratch(ch, SCR_IN_B, (size_t)std::max<int64_t>(1, n_items) * 4);
+    int32_t* d_oi = (int32_t*)scratch(ch, SCR_OUT_A, (size_t)n_users * k * 4);
+    float* d_os = (float*)scratch(ch, SCR_OUT_B, (size_t)n_users * k * 4);
     CQL_CUDA(cudaMemcpyAsync(d_users, users, (size_t)n_users * 4, cudaMemcpyHostToDevice, st));
     if (n_items) CQL_CUDA(cudaMemcpyAsync(d_items, items, (size_t)n_items * 4, cudaMemcpyHostToDevice, st));
-    int64_t* d_ptr = nullptr;
-    int32_t* d_seen = nullptr;
-    if (seen_indptr) {
-      int32_t mx = 0;
-      for (int64_t i = 0; i < n_users; ++i) {
-        CQL_REQUIRE(users[i] >= 0, "cql_score_topk: negative user id");
-        mx = std::max(mx, users[i]);
-      }
-      const int64_t np = (int64_t)mx + 2;
-      const int64_t ns = seen_indptr[np - 1];
-      d_ptr = (int64_t*)scratch(ch, 4, (size_t)np * 8);
-      d_seen = (int32_t*)scratch(ch, 5, (size_t)std::max<int64_t>(1, ns) * 4);
-      CQL_CUDA(cudaMemcpyAsync(d_ptr, seen_indptr, (size_t)np * 8, cudaMemcpyHostToDevice, st));
-      if (ns) {
-        CQL_REQUIRE(seen_items, "cql_score_topk: seen_items is NULL");
-        CQL_CUDA(cudaMemcpyAsync(d_seen, seen_items, (size_t)ns * 4, cudaMemcpyHostToDevice, st));
-      }
-    }
-    score_topk_dev_impl(ch, d_users, n_users, d_items, n_items, d_ptr, d_seen, k, mode, d_oi, d_os, st);
+    DevCsr seen{};
+    if (seen_indptr) seen = upload_csr(ch, "cql_score_topk", users, n_users, seen_indptr, seen_items, "seen_items", st);
+    score_topk_dev_impl(ch, d_users, n_users, d_items, n_items, seen.indptr, seen.items, k, mode, d_oi, d_os, st);
     CQL_CUDA(cudaMemcpyAsync(out_items, d_oi, (size_t)n_users * k * 4, cudaMemcpyDeviceToHost, st));
     CQL_CUDA(cudaMemcpyAsync(out_scores, d_os, (size_t)n_users * k * 4, cudaMemcpyDeviceToHost, st));
     CQL_CUDA(cudaStreamSynchronize(st));
@@ -1196,9 +1221,9 @@ int cql_score_pairs(cql_handle* ch, const int32_t* users, const int32_t* items, 
     CQL_REQUIRE(mode == CQL_SCORE_Q || mode == CQL_SCORE_POLICY, "cql_score_pairs: bad mode");
     if (n == 0) return;
     cudaStream_t st = pick_stream(&h, stream);
-    int32_t* d_u = (int32_t*)scratch(ch, 0, (size_t)n * 4);
-    int32_t* d_i = (int32_t*)scratch(ch, 1, (size_t)n * 4);
-    float* d_o = (float*)scratch(ch, 3, (size_t)n * 4);
+    int32_t* d_u = (int32_t*)scratch(ch, SCR_IN_A, (size_t)n * 4);
+    int32_t* d_i = (int32_t*)scratch(ch, SCR_IN_B, (size_t)n * 4);
+    float* d_o = (float*)scratch(ch, SCR_OUT_B, (size_t)n * 4);
     CQL_CUDA(cudaMemcpyAsync(d_u, users, (size_t)n * 4, cudaMemcpyHostToDevice, st));
     CQL_CUDA(cudaMemcpyAsync(d_i, items, (size_t)n * 4, cudaMemcpyHostToDevice, st));
     k_score_pairs<<<(unsigned)((n + BM - 1) / BM), NT, FWD_SMEM, st>>>(h.params, d_u, d_i, n, h.C, mode, d_o, h.prep);
@@ -1222,25 +1247,15 @@ int cql_rank_metrics(cql_handle* ch, const int32_t* rec_items, int64_t n_users, 
     }
     CQL_REQUIRE(rec_items && users && gt_indptr, "cql_rank_metrics: NULL input");
     cudaStream_t st = pick_stream(&h, stream);
-    int32_t mx = 0;
-    for (int64_t i = 0; i < n_users; ++i) {
-      CQL_REQUIRE(users[i] >= 0, "cql_rank_metrics: negative user id");
-      mx = std::max(mx, users[i]);
-    }
-    const int64_t np = (int64_t)mx + 2, ng = gt_indptr[np - 1];
-    CQL_REQUIRE(ng == 0 || gt_items, "cql_rank_metrics: gt_items is NULL");
-    int32_t* d_rec = (int32_t*)scratch(ch, 0, (size_t)n_users * k_rec * 4);
-    int32_t* d_users = (int32_t*)scratch(ch, 1, (size_t)n_users * 4);
-    int64_t* d_ptr = (int64_t*)scratch(ch, 4, (size_t)np * 8);
-    int32_t* d_gt = (int32_t*)scratch(ch, 5, (size_t)std::max<int64_t>(1, ng) * 4);
-    double* d_pu = (double*)scratch(ch, 2, (size_t)MET_COUNT * n_ks * n_users * 8);
-    double* d_out = (double*)scratch(ch, 3, (size_t)MET_COUNT * n_ks * 8);
+    const DevCsr gt = upload_csr(ch, "cql_rank_metrics", users, n_users, gt_indptr, gt_items, "gt_items", st);
+    int32_t* d_rec = (int32_t*)scratch(ch, SCR_IN_A, (size_t)n_users * k_rec * 4);
+    int32_t* d_users = (int32_t*)scratch(ch, SCR_IN_B, (size_t)n_users * 4);
+    double* d_pu = (double*)scratch(ch, SCR_OUT_A, (size_t)MET_COUNT * n_ks * n_users * 8);
+    double* d_out = (double*)scratch(ch, SCR_OUT_B, (size_t)MET_COUNT * n_ks * 8);
     CQL_CUDA(cudaMemcpyAsync(d_rec, rec_items, (size_t)n_users * k_rec * 4, cudaMemcpyHostToDevice, st));
     CQL_CUDA(cudaMemcpyAsync(d_users, users, (size_t)n_users * 4, cudaMemcpyHostToDevice, st));
-    CQL_CUDA(cudaMemcpyAsync(d_ptr, gt_indptr, (size_t)np * 8, cudaMemcpyHostToDevice, st));
-    if (ng) CQL_CUDA(cudaMemcpyAsync(d_gt, gt_items, (size_t)ng * 4, cudaMemcpyHostToDevice, st));
     MetricArgs ma{};
-    ma.rec_items = d_rec; ma.users = d_users; ma.gt_indptr = d_ptr; ma.gt_items = d_gt;
+    ma.rec_items = d_rec; ma.users = d_users; ma.gt_indptr = gt.indptr; ma.gt_items = gt.items;
     ma.n_users = n_users; ma.k_rec = k_rec; ma.n_ks = n_ks; ma.per_user = d_pu;
     for (int q = 0; q < n_ks; ++q) ma.ks[q] = ks[q];
     k_rank_metrics<<<(unsigned)((n_users + 127) / 128), 128, 0, st>>>(ma);

@@ -324,7 +324,7 @@ class CQL(Recommender):
         if kk <= 0:                                     # k = 0: nothing to recommend (the reference returns an empty frame)
             return _rec_frame([], [], [])
         from . import _lib
-        on_device = kk <= _lib.MAX_TOPK and u_local.size > 0 and hasattr(self.engine, "seen_csr_device")
+        on_device = kk <= _lib.MAX_TOPK and u_local.size > 0
         n_dim = int(u.max()) + 1
         if filter_seen_items and log is not None and len(log):
             wanted = np.zeros(n_dim, dtype=np.uint8)     # rows of the requested users: a table lookup, not isin()'s sort

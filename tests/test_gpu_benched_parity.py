@@ -9,7 +9,7 @@
   comparison documents a spot where the CPU float32 path itself misses (SURVEY.md:289-291: raw indices as floats).
   Every step restarts from the oracle's state WITH non-trivial Adam moments, so the weights move by
   lr * m / (sqrt(v) + eps) with the gradient's magnitude in it, not just by its sign (first-step Adam).
-* fused scorer (tc_score_h_kernel): I = 26 744 items, U = 2048 users, the bench's heavy-tailed seen lists, against
+* fused scorer (tc_score_kernel<SplitF16>): I = 26 744 items, U = 2048 users, the bench's heavy-tailed seen lists, against
   the brute-force per-user oracle on a user sample.
 """
 import numpy as np
@@ -73,7 +73,7 @@ def test_update_on_benched_configuration(engine_factory, precision, B, n_users, 
 
 
 def test_fused_scorer_at_baseline_item_count(engine_factory):
-    """tc_score_h_kernel on the BASELINE shape: all 26 744 items, 2048 users, the ML-20M-shaped log's real
+    """tc_score_kernel<SplitF16> on the BASELINE shape: all 26 744 items, 2048 users, the ML-20M-shaped log's real
     heavy-tailed seen lists (a few users have thousands of seen items), k = 10 -- scores within 1e-5 of max|Q| and
     lists identical up to (near-)ties against the brute-force oracle on 24 of the users (first, last, the three
     longest seen lists, and a random draw)."""

@@ -8,9 +8,10 @@ merge:
     precision      top-k scorer                                       fold                                  merge
     fp32           k_score_topk (64-item tiles, grid (chunks, users)  warp_fold_tile                        k_topk_merge when
                    in slabs of 65 535 users)                                                                chunks > 1
-    tf32x3, bf16   tc_score_kernel (W2 packed by k_pack_w2,           fold_block_select for k <= 32,        k_topk_merge when
-                   gridDim.y = C)                                     warp 0's sequential fold for k > 32   I > 2048
-    f16x3          tc_score_h_kernel (k_pack_multi_h, C + 1 jobs)     same                                  same
+    tf32x3, bf16   tc_score_kernel<SplitTf32> (W2 packed by           fold_block_select for k <= 32,        k_topk_merge when
+                   k_pack_w2, gridDim.y = C)                          warp 0's sequential fold for k > 32   I > 2048
+    f16x3          tc_score_kernel<SplitF16> (k_pack_multi_h,         same                                  same
+                   C + 1 jobs)
     all            k_score_pairs                                      --                                    --
 
 A tensor-core block is SC_CH * 128 = 2048 items of one user; the U * chunks blocks are split over min(U * chunks, SMs)
