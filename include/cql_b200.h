@@ -339,6 +339,31 @@ typedef struct cql_offline_sums {
 } cql_offline_sums;
 int  cql_offline_eval(cql_handle* h, float return_threshold, cql_offline_sums* out, void* stream);
 
+/* Fitted Q evaluation (DESIGN.md section 1, "FQE").  An FQE handle is an ordinary handle -- created with
+ * n_action_samples = 1, critic_lr = FQE's learning rate, betas (0.9, 0.999), eps 1e-8, FQE's batch size, gamma and seed
+ * -- whose actor slot holds the frozen policy pi(x) = tanh(mu(x)) and whose critic slots hold the FQE critics (target
+ * slots equal to them).  One update on minibatch rows (s, a, r | s', term, discount), scalers applied as in the CQL update:
+ *   y = r + gamma_k * min_c Q_targ_c(s', pi(s')) * (1 - term)   (gamma_k = the row's slot-7 discount when n_steps > 1)
+ *   loss = sum_c mean_b (Q_c(s, a) - y)^2, then Adam on the critics with the handle's step counter.
+ * The target is a hard copy: bit-equal to the critics after updates 1, 1 + I, 1 + 2I, ... (1-based, I =
+ * target_update_interval) and bit-unchanged after every other update.  The actor slot never changes.
+ * cql_fqe_enable: puts a handle that has run no update (step counter 0) into FQE mode; afterwards cql_update,
+ *   cql_update_batch, cql_update_batch_rows, cql_update_batches, cql_step_phase, cql_upload_batch and cql_timed_update
+ *   return 3.  Weights, optimizer state, table producers, preprocessing, scoring and cql_offline_eval work unchanged
+ *   (cql_offline_eval on an FQE handle is d3rlpy's scorers applied to the FQE object).
+ * cql_fqe_update: n_steps sampled updates; minibatch rows at epoch-permutation positions (step * B + j), the rows
+ *   cql_sample_rows returns for the same positions.  loss_out (may be NULL) receives the last update's loss.
+ * cql_fqe_update_rows: one update on rows_host [B][8] (the table's row format, raw); the same target schedule.
+ *   loss_out and grads_out ([n_critics][NET_STRIDE] critic gradients) may be NULL.  Synchronises.
+ * replaces: d3rlpy.ope.FQE.fit / FQEImpl.update, update_target [EXT d3rlpy 1.x ope/fqe.py, ope/torch/fqe_impl.py] */
+int  cql_fqe_enable(cql_handle* h, int32_t target_update_interval);
+int  cql_fqe_update(cql_handle* h, int64_t n_steps, float* loss_out, void* stream);
+int  cql_fqe_update_rows(cql_handle* h, const float* rows_host, float* loss_out, float* grads_out, void* stream);
+
+/* The replay table of `src` (rows and column statistics) copied device to device into `dst`; both handles on one device
+ * with the same n-step horizon (cql_set_n_steps), else 3.  `src` is not modified.  Synchronises. */
+int  cql_copy_table(cql_handle* dst, const cql_handle* src, void* stream);
+
 /* Measurement aid: runs ONE sampled update with CUDA events around the heavy launches and
  * returns their durations in milliseconds (synchronises).  out_ms[0] = critic forward (alpha +
  * critic + target rows), [1] = critic backward-1, [2] = critic backward-2 (dW2), [3] = whole

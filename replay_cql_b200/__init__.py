@@ -10,5 +10,14 @@ Only what the path needs lives here:
 * ``recommender``  pandas/pyarrow mirror of RePlay's ``Recommender`` template methods
 * ``models``       ``CQL`` -- the drop-in model class
 * ``model_handler`` ``save`` / ``load`` with the reference's directory layout
+* ``ope``          ``FQE`` -- fitted Q evaluation of a trained ``CQL`` policy (``replay_cql_b200.FQE``)
 """
 __version__ = "0.1.0"
+
+
+def __getattr__(name):
+    # imported on first use: the package itself stays light to import
+    if name == "FQE":
+        from .ope import FQE
+        return FQE
+    raise AttributeError(f"module {__name__!r} has no attribute {name!r}")

@@ -127,6 +127,10 @@ SIGNATURES = {
     "cql_selftest_umma": (C.c_int, [_P, C.c_int, _P, _P, C.c_int, C.c_int, _P]),
     "cql_offline_eval": (C.c_int, [_P, C.c_float, C.POINTER(OfflineSums), _P]),
     "cql_launch_count": (C.c_int64, [_P]),
+    "cql_fqe_enable": (C.c_int, [_P, C.c_int32]),
+    "cql_fqe_update": (C.c_int, [_P, C.c_int64, _P, _P]),
+    "cql_fqe_update_rows": (C.c_int, [_P, _P, _P, _P, _P]),
+    "cql_copy_table": (C.c_int, [_P, _P, _P]),
 }
 
 _lib = None

@@ -13,6 +13,7 @@
 #include "dp_peer.cuh"
 #include "mma_bench.cuh"
 #include "offline_eval.cuh"
+#include "fqe.cuh"
 
 using namespace cql;
 
@@ -91,6 +92,9 @@ struct cql_handle {
   cudaEvent_t ev_met[8] = {};        // compute stream: slot's metrics are in dev_metrics
   cudaEvent_t ev_met_out[8] = {};    // copy stream: slot's metrics have left dev_metrics
   void* dp_local = nullptr;          // epochs | tickets | error flag
+  // FQE mode (cql_fqe_enable): sampled updates, updates on caller rows, and the target synchronisation
+  FqeState fqe;
+  StepGraph fqe_graph, fqe_rows_graph, fqe_sync_graph;
 };
 
 static thread_local std::string g_create_error;
@@ -306,6 +310,58 @@ void destroy_graph(cql_handle* ch) {
   ch->update_graph.reset();
   for (auto& g : ch->batch_graph) g.reset();
   ch->step_graph.reset();
+  ch->fqe_graph.reset();
+  ch->fqe_rows_graph.reset();
+  ch->fqe_sync_graph.reset();
+}
+
+// the CQL update entry points refuse an FQE handle (its critics would otherwise take CQL steps)
+void require_cql_mode(const cql_handle* ch, const char* fn) {
+  CQL_REQUIRE(!ch->fqe.on, std::string(fn) + ": the handle is in FQE mode (cql_fqe_enable); use cql_fqe_update");
+}
+
+// FQE updates (sampled, or one on the caller's rows staged in h.batch_in) continuing from the device step counter
+// `done`; the target is synchronised after every update whose 0-based index is a multiple of the interval
+void fqe_run(cql_handle* ch, int64_t n, bool rows, long long done, cudaStream_t st) {
+  Handle& h = ch->h;
+  StepGraph& g = rows ? ch->fqe_rows_graph : ch->fqe_graph;
+  auto step = [&] {
+    if (rows) CQL_CUDA(cudaMemcpyAsync(h.batch_in, h.batch_host, (size_t)h.B * 8 * sizeof(float), cudaMemcpyHostToDevice, st));
+    with_precision(&h, [&](auto p) {
+      fqe_step<decltype(p)::value>(&h, ch->fqe, st, rows ? reinterpret_cast<const float4*>(h.batch_in) : nullptr);
+    });
+  };
+  const int64_t I = ch->fqe.interval;
+  for (int64_t i = 0; i < n;) {
+    const int64_t k = (done + i) % I;
+    const int64_t m = k == 0 ? 1 : std::min<int64_t>(n - i, I - k);
+    g.run(h, st, m, step);
+    if (k == 0) ch->fqe_sync_graph.run(h, st, 1, [&] { fqe_sync_target(&h, st); });
+    i += m;
+  }
+}
+
+// the device step counter, after the work queued on st
+long long completed_updates(Handle& h, cudaStream_t st) {
+  long long done = 0;
+  CQL_CUDA(cudaMemcpyAsync(h.metrics_host, h.step_dev, sizeof(done), cudaMemcpyDeviceToHost, st));
+  CQL_CUDA(cudaStreamSynchronize(st));
+  std::memcpy(&done, h.metrics_host, sizeof(done));
+  return done;
+}
+
+// the statistics of the table's one-step rows (cql_get_table_stats), from the producer's pending copy if it has not
+// been read yet
+cql_table_stats current_stats(const Handle& h) {
+  if (!h.stats_pending) return h.stats;
+  CQL_CUDA(cudaDeviceSynchronize());   // the producer's asynchronous copy: every producer synchronises before returning
+  cql_table_stats s{};
+  const double* m = h.stats_host;      // per column: n, mean, m2, min, max (struct Moments)
+  for (int c = 0; c < 4; ++c)
+    s.col[c] = cql_column_stats{(int64_t)m[5 * c], m[5 * c + 3], m[5 * c + 4], m[5 * c + 1], m[5 * c + 2]};
+  s.rew_available = h.stats_rew_ok ? 1 : 0;
+  if (!h.stats_rew_ok) s.col[3] = cql_column_stats{};
+  return s;
 }
 
 template <typename F>
@@ -731,13 +787,8 @@ int cql_get_table_stats(cql_handle* ch, cql_table_stats* out) {
   return guarded(ch, [&] {
     CQL_REQUIRE(out != nullptr, "cql_get_table_stats: NULL output");
     Handle& h = ch->h;
-    if (h.stats_pending) {            // the producer's asynchronous copy: every producer synchronises before returning
-      CQL_CUDA(cudaDeviceSynchronize());
-      const double* m = h.stats_host;   // per column: n, mean, m2, min, max (struct Moments)
-      for (int c = 0; c < 4; ++c)
-        h.stats.col[c] = cql_column_stats{(int64_t)m[5 * c], m[5 * c + 3], m[5 * c + 4], m[5 * c + 1], m[5 * c + 2]};
-      h.stats.rew_available = h.stats_rew_ok ? 1 : 0;
-      if (!h.stats_rew_ok) h.stats.col[3] = cql_column_stats{};
+    if (h.stats_pending) {
+      h.stats = current_stats(h);
       h.stats_pending = false;
     }
     *out = h.n_trans > 0 ? h.stats : cql_table_stats{};
@@ -867,6 +918,7 @@ int cql_sample_rows(cql_handle* ch, const int64_t* idx_dev, int64_t pos, int64_t
 
 int cql_update(cql_handle* ch, int64_t n_steps, float* metrics6, void* stream) {
   return guarded(ch, [&] {
+    require_cql_mode(ch, "cql_update");
     NvtxRange nvtx("cql_update: graph replays");
     Handle& h = ch->h;
     CQL_REQUIRE(n_steps >= 0, "cql_update: n_steps < 0");
@@ -946,6 +998,7 @@ int cql_mma_bench(cql_handle* ch, int mode, int iters, int64_t* out_clk2) {
 
 int cql_timed_update(cql_handle* ch, float* out_ms8, void* stream) {
   return guarded(ch, [&] {
+    require_cql_mode(ch, "cql_timed_update");
     Handle& h = ch->h;
     CQL_REQUIRE(out_ms8 != nullptr, "cql_timed_update: out is NULL");
     CQL_REQUIRE(h.n_trans > 0, "cql_timed_update: no transitions loaded");
@@ -974,6 +1027,7 @@ int cql_timed_update(cql_handle* ch, float* out_ms8, void* stream) {
 int cql_update_batch(cql_handle* ch, const float* obs, const float* act, const float* rew, const float* next_obs,
                      const float* term, const float* noise, float* metrics6, float* grads_out, void* stream) {
   return guarded(ch, [&] {
+    require_cql_mode(ch, "cql_update_batch");
     Handle& h = ch->h;
     CQL_REQUIRE(obs && act && rew && next_obs && term, "cql_update_batch: NULL batch pointer");
     cudaStream_t st = pick_stream(&h, stream);
@@ -985,6 +1039,7 @@ int cql_update_batch(cql_handle* ch, const float* obs, const float* act, const f
 int cql_update_batch_rows(cql_handle* ch, const float* rows, const float* noise, float* metrics6, float* grads_out,
                           void* stream) {
   return guarded(ch, [&] {
+    require_cql_mode(ch, "cql_update_batch_rows");
     Handle& h = ch->h;
     CQL_REQUIRE(rows != nullptr, "cql_update_batch_rows: NULL rows");
     cudaStream_t st = pick_stream(&h, stream);
@@ -996,6 +1051,7 @@ int cql_update_batch_rows(cql_handle* ch, const float* rows, const float* noise,
 int cql_update_batches(cql_handle* ch, int64_t n_batches, const float* obs, const float* act, const float* rew,
                        const float* next_obs, const float* term, float* metrics_out, void* stream) {
   return guarded(ch, [&] {
+    require_cql_mode(ch, "cql_update_batches");
     NvtxRange nvtx("cql_update_batches");
     Handle& h = ch->h;
     CQL_REQUIRE(n_batches >= 0, "cql_update_batches: n_batches < 0");
@@ -1063,6 +1119,7 @@ int cql_update_batches(cql_handle* ch, int64_t n_batches, const float* obs, cons
 int cql_upload_batch(cql_handle* ch, const float* obs, const float* act, const float* rew, const float* next_obs,
                      const float* term, void* stream) {
   return guarded(ch, [&] {
+    require_cql_mode(ch, "cql_upload_batch");
     Handle& h = ch->h;
     CQL_REQUIRE(obs && act && rew && next_obs && term, "cql_upload_batch: NULL batch pointer");
     cudaStream_t st = pick_stream(&h, stream);
@@ -1075,6 +1132,7 @@ int cql_upload_batch(cql_handle* ch, const float* obs, const float* act, const f
 
 int cql_step_phase(cql_handle* ch, int phase, void* stream) {
   return guarded(ch, [&] {
+    require_cql_mode(ch, "cql_step_phase");
     Handle& h = ch->h;
     cudaStream_t st = pick_stream(&h, stream);
     with_precision(&h, [&](auto p) {
@@ -1307,6 +1365,83 @@ int cql_offline_eval(cql_handle* ch, float return_threshold, cql_offline_sums* o
     double s[OE_SUMS];
     with_precision(&h, [&](auto p) { offline_eval<decltype(p)::value>(&h, return_threshold, s, pick_stream(&h, stream)); });
     *out = cql_offline_sums{s[0], s[1], s[2], s[3], s[4], s[5], s[6], s[7], h.n_trans, (int64_t)s[8], (int64_t)s[9]};
+  });
+}
+
+int cql_fqe_enable(cql_handle* ch, int32_t target_update_interval) {
+  return guarded(ch, [&] {
+    Handle& h = ch->h;
+    CQL_REQUIRE(target_update_interval >= 1, "cql_fqe_enable: target_update_interval must be >= 1");
+    CQL_CUDA(cudaDeviceSynchronize());
+    long long done = 0;
+    CQL_CUDA(cudaMemcpy(&done, h.step_dev, sizeof(done), cudaMemcpyDeviceToHost));
+    CQL_REQUIRE(done == 0, "cql_fqe_enable: the handle has already run updates (step counter != 0)");
+    FqeState& fq = ch->fqe;
+    if (!fq.on) {
+      fq.sink.params = h.dalloc<float>((size_t)h.C * NET_STRIDE);
+      if (h.packed_fwd) fq.sink.fwd = h.dalloc<uint8_t>((size_t)h.C * h.packed_net_bytes);
+      if (h.packed_fwd2) fq.sink.fwd2 = h.dalloc<uint8_t>((size_t)h.C * h.packed_net_bytes2);
+    }
+    fq.on = true;
+    fq.interval = target_update_interval;
+    destroy_graph(ch);
+  });
+}
+
+int cql_fqe_update(cql_handle* ch, int64_t n_steps, float* loss_out, void* stream) {
+  return guarded(ch, [&] {
+    NvtxRange nvtx("cql_fqe_update: graph replays");
+    Handle& h = ch->h;
+    CQL_REQUIRE(ch->fqe.on, "cql_fqe_update: the handle is not in FQE mode (call cql_fqe_enable first)");
+    CQL_REQUIRE(n_steps >= 0, "cql_fqe_update: n_steps < 0");
+    CQL_REQUIRE(h.n_trans > 0, "cql_fqe_update: no transitions loaded");
+    cudaStream_t st = pick_stream(&h, stream);
+    if (n_steps > 0) fqe_run(ch, n_steps, false, completed_updates(h, st), st);
+    if (loss_out) {
+      CQL_CUDA(cudaMemcpyAsync(h.metrics_host, fqe_loss(&h), sizeof(float), cudaMemcpyDeviceToHost, st));
+      CQL_CUDA(cudaStreamSynchronize(st));
+      *loss_out = h.metrics_host[0];
+    }
+  });
+}
+
+int cql_fqe_update_rows(cql_handle* ch, const float* rows_host, float* loss_out, float* grads_out, void* stream) {
+  return guarded(ch, [&] {
+    Handle& h = ch->h;
+    CQL_REQUIRE(ch->fqe.on, "cql_fqe_update_rows: the handle is not in FQE mode (call cql_fqe_enable first)");
+    CQL_REQUIRE(rows_host != nullptr, "cql_fqe_update_rows: NULL rows");
+    cudaStream_t st = pick_stream(&h, stream);
+    const long long done = completed_updates(h, st);     // (also: the staging buffer is no longer in flight)
+    std::memcpy(h.batch_host, rows_host, (size_t)h.B * 8 * sizeof(float));
+    fqe_run(ch, 1, true, done, st);
+    if (grads_out)
+      CQL_CUDA(cudaMemcpyAsync(grads_out, h.g_critics(), (size_t)h.C * NET_STRIDE * sizeof(float), cudaMemcpyDeviceToHost, st));
+    CQL_CUDA(cudaMemcpyAsync(h.metrics_host, fqe_loss(&h), sizeof(float), cudaMemcpyDeviceToHost, st));
+    CQL_CUDA(cudaStreamSynchronize(st));
+    if (loss_out) *loss_out = h.metrics_host[0];
+  });
+}
+
+int cql_copy_table(cql_handle* dst, const cql_handle* src, void* stream) {
+  return guarded(dst, [&] {
+    Handle& h = dst->h;
+    CQL_REQUIRE(src != nullptr, "cql_copy_table: NULL source handle");
+    const Handle& s = src->h;
+    CQL_REQUIRE(s.n_trans > 0, "cql_copy_table: the source handle holds no replay table");
+    CQL_REQUIRE(s.cfg.device == h.cfg.device, "cql_copy_table: the handles live on different devices");
+    CQL_REQUIRE(s.n_steps == h.n_steps, "cql_copy_table: the handles' n-step horizons differ (cql_set_n_steps)");
+    if (src == dst) return;
+    CQL_CUDA(cudaDeviceSynchronize());
+    const cql_table_stats stats = current_stats(s);
+    const int64_t n = s.n_trans;
+    ensure_table(h, n);
+    cudaStream_t st = pick_stream(&h, stream);
+    CQL_CUDA(cudaMemcpyAsync(h.table, s.table, (size_t)n * 8 * sizeof(float), cudaMemcpyDeviceToDevice, st));
+    CQL_CUDA(cudaStreamSynchronize(st));
+    h.stats = stats;
+    h.stats_rew_ok = stats.rew_available != 0;
+    h.n_trans = n;
+    destroy_graph(dst);
   });
 }
 

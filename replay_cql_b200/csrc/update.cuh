@@ -1141,8 +1141,18 @@ struct NetGroup { int first_slot, n_nets, in_dim, out_dim; float lr; };
 inline NetGroup critic_group(const Handle* h) { return NetGroup{slot_critic(0), h->C, 3, 1, h->cfg.critic_lr}; }
 inline NetGroup actor_group(const Handle* h) { return NetGroup{slot_actor(), 1, 2, 2, h->cfg.actor_lr}; }
 
+// Where an optimizer step may write the group's target copy instead of its target slots.  FQE's ordinary updates
+// (fqe.cuh) leave the target slots and their packed copies as they are: k_adam_polyak then gets no target, the target
+// slots are not repacked, and k_adam_pack -- which always writes a target copy -- writes it into this scratch.
+struct TargetSink {
+  float* params;     // [n_nets][NET_STRIDE]
+  uint8_t* fwd;      // [n_nets][packed_net_bytes]
+  uint8_t* fwd2;     // [n_nets][packed_net_bytes2] (f16x3)
+};
+
 // f16x3: Adam + Polyak + every operand copy of W2 (network and target, both orientations, both layouts) in one launch
-inline void adam_pack(Handle* h, const NetGroup& g, const BwdPlan& plan, cudaStream_t st, bool last) {
+inline void adam_pack(Handle* h, const NetGroup& g, const BwdPlan& plan, cudaStream_t st, bool last,
+                      const TargetSink* sink = nullptr) {
   const cql_config& c = h->cfg;
   const bool critic = g.in_dim == 3;
   tc::AdamPackJobs j{};
@@ -1167,6 +1177,11 @@ inline void adam_pack(Handle* h, const NetGroup& g, const BwdPlan& plan, cudaStr
     n.bwd2 = critic ? h->packed_bwd2 + (size_t)slot * h->packed_net_bytes2 : nullptr;
     n.tfwd2 = critic ? h->packed_fwd2 + (size_t)tslot * h->packed_net_bytes2 : nullptr;
     n.w2max = h->w2max + slot * 4;
+    if (sink) {
+      n.targ = sink->params + (size_t)i * NET_STRIDE;
+      n.tfwd = sink->fwd + (size_t)i * h->packed_net_bytes;
+      n.tfwd2 = critic ? sink->fwd2 + (size_t)i * h->packed_net_bytes2 : nullptr;
+    }
   }
   if (plan.fold) {                     // the partials of this group's backward (launch_bwd)
     j.small1 = h->small1; j.small2 = h->small2; j.pw2 = h->pw2_tc;
@@ -1178,21 +1193,24 @@ inline void adam_pack(Handle* h, const NetGroup& g, const BwdPlan& plan, cudaStr
 }
 
 // Adam + Polyak of one group and the refresh of its packed W2 copies; `last`: the update's final launch, which also counts
-// the step.  plan: the group's backward (launch_bwd), whose partials f16x3 sums here.
+// the step.  plan: the group's backward (launch_bwd), whose partials f16x3 sums here.  sink: the target slots stay as
+// they are (TargetSink).
 template <Prec P>
-inline void optimizer_step(Handle* h, const NetGroup& g, const BwdPlan& plan, cudaStream_t st, bool last) {
+inline void optimizer_step(Handle* h, const NetGroup& g, const BwdPlan& plan, cudaStream_t st, bool last,
+                           const TargetSink* sink = nullptr) {
   if (P == Prec::F16X3 && !switches().no_fused_adam) {
-    adam_pack(h, g, plan, st, last);
+    adam_pack(h, g, plan, st, last, sink);
     return;
   }
   const cql_config& c = h->cfg;
   const int64_t cnt = (int64_t)g.n_nets * NET_STRIDE, off = (int64_t)g.first_slot * NET_STRIDE;
   const int tslot = g.first_slot + 1 + h->C;
   launch(h, st, PDL, k_adam_polyak, dim3((int)((cnt + 255) / 256)), dim3(256), 0, h->net_params(g.first_slot), h->adam_m + off,
-         h->adam_v + off, h->grads + off, h->net_params(tslot), cnt, g.lr, c.beta1, c.beta2, c.adam_eps, c.tau, h->stepinfo);
+         h->adam_v + off, h->grads + off, sink ? nullptr : h->net_params(tslot), cnt, g.lr, c.beta1, c.beta2, c.adam_eps, c.tau,
+         h->stepinfo);
   int slots[2 * CQL_MAX_CRITICS], n = 0;
   for (int i = 0; i < g.n_nets; ++i) slots[n++] = g.first_slot + i;
-  if (g.in_dim == 3)                   // the target critics' forward (TD target) reads the packed copy; the target actor's none
+  if (g.in_dim == 3 && !sink)          // the target critics' forward (TD target) reads the packed copy; the target actor's none
     for (int i = 0; i < g.n_nets; ++i) slots[n++] = tslot + i;
   pack_slots<P>(h, slots, n, st);
   if (last) launch(h, st, PDL, k_step_end, dim3(1), dim3(1), 0, h->step_dev);

@@ -501,6 +501,35 @@ class CqlEngine:
         self._check(self._lib.cql_offline_eval(self._h, thr, C.byref(out), stream), "cql_offline_eval")
         return {k: (int if k.startswith("n_") else float)(getattr(out, k)) for k in OFFLINE_SUM_KEYS}
 
+    # ------------------------------------------------------------------ fitted Q evaluation
+    def fqe_enable(self, target_update_interval: int) -> None:
+        """FQE mode (``cql_fqe_enable``): from now on this engine trains its critics by FQE updates under the policy in
+        its actor slot; the CQL update calls are refused."""
+        self._check(self._lib.cql_fqe_enable(self._h, int(target_update_interval)), "cql_fqe_enable")
+
+    def fqe_update(self, n_steps: int = 1, stream: int | None = None) -> float:
+        """``n_steps`` sampled FQE updates (CUDA-graph replays) -> the last update's loss."""
+        loss = np.zeros(1, dtype=np.float32)
+        self._check(self._lib.cql_fqe_update(self._h, int(n_steps), _ptr(loss), stream), "cql_fqe_update")
+        return float(loss[0])
+
+    def fqe_update_rows(self, rows, want_grads: bool = False, stream: int | None = None):
+        """One FQE update on [B, 8] table-format rows (raw) -> (loss, [n_critics] gradient dicts or None)."""
+        rows = _f32(rows, (self.hp.batch_size, 8))
+        loss = np.zeros(1, dtype=np.float32)
+        C = self.hp.n_critics
+        g = np.zeros(C * layout.NET_STRIDE, dtype=np.float32) if want_grads else None
+        self._check(self._lib.cql_fqe_update_rows(self._h, _ptr(rows), _ptr(loss), _ptr(g), stream), "cql_fqe_update_rows")
+        grads = None
+        if want_grads:
+            grads = [layout.unpack_net(g[c * layout.NET_STRIDE:(c + 1) * layout.NET_STRIDE], layout.CRITIC_IN,
+                                       layout.CRITIC_OUT) for c in range(C)]
+        return float(loss[0]), grads
+
+    def copy_table_from(self, other: "CqlEngine", stream: int | None = None) -> None:
+        """This engine's replay table := ``other``'s (device to device, ``cql_copy_table``); ``other`` is unchanged."""
+        self._check(self._lib.cql_copy_table(self._h, other._h, stream), "cql_copy_table")
+
     # ------------------------------------------------------------------ scoring
     def score_topk(self, users, items, k: int, seen_indptr=None, seen_items=None, mode: str = "q"):
         """Top-``k`` unseen items per user.  -> (items [U,k] int32 (-1 pad), scores [U,k] float32 (-inf pad))"""

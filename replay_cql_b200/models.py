@@ -427,50 +427,8 @@ class CQL(Recommender):
         Nothing of the model changes: ``fit -> offline_metrics -> resume`` equals ``fit -> resume``."""
         if self.engine is None:
             raise AttributeError("CQL model is not fitted or loaded")
-        if return_threshold is not None:
-            if isinstance(return_threshold, bool) or not isinstance(return_threshold, (int, float, np.integer, np.floating)) \
-                    or not np.isfinite(float(return_threshold)):
-                raise ValueError("return_threshold must be a finite number or None")
-            return_threshold = float(return_threshold)
-        eng = self.engine
-        rank, world, local_rank = dist_info()
-        if log is None:
-            if eng.hp.n_steps > 1:
-                raise ValueError("offline_metrics: the replay table holds n-step rows (n_steps > 1) -- pass the log to "
-                                 "evaluate its one-step transitions")
-            if eng.n_transitions == 0:
-                raise ValueError("offline_metrics: the model holds no replay table (e.g. loaded from a checkpoint saved "
-                                 "without save_replay_table) -- pass the log")
-            sums = eng.offline_metrics(return_threshold)
-            sharded = world > 1 and getattr(self, "_table_sharded", False)
-        else:
-            n_log = int(log.num_rows) if hasattr(log, "num_rows") else len(log)
-            if n_log == 0:
-                raise ValueError("offline_metrics: empty log")
-            sharded = world > 1
-            if sharded:
-                from .mdp import shard_log_by_user
-                log = shard_log_by_user(log, rank, world)
-            n_local = int(log.num_rows) if hasattr(log, "num_rows") else len(log)
-            sums = {k: 0 for k in OFFLINE_SUM_KEYS}
-            if n_local:
-                ev = CqlEngine(dataclasses.replace(eng.hp, n_steps=1), device=local_rank, rank=rank, world_size=world)
-                try:
-                    ev.set_state(eng.get_state())
-                    prep = eng.get_preprocessing()
-                    if any(v is not None for v in prep.values()):
-                        ev.set_preprocessing(**prep)
-                    build_mdp_on_device(ev, log, top_k=self.top_k, action_randomization_scale=self.action_randomization_scale)
-                    sums = ev.offline_metrics(return_threshold)
-                finally:
-                    ev.close()
-        if sharded:
-            parts = gather_rows(np.array([[sums[k] for k in OFFLINE_SUM_KEYS]], dtype=np.float64))
-            total = np.zeros(len(OFFLINE_SUM_KEYS), dtype=np.float64)
-            for row in parts:                               # rank order: every rank adds the same values in the same order
-                total = total + row
-            sums = {k: (int(v) if k.startswith("n_") else float(v)) for k, v in zip(OFFLINE_SUM_KEYS, total)}
-        return offline_scores(sums, return_threshold is not None)
+        return evaluate_offline(self.engine, log, return_threshold, self.top_k, self.action_randomization_scale,
+                                getattr(self, "_table_sharded", False))
 
     def _default_criterion(self):
         """``optimize`` trials score NDCG@k on the GPU (``cql_rank_metrics``) instead of the pandas criterion."""
@@ -509,3 +467,58 @@ class CQL(Recommender):
         if meta.get("replay_rows"):
             # verbatim: n-step rows cannot be rebuilt from their columns, and one-step rows come back bit for bit
             eng.set_table_rows(np.load(os.path.join(path, "replay_table.npy")))
+
+
+def evaluate_offline(eng: CqlEngine, log: Any, return_threshold: Optional[float], top_k: int,
+                     action_randomization_scale: float, table_sharded: bool,
+                     mdp_seed: Optional[int] = None) -> Dict[str, float]:
+    """d3rlpy's offline scorers of ``eng``'s networks (``CQL.offline_metrics``, ``ope.FQE.offline_metrics``).
+
+    ``log=None`` evaluates the engine's replay table (one-step, present; ``table_sharded``: in a data-parallel job it
+    holds only this rank's users).  With a ``log`` the one-step rows are built by the MDP builder (``top_k``,
+    ``action_randomization_scale``; ``mdp_seed``, default ``eng``'s seed, draws the action noise) on a short-lived
+    evaluation engine holding ``eng``'s networks and scalers; in a data-parallel job each rank evaluates its own user range.  Sharded sums are combined in rank order."""
+    if return_threshold is not None:
+        if isinstance(return_threshold, bool) or not isinstance(return_threshold, (int, float, np.integer, np.floating)) \
+                or not np.isfinite(float(return_threshold)):
+            raise ValueError("return_threshold must be a finite number or None")
+        return_threshold = float(return_threshold)
+    rank, world, local_rank = dist_info()
+    if log is None:
+        if eng.hp.n_steps > 1:
+            raise ValueError("offline_metrics: the replay table holds n-step rows (n_steps > 1) -- pass the log to "
+                             "evaluate its one-step transitions")
+        if eng.n_transitions == 0:
+            raise ValueError("offline_metrics: the model holds no replay table (e.g. loaded from a checkpoint saved "
+                             "without save_replay_table) -- pass the log")
+        sums = eng.offline_metrics(return_threshold)
+        sharded = world > 1 and table_sharded
+    else:
+        n_log = int(log.num_rows) if hasattr(log, "num_rows") else len(log)
+        if n_log == 0:
+            raise ValueError("offline_metrics: empty log")
+        sharded = world > 1
+        if sharded:
+            from .mdp import shard_log_by_user
+            log = shard_log_by_user(log, rank, world)
+        n_local = int(log.num_rows) if hasattr(log, "num_rows") else len(log)
+        sums = {k: 0 for k in OFFLINE_SUM_KEYS}
+        if n_local:
+            hp = dataclasses.replace(eng.hp, n_steps=1, seed=eng.hp.seed if mdp_seed is None else mdp_seed)
+            ev = CqlEngine(hp, device=local_rank, rank=rank, world_size=world)
+            try:
+                ev.set_state(eng.get_state())
+                prep = eng.get_preprocessing()
+                if any(v is not None for v in prep.values()):
+                    ev.set_preprocessing(**prep)
+                build_mdp_on_device(ev, log, top_k=top_k, action_randomization_scale=action_randomization_scale)
+                sums = ev.offline_metrics(return_threshold)
+            finally:
+                ev.close()
+    if sharded:
+        parts = gather_rows(np.array([[sums[k] for k in OFFLINE_SUM_KEYS]], dtype=np.float64))
+        total = np.zeros(len(OFFLINE_SUM_KEYS), dtype=np.float64)
+        for row in parts:                                   # rank order: every rank adds the same values in the same order
+            total = total + row
+        sums = {k: (int(v) if k.startswith("n_") else float(v)) for k, v in zip(OFFLINE_SUM_KEYS, total)}
+    return offline_scores(sums, return_threshold is not None)
