@@ -57,7 +57,9 @@ typedef struct cql_config {
   int32_t n_action_samples;     /* n, 1..CQL_MAX_ACTION_SAMPLES */
   int32_t precision;            /* CQL_PREC_* */
   int32_t squash;               /* CQL_SQUASH_* */
-  int32_t rank, world_size;     /* data-parallel position (sampling streams only; no comms inside) */
+  int32_t rank, world_size;     /* data-parallel position (sampling streams only; no comms inside).  world_size
+                                 * 1..256 (else cql_create returns 3): the Philox noise stream of an update holds 8 rank
+                                 * bits, so rank 256 would draw rank 0's noise */
   float gamma, tau;
   float actor_lr, critic_lr, temp_lr, alpha_lr;
   float initial_temperature, initial_alpha;
@@ -230,7 +232,12 @@ enum { CQL_BUF_SCALAR_GRADS = 0,   /* 64 floats: [0]=d log_temp [1]=d log_alpha 
        CQL_BUF_ACTOR_GRADS = 2,    /* NET floats */
        CQL_BUF_METRICS = 3,        /* 8 floats */
        CQL_BUF_PARAMS = 4,
-       CQL_BUF_ALL_GRADS = 5 };    /* (1+C)*NET+64 floats: [actor | critics | scalars] */
+       CQL_BUF_ALL_GRADS = 5,      /* (1+C)*NET+64 floats: [actor | critics | scalars] */
+       /* read-only: what the last update on the handle consumed */
+       CQL_BUF_NOISE = 6,          /* 2B+6Bn floats: its seven draws, packed as cql_update_batch's noise argument
+                                    * (the Philox draws, or the caller's noise when one was given) */
+       CQL_BUF_BATCH = 7 };        /* B*8 floats: its minibatch rows in table format, after the scalers (the rows it
+                                    * trained on; a minibatch staged by cql_upload_batch appears here once phase 4 ran) */
 int  cql_device_buffer(cql_handle* h, int which, void** dev_ptr, int64_t* n_floats);
 
 /* Seen-items CSR of an interaction log, built on the device -- the structure the scorer's lazy seen filter searches

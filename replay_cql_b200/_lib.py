@@ -17,7 +17,7 @@ LIB_PATH = Path(os.environ["CQL_LIB"]) if os.environ.get("CQL_LIB") else Path(__
 PREC_FP32, PREC_TF32X3, PREC_BF16, PREC_F16X3 = 0, 1, 2, 3
 SQUASH_EPS, SQUASH_SOFTPLUS = 0, 1
 SCORE_Q, SCORE_POLICY = 0, 1
-BUF_SCALAR_GRADS, BUF_CRITIC_GRADS, BUF_ACTOR_GRADS, BUF_METRICS, BUF_PARAMS, BUF_ALL_GRADS = range(6)
+BUF_SCALAR_GRADS, BUF_CRITIC_GRADS, BUF_ACTOR_GRADS, BUF_METRICS, BUF_PARAMS, BUF_ALL_GRADS, BUF_NOISE, BUF_BATCH = range(8)
 MAX_TOPK = 1024
 MAX_N_STEPS = 64                                     # CQL_MAX_N_STEPS: longest n-step TD horizon
 MAX_CRITICS = 10                                     # CQL_MAX_CRITICS: largest critic ensemble (n_critics)

@@ -257,6 +257,8 @@ void create_impl(const cql_config* cfg, cql_handle* ch) {
               "cql_create: bad precision");
   CQL_REQUIRE(cfg->squash == CQL_SQUASH_EPS || cfg->squash == CQL_SQUASH_SOFTPLUS, "cql_create: bad squash");
   CQL_REQUIRE(cfg->world_size >= 1 && cfg->rank >= 0 && cfg->rank < cfg->world_size, "cql_create: bad rank/world_size");
+  // the update's Philox stream is (step << 8) | rank: a 257th rank would repeat rank 0's noise bit for bit
+  CQL_REQUIRE(cfg->world_size <= 256, "cql_create: world_size must be <= 256 (the noise stream holds 8 rank bits)");
   int ndev = 0;
   cudaError_t e = cudaGetDeviceCount(&ndev);
   if (e != cudaSuccess || ndev == 0)
@@ -1228,6 +1230,8 @@ int cql_device_buffer(cql_handle* ch, int which, void** dev_ptr, int64_t* n_floa
       case CQL_BUF_METRICS: *dev_ptr = h.metrics; *n_floats = 8; break;
       case CQL_BUF_PARAMS: *dev_ptr = h.params; *n_floats = state_floats(h.C); break;
       case CQL_BUF_ALL_GRADS: *dev_ptr = h.grads; *n_floats = grad_floats(h.C); break;
+      case CQL_BUF_NOISE: *dev_ptr = h.noise; *n_floats = h.noise_floats; break;
+      case CQL_BUF_BATCH: *dev_ptr = h.batch; *n_floats = (int64_t)h.B * 8; break;
       default: throw Error{"cql_device_buffer: unknown buffer id"};
     }
   });

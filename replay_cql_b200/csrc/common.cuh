@@ -83,7 +83,7 @@ struct Philox {
     out[0] = c[0]; out[1] = c[1]; out[2] = c[2]; out[3] = c[3];
   }
 };
-// (0,1) open interval from 32 bits
+// (0, 1] from 32 bits: the float32 sum rounds to even from x >> 8 = 2^23 on, so x >> 8 = 2^24 - 1 gives exactly 1
 __host__ __device__ inline float u01(uint32_t x) { return ((float)(x >> 8) + 0.5f) * (1.0f / 16777216.0f); }
 
 }  // namespace cql
