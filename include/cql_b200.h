@@ -371,6 +371,27 @@ int  cql_fqe_update_rows(cql_handle* h, const float* rows_host, float* loss_out,
  * with the same n-step horizon (cql_set_n_steps), else 3.  `src` is not modified.  Synchronises. */
 int  cql_copy_table(cql_handle* dst, const cql_handle* src, void* stream);
 
+/* ---- per-observation inference ----------------------------------------- */
+/* d3rlpy's predict_value / predict / sample_action on observations x_i = (users[i], items[i]) (DESIGN.md section 1,
+ * "Inference"), on the update's forward kernels in the handle's precision.  Host pointers; synchronises `stream`.
+ * Observations are observation-scaled as the update scales them; the handle's scalers apply.  Ids must lie in
+ * [0, 2^24) (exact in float32).  Nothing of the handle's state changes except cql_sample_action's call counter.
+ * cql_predict_value: mean_out[i] = mean_c Q_c(x_i, a_i) in float32 (critic order 0..C-1, rounded sums); actions NULL =
+ *   the greedy action a_i = tanh(mu(x_i)) in network space, else actions[i] in raw rating units, action-scaled into Q.
+ *   std_out (may be NULL) receives the population std of the Q_c (two-pass, ddof 0; exactly 0 at n_critics = 1).
+ * cql_sample_action: out[i] = reverse(tanh(mu(x_i))) with greedy = 1 (the value of CQL_SCORE_POLICY); with greedy = 0,
+ *   reverse(tanh(mu + exp(clamp(logstd, -20, 2)) * eps_i)) with eps_i the Box-Muller draw of Philox4x32-10 words 0
+ *   and 1 at key seed ^ 0xE7037ED1A0B428DB, stream = the handle's count of earlier greedy = 0 calls with n > 0, index
+ *   i.  That count starts at 0 with the handle and is not part of the saved state.
+ * Rejected (3): n < 0, a NULL array for n > 0, an id outside [0, 2^24), a non-finite action, greedy not 0 or 1.
+ * n = 0 returns at once.  Works on an FQE handle (its actor slot holds the evaluated policy).
+ * replaces: d3rlpy AlgoBase.predict_value(x, action, with_std), predict(x), sample_action(x) [EXT d3rlpy 1.x
+ *           algos/base.py] and d3rlpy.ope.FQE.predict_value */
+int  cql_predict_value(cql_handle* h, const int32_t* users, const int32_t* items, const float* actions, int64_t n,
+                       float* mean_out, float* std_out, void* stream);
+int  cql_sample_action(cql_handle* h, const int32_t* users, const int32_t* items, int64_t n, int32_t greedy,
+                       float* out, void* stream);
+
 /* Measurement aid: runs ONE sampled update with CUDA events around the heavy launches and
  * returns their durations in milliseconds (synchronises).  out_ms[0] = critic forward (alpha +
  * critic + target rows), [1] = critic backward-1, [2] = critic backward-2 (dW2), [3] = whole

@@ -131,6 +131,8 @@ SIGNATURES = {
     "cql_fqe_update": (C.c_int, [_P, C.c_int64, _P, _P]),
     "cql_fqe_update_rows": (C.c_int, [_P, _P, _P, _P, _P]),
     "cql_copy_table": (C.c_int, [_P, _P, _P]),
+    "cql_predict_value": (C.c_int, [_P, _P, _P, _P, C.c_int64, _P, _P, _P]),
+    "cql_sample_action": (C.c_int, [_P, _P, _P, C.c_int64, C.c_int32, _P, _P]),
 }
 
 _lib = None

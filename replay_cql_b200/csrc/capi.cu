@@ -14,6 +14,7 @@
 #include "mma_bench.cuh"
 #include "offline_eval.cuh"
 #include "fqe.cuh"
+#include "infer.cuh"
 
 using namespace cql;
 
@@ -95,6 +96,9 @@ struct cql_handle {
   // FQE mode (cql_fqe_enable): sampled updates, updates on caller rows, and the target synchronisation
   FqeState fqe;
   StepGraph fqe_graph, fqe_rows_graph, fqe_sync_graph;
+  // cql_sample_action: Philox stream of the next stochastic call (not part of the update state: never saved, never read
+  // by an update)
+  uint64_t sample_calls = 0;
 };
 
 static thread_local std::string g_create_error;
@@ -606,6 +610,17 @@ void update_staged_batch(cql_handle* ch, const float* noise, float* metrics6, fl
   if (metrics6) std::memcpy(metrics6, h.metrics_host, 6 * sizeof(float));
 }
 
+// cql_predict_value / cql_sample_action inputs: ids in [0, 2^24) (exact in float32 observations), finite actions
+void check_pairs(const char* fn, const int32_t* users, const int32_t* items, const float* actions, int64_t n) {
+  CQL_REQUIRE(n >= 0, std::string(fn) + ": n < 0");
+  CQL_REQUIRE(n == 0 || (users && items), std::string(fn) + ": NULL users or items");
+  bool ids_ok = true, acts_ok = true;
+  for (int64_t i = 0; i < n; ++i) ids_ok &= ((uint32_t)users[i] | (uint32_t)items[i]) < (1u << 24);
+  if (actions)
+    for (int64_t i = 0; i < n; ++i) acts_ok &= std::isfinite(actions[i]);
+  CQL_REQUIRE(ids_ok, std::string(fn) + ": a user or item id is outside [0, 2^24)");
+  CQL_REQUIRE(acts_ok, std::string(fn) + ": an action is not finite");
+}
 }  // namespace
 
 void cql::expand_n_steps(Handle& h, const float* one_step, int64_t n, cudaStream_t st) {
@@ -1446,6 +1461,37 @@ int cql_copy_table(cql_handle* dst, const cql_handle* src, void* stream) {
     h.stats_rew_ok = stats.rew_available != 0;
     h.n_trans = n;
     destroy_graph(dst);
+  });
+}
+
+int cql_predict_value(cql_handle* ch, const int32_t* users, const int32_t* items, const float* actions, int64_t n,
+                      float* mean_out, float* std_out, void* stream) {
+  return guarded(ch, [&] {
+    NvtxRange nvtx("cql_predict_value");
+    Handle& h = ch->h;
+    check_pairs("cql_predict_value", users, items, actions, n);
+    CQL_REQUIRE(n == 0 || mean_out, "cql_predict_value: NULL mean_out");
+    if (n == 0) return;
+    with_precision(&h, [&](auto p) {
+      infer_pairs<decltype(p)::value>(&h, users, items, actions, n, false, 0, 0, mean_out, std_out, pick_stream(&h, stream));
+    });
+  });
+}
+
+int cql_sample_action(cql_handle* ch, const int32_t* users, const int32_t* items, int64_t n, int32_t greedy, float* out,
+                      void* stream) {
+  return guarded(ch, [&] {
+    NvtxRange nvtx("cql_sample_action");
+    Handle& h = ch->h;
+    check_pairs("cql_sample_action", users, items, nullptr, n);
+    CQL_REQUIRE(greedy == 0 || greedy == 1, "cql_sample_action: greedy must be 0 or 1");
+    CQL_REQUIRE(n == 0 || out, "cql_sample_action: NULL out");
+    if (n == 0) return;
+    const uint64_t call = greedy ? 0 : ch->sample_calls;
+    with_precision(&h, [&](auto p) {
+      infer_pairs<decltype(p)::value>(&h, users, items, nullptr, n, true, greedy, call, out, nullptr, pick_stream(&h, stream));
+    });
+    if (!greedy) ch->sample_calls++;
   });
 }
 

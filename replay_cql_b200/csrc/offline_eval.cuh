@@ -81,6 +81,22 @@ __device__ __forceinline__ float oe_mean(const QSrc& s, int C, int r) {
   return __fdiv_rn(v, (float)C);
 }
 
+// mean_c Q_c of row r and, when sd is not null, the population std over the critics (numpy std, ddof 0; exactly 0 at
+// C = 1): float32, critic order 0..C-1, separately rounded sums, a two-pass variance.  The offline scorers' V and
+// sigma and cql_predict_value (infer.cuh) both come from here.
+__device__ __forceinline__ float ens_mean_std(const QSrc& s, int C, int r, float* sd) {
+  float qc[CQL_MAX_CRITICS];
+  float sum = 0.f;
+  for (int c = 0; c < C; ++c) { qc[c] = q_at(s, c, r); sum = __fadd_rn(sum, qc[c]); }
+  const float mean = __fdiv_rn(sum, (float)C);
+  if (sd) {
+    float var = 0.f;
+    for (int c = 0; c < C; ++c) { const float d = __fsub_rn(qc[c], mean); var = __fadd_rn(var, __fmul_rn(d, d)); }
+    *sd = sqrtf(__fdiv_rn(var, (float)C));
+  }
+  return mean;
+}
+
 // per data row: Q(s,a), V(s), sigma(s), TD error
 __global__ void k_oe_rows(const float4* __restrict__ rows, int64_t c0, int m, int ma, const int* __restrict__ xslot,
                           const QSrc srcQ, int C, float gamma, const Prep prep, float* __restrict__ qd,
@@ -90,12 +106,8 @@ __global__ void k_oe_rows(const float4* __restrict__ rows, int64_t c0, int m, in
   if (l >= m) return;
   const int64_t i = c0 + l;
   const float q = oe_mean(srcQ, C, l);
-  float qc[CQL_MAX_CRITICS];
-  float s = 0.f;
-  for (int c = 0; c < C; ++c) { qc[c] = q_at(srcQ, c, m + l); s = __fadd_rn(s, qc[c]); }
-  const float vs = __fdiv_rn(s, (float)C);
-  float var = 0.f;
-  for (int c = 0; c < C; ++c) { const float d = __fsub_rn(qc[c], vs); var = __fadd_rn(var, __fmul_rn(d, d)); }
+  float sd;
+  const float vs = ens_mean_std(srcQ, C, m + l, &sd);
   const float4 r0 = rows[2 * i], r1 = rows[2 * i + 1];
   float vn = 0.f;                                       // a terminal row's bootstrap is multiplied by 0
   if (r1.z == 0.f) vn = oe_mean(srcQ, C, xslot[l] >= 0 ? m + ma + xslot[l] : m + l + 1);
@@ -103,7 +115,7 @@ __global__ void k_oe_rows(const float4* __restrict__ rows, int64_t c0, int m, in
   const float e = __fsub_rn(q, y);
   qd[i] = q;
   v[i] = vs;
-  sg[i] = sqrtf(__fdiv_rn(var, (float)C));
+  sg[i] = sd;
   td[i] = __fmul_rn(e, e);
 }
 

@@ -84,6 +84,44 @@ def check_ensemble(n_critics, n_action_samples) -> None:
         raise ValueError(f"n_action_samples must be an integer in 1..{_lib.MAX_ACTION_SAMPLES}")
 
 
+MAX_ID = 2 ** 24                                     # ids are exact in float32 observations below this
+
+
+def _column(x) -> np.ndarray:
+    """1-D view of an array or an [n, 1] column (d3rlpy passes actions as [n, action_size])."""
+    a = np.asarray(x)
+    return a[:, 0] if a.ndim == 2 and a.shape[1] == 1 else a
+
+
+def inference_inputs(users, items, actions=None):
+    """Arguments of the per-observation inference calls -> (users int32, items int32, actions float32 or None), 1-D
+    and contiguous.  ``ValueError`` unless users and items are integer ids in [0, 2^24) of one length and ``actions``
+    (if given) holds one finite number per pair; the same checks the library makes (return code 3)."""
+    out = []
+    for name, ids in (("users", users), ("items", items)):
+        a = _column(ids)
+        if a.ndim != 1 or (a.size and a.dtype.kind not in "iu"):
+            raise ValueError(f"{name} must be a 1-D array of integer ids")
+        if a.size and (int(a.min()) < 0 or int(a.max()) >= MAX_ID):
+            raise ValueError(f"{name}: ids must be in [0, 2**24) to be exact in float32 observations")
+        out.append(np.ascontiguousarray(a, dtype=np.int32))
+    u, i = out
+    if u.size != i.size:
+        raise ValueError("users and items must have the same length")
+    if actions is None:
+        return u, i, None
+    a = _column(actions)
+    if a.ndim != 1 or a.size != u.size:
+        raise ValueError("actions must hold one action per (user, item) pair")
+    if a.size and a.dtype.kind not in "iuf":
+        raise ValueError("actions must be numbers")
+    with np.errstate(over="ignore"):                  # a value beyond float32 becomes inf and is rejected below
+        a = np.ascontiguousarray(a, dtype=np.float32)
+    if not np.isfinite(a).all():
+        raise ValueError("actions must be finite (as float32)")
+    return u, i, a
+
+
 def _ptr(arr: Optional[np.ndarray]):
     return None if arr is None else arr.ctypes.data_as(C.c_void_p)
 
@@ -562,6 +600,38 @@ class CqlEngine:
         out = np.empty(users.size, dtype=np.float32)
         self._check(self._lib.cql_score_pairs(self._h, _ptr(users), _ptr(items), users.size, SCORE_MODES[mode],
                                               _ptr(out), None), "cql_score_pairs")
+        return out
+
+    # ------------------------------------------------------------------ per-observation inference
+    def predict_value(self, users, items, actions=None, with_std: bool = False, stream: int | None = None):
+        """d3rlpy's ``predict_value(x, action, with_std)`` for ``x = (users[i], items[i])`` (``cql_predict_value``):
+        float32 ``mean_c Q_c(x, a)`` per pair, and with ``with_std`` also the population std over the critics
+        (``(mean, std)``).  ``actions`` are raw rating units (the action scaler maps them into Q); None = the greedy
+        action ``tanh(mu(x))`` in network space, as ``score_pairs(mode="q")``.  The model is not modified."""
+        u, i, a = inference_inputs(users, items, actions)
+        mean = np.empty(u.size, dtype=np.float32)
+        std = np.empty(u.size, dtype=np.float32) if with_std else None
+        self._check(self._lib.cql_predict_value(self._h, _ptr(u), _ptr(i), _ptr(a), u.size, _ptr(mean), _ptr(std),
+                                                stream), "cql_predict_value")
+        return (mean, std) if with_std else mean
+
+    def predict_action(self, users, items, stream: int | None = None) -> np.ndarray:
+        """d3rlpy's ``predict(x)``: the greedy action ``tanh(mu(x))`` reverse-transformed into rating units (the value of
+        ``score_pairs(mode="policy")``), float32 (``cql_sample_action`` with ``greedy = 1``)."""
+        return self._sample(users, items, 1, stream)
+
+    def sample_action(self, users, items, stream: int | None = None) -> np.ndarray:
+        """d3rlpy's ``sample_action(x)``: ``reverse(tanh(mu + exp(clamp(logstd, -20, 2)) * eps))`` per pair, float32.
+        ``eps`` is drawn from this engine's Philox stream numbered by its earlier ``sample_action`` calls (DESIGN.md
+        section 1, "Inference"): consecutive calls differ, a fresh engine with the same seed repeats them.  The counter
+        is not part of the update state; the model is not modified."""
+        return self._sample(users, items, 0, stream)
+
+    def _sample(self, users, items, greedy: int, stream) -> np.ndarray:
+        u, i, _ = inference_inputs(users, items)
+        out = np.empty(u.size, dtype=np.float32)
+        self._check(self._lib.cql_sample_action(self._h, _ptr(u), _ptr(i), u.size, int(greedy), _ptr(out), stream),
+                    "cql_sample_action")
         return out
 
     METRIC_NAMES = ("NDCG", "HitRate", "MAP", "MRR", "Precision", "Recall")

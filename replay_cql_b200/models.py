@@ -16,6 +16,7 @@ import numpy as np
 import pandas as pd
 
 from .engine import OFFLINE_SUM_KEYS, CqlEngine, CqlHyperParams, check_ensemble, offline_scores
+from .engine import inference_inputs as _inference_inputs
 from .mdp import build_mdp_on_device, seen_csr
 from .parallel import GradAllReducer, dist_info, gather_rows, shard_range
 from .recommender import Recommender, _rec_frame, get_top_k_recs
@@ -388,6 +389,37 @@ class CQL(Recommender):
         it = pairs["item_idx"].to_numpy().astype(np.int32)
         rel = self.engine.score_pairs(u, it, mode=self.score) if u.size else np.zeros(0, dtype=np.float32)
         return _rec_frame(u, it, rel)
+
+    # ------------------------------------------------------------------ per-observation inference (d3rlpy's algo calls)
+    def predict_value(self, users, items, actions=None, with_std: bool = False):
+        """d3rlpy's ``predict_value(x, action, with_std)`` on observations ``x = (users[i], items[i])`` (DESIGN.md
+        section 1, "Inference"): float32 ``mean_c Q_c(x, a)`` per pair and, with ``with_std``, ``(mean, std)`` with the
+        population std over the critics (0 at ``n_critics = 1``).  ``actions`` are in rating units and pass through the
+        fitted action scaler; None uses the greedy action ``tanh(mu(x))`` in network space (the value of
+        ``score="q"``).  Ids must lie in [0, 2^24).  Data parallel: every rank computes its own inputs locally, with no
+        collective.  The model is not modified."""
+        u, i, a = _inference_inputs(users, items, actions)
+        return self._fitted_engine().predict_value(u, i, a, with_std=with_std)
+
+    def predict_action(self, users, items) -> np.ndarray:
+        """d3rlpy's ``predict(x)``: the greedy action ``tanh(mu(x))`` per pair in rating units (the value of
+        ``score="policy"``), float32.  Data parallel: every rank computes its own inputs locally."""
+        u, i, _ = _inference_inputs(users, items)
+        return self._fitted_engine().predict_action(u, i)
+
+    def sample_action(self, users, items) -> np.ndarray:
+        """d3rlpy's ``sample_action(x)``: one draw per pair from the squashed Gaussian policy, in rating units, float32.
+        The noise comes from a Philox stream keyed by ``seed`` and numbered by this model's earlier ``sample_action``
+        calls since its engine was created (``fit`` or ``load``): consecutive calls differ, and a model fitted or loaded
+        the same way repeats them.  The counter is not saved and the update never reads it.  Data parallel: every rank
+        computes its own inputs locally, with no collective (ranks asking for the same rows draw the same noise)."""
+        u, i, _ = _inference_inputs(users, items)
+        return self._fitted_engine().sample_action(u, i)
+
+    def _fitted_engine(self) -> CqlEngine:
+        if self.engine is None:
+            raise AttributeError("CQL model is not fitted or loaded")
+        return self.engine
 
     # ------------------------------------------------------------------ evaluation (the step right after predict)
     def evaluate(self, recs: pd.DataFrame, ground_truth: pd.DataFrame, k) -> dict:

@@ -136,9 +136,17 @@ class FQE:
             self.last_loss = self.engine.fqe_update(total)
         return self
 
-    def predict_value(self, users, items) -> np.ndarray:
-        """``mean_c Q_fqe_c(x, pi(x))`` for the pairs ``x = (users[i], items[i])`` (float32)."""
-        return self.engine.score_pairs(users, items, mode="q")
+    def predict_value(self, users, items, actions=None, with_std: bool = False):
+        """d3rlpy's ``FQE.predict_value(x, action, with_std)`` on the FQE critics for the pairs
+        ``x = (users[i], items[i])``, float32: ``mean_c Q_fqe_c(x, a)`` and, with ``with_std``, ``(mean, std)`` with the
+        population std over the FQE critics.  ``actions`` are in rating units (the model's action scaler applies); None
+        evaluates the policy's own greedy action ``pi(x)``.  The two-argument call runs on the pair scorer
+        (``score_pairs``), as it always has; explicit actions or ``with_std`` run on the forward kernels
+        (``CQL.predict_value``), which agree with it within the 1e-5 Q-score gate.  Every rank of a data-parallel job computes its
+        own inputs locally, with no collective."""
+        if actions is None and not with_std:
+            return self.engine.score_pairs(users, items, mode="q")
+        return self.engine.predict_value(users, items, actions, with_std=with_std)
 
     def offline_metrics(self, log: Any = None, return_threshold: Optional[float] = None) -> Dict[str, float]:
         """d3rlpy's offline scorers on the FQE critics (same keys as ``CQL.offline_metrics``):
